@@ -2,6 +2,7 @@
 """bench.py — throughput of the quasi-MCP downsampling hot path on B200 (one JSON line on stdout).
 
     python bench.py --gpus N --steps K --warmup W [--workload c5|c4|c2|c1] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (validate -> bundle sort -> coverage/demand/CSR ->
 component split -> push-relabel max-flow -> kept-read bitmap) over one batch of synthetic reads.
@@ -283,7 +284,8 @@ def cpu_make_input(O, wl, k, pairs, L):
 
 
 def cpu_solve_one(O, wl, inp, L):
-    """The reference's CPU path on one input: (filter,) coverage, graph, max-flow, selection."""
+    """The reference's CPU path on one input: (filter,) coverage, graph, max-flow, selection.
+    Returns (flow value, kept count, kept flag of every (post-filter) read)."""
     if "filter" in wl:
         s, e, q, l, a0, a1 = inp
         pp, kept = O.filter_pairs(s, e, q, l, wl["filter"]["min_len"], wl["filter"]["min_mapq"],
@@ -295,10 +297,10 @@ def cpu_solve_one(O, wl, inp, L):
     if ALGORITHM == "mcp":  # mcp-cpu's objective: greedy interval multicover (== min-cost optimum)
         cov = O.coverage_fast(s, e, L)
         fstar = int(np.maximum(0, np.diff(np.minimum(np.concatenate([[0], cov]), wl["M"]).astype(np.int64))).sum())
-        _, nk = O.greedy_multicover(s, e, L, wl["M"])
-        return fstar, int(nk)
+        kept, nk = O.greedy_multicover(s, e, L, wl["M"])
+        return fstar, int(nk), kept
     kept, st = O.ref_solve(s, e, L, wl["M"])
-    return int(st.flow_value), int(st.n_kept)
+    return int(st.flow_value), int(st.n_kept), kept
 
 
 def run_reference(args, wl, wname):
@@ -324,6 +326,13 @@ def run_reference(args, wl, wname):
     for _ in range(args.steps):
         res = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:  # solve 0: the same input whatever the number of host threads
+        flow, n_kept, kept = res[0]
+        idx = sample_index(len(kept))
+        save_npy(args.dump_outputs, "kept_sample_index", idx)
+        save_npy(args.dump_outputs, "kept_sample", kept[idx], np.float32)
+        save_npy(args.dump_outputs, "flow_value", [flow])
+        save_npy(args.dump_outputs, "n_kept", [n_kept])
     reads = 2 * pairs * cores * args.steps
     value = reads / dt
     sample = "%d independent solves per step (one per host thread), each %d reads over %d bp, M=%d" \
@@ -620,6 +629,9 @@ def run_b200(args, wl, wname):
             if not clk.rejected():
                 break
             log("clock record shows %s — measuring once more" % sorted(clk.reasons))
+        if args.dump_outputs and rank == 0:  # before the e2e legs reuse the bitmap
+            dump_outputs(args.dump_outputs, bitmaps2[(step_no[0] - 1) % 2] if world > 1 else bitmap,
+                         r_last["filt_off"] if fx is not None else read_off, r_last, pair_pass)
         prof = solver.kernel_profile()
         e2e_runs = {}
         if compact_ok:
@@ -769,6 +781,51 @@ def run_b200(args, wl, wname):
     emit(line)
 
 
+DUMP_READS = 1 << 21   # --dump-outputs: flags of at most this many reads (and pairs), < 64 MB in all
+
+
+def save_npy(out_dir, name, values, dtype=np.float64):
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), np.asarray(values, dtype=dtype))
+
+
+def sample_index(n):
+    """Every index below n when n <= DUMP_READS, else an ascending fixed seeded sample of them."""
+    if n <= DUMP_READS:
+        return np.arange(n, dtype=np.int64)
+    return np.unique(np.random.default_rng(0).integers(0, n, size=DUMP_READS, dtype=np.int64))
+
+
+def dump_outputs(out_dir, bitmap, off, r, pair_pass=None):
+    """What a caller of the timed path receives from its last step, as .npy files: the kept-read
+    count of every sample, the kept flags of a sample of reads (sample_index), with the pair filter
+    the verdicts of a sample of pairs, and the result's counters.  off holds the offsets of the
+    samples' reads in the bitmap (post-filter offsets with the pair filter: the bitmap indexes the
+    reads that passed).  Comparable between builds: the inputs depend only on the workload's seeds."""
+    import torch
+    off = [int(x) for x in off]
+    words = bitmap[:(off[-1] + 31) // 32]
+    shifts = torch.arange(32, dtype=torch.int32, device=words.device)
+    per_sample = []
+    for lo, hi in zip(off[:-1], off[1:]):
+        w0 = lo // 32
+        flags = ((words[w0:(hi + 31) // 32].unsqueeze(1) >> shifts) & 1).flatten()[lo - 32 * w0:hi - 32 * w0]
+        per_sample.append(int(flags.sum().item()))
+    save_npy(out_dir, "kept_per_sample", per_sample)
+    idx = sample_index(off[-1])
+    d_idx = torch.from_numpy(idx).to(words.device)
+    save_npy(out_dir, "kept_sample_index", idx)
+    save_npy(out_dir, "kept_sample", ((words[d_idx >> 5] >> (d_idx & 31).int()) & 1).cpu().numpy(),
+             np.float32)
+    if pair_pass is not None:
+        idx = sample_index(len(pair_pass))
+        save_npy(out_dir, "pair_pass_sample_index", idx)
+        save_npy(out_dir, "pair_pass_sample",
+                 pair_pass[torch.from_numpy(idx).to(pair_pass.device)].cpu().numpy(), np.float32)
+    for k in ("fstar", "flow_value", "n_filtered", "n_kept"):
+        save_npy(out_dir, k, [int(getattr(r, k))])
+
+
 def emit(line):
     """The ONE JSON line goes to the real stdout; everything else (NCCL's version banner, library
     chatter) was redirected to stderr by main()."""
@@ -809,7 +866,12 @@ def main():
     ap.add_argument("--algorithm", default="quasi-mcp", choices=["quasi-mcp", "mcp"],
                     help="quasi-mcp: maximum flow by push-relabel (the north-star path, default); mcp: the "
                          "minimum-cardinality solve (gds_params.algorithm = 1, plugin mcp-b200)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                         "(rank 0's samples when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global ALGORITHM, SEG_LEN, SCHEDULE
     ALGORITHM = args.algorithm
     SEG_LEN = args.seg_len

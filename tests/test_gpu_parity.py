@@ -1,12 +1,18 @@
 """GPU parity tests proper: every call goes through the C ABI (include/gds.h) and is compared
 with the CPU oracle on the same seeded inputs — bit-exact for F*, demand vector, capped coverage,
 kept bitmap (deterministic schedule) and even the round count."""
+import hashlib
+
 import numpy as np
 import pytest
 
 from conftest import PRM
 
 pytestmark = pytest.mark.gpu
+
+
+def sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def assert_parity(O, r, s, e, ref_lens, read_off, M, prm=PRM):
@@ -171,10 +177,10 @@ def test_filter_path_c2_small(solver, O):
             assert_parity(O, r, fs, fe, [30_000], [0, kept], M, oprm)
 
 
-def test_c2_full_size_filter_and_solve(solver, O, R):
+def test_c2_full_size_filter_and_solve(solver, O, golden):
     # BASELINE config 2 at full size: 10M reads, -l 90 -q 30, synthetic ARTIC BED/TSV, M=100.
-    # The device filter must equal the oracle's AND the reference's own read_bam filter (oracle/_ref
-    # on a 1/20 slice, the fake in-memory BAM is slow); the solve is checked bit for bit.
+    # The device filter must equal the oracle's AND the reference's own read_bam filter (golden.json
+    # holds its output for the first 20k pairs of this stream); the solve is checked bit for bit.
     bed, tsv = O.artic_scheme()
     a0, a1 = O.parse_amplicons(bed, tsv)
     s, e, q, l = O.gen_reads_amplicon(12345, 5_000_000, 30_000, a0, a1)
@@ -185,11 +191,15 @@ def test_c2_full_size_filter_and_solve(solver, O, R):
     assert np.array_equal(r.pair_pass, pp) and r.n_filtered == kept and 0 < kept < len(s)
     mask = np.repeat(pp, 2).astype(bool)
     assert_parity(O, r, s[mask].copy(), e[mask].copy(), [30_000], [0, kept], 100, (64, 150, 1, 0, 0, 3))
-    n_ref = 500_000
-    ref = R.read_bam(s[:n_ref].copy(), e[:n_ref].copy(), q[:n_ref].copy(), l[:n_ref].copy(), 30_000,
-                     90, 30, bed, tsv)
-    assert np.array_equal(ref["start"], s[:n_ref][mask[:n_ref]])
-    assert np.array_equal(ref["end"], e[:n_ref][mask[:n_ref]])
+    gf = golden["filter"]
+    ref = gf["cases"]["l90_q30_tsv"]
+    assert (gf["seed"], gf["L"], gf["bed"], gf["tsv"]) == (12345, 30_000, bed, tsv)
+    assert (ref["min_len"], ref["min_mapq"], ref["use_bed"], ref["use_tsv"]) == (90, 30, True, True)
+    n_ref = 2 * gf["pairs"]
+    dev = np.repeat(r.pair_pass[:n_ref // 2], 2).astype(bool)
+    assert int(dev.sum()) == ref["n_kept"]
+    assert sha(np.nonzero(dev)[0].astype(np.uint64)) == ref["bam_id"]
+    assert sha(s[:n_ref][dev]) == ref["start"] and sha(e[:n_ref][dev]) == ref["end"]
 
 
 def test_filter_on_batches_keeps_sample_offsets(solver, O):

@@ -1,59 +1,89 @@
-"""The oracle against the REFERENCE'S OWN code, live (oracle/_ref/libgds_ref.so built from
-/root/reference).  Skipped when the .so is absent.  The same outputs are frozen in
-tests/golden/golden.json for boxes that cannot build it."""
+"""The project's restatements against the REFERENCE'S OWN outputs: tests/golden/make_golden.py
+froze them in tests/golden/golden.json from a build of the reference's unmodified sources.
+tests/test_oracle.py checks the oracle's generator and filter against the same entries; the tests
+here check the host mirror's generators and BAM reader, the exact per-read coverage routine,
+find_pairs on a bitmap, and the reference's CoverageTester against the oracle's solver."""
+import hashlib
+
 import numpy as np
+import pytest
 
 from conftest import PRM
 
 
-def test_generators_bit_exact(O, R):
-    for shape, name in enumerate(["uniform", "low_sides", "hole", "zero_sides"]):
-        for seed, pairs, L, Rl in [(12345, 20_000, 30_000, 150), (9, 500, 700, 31)]:
-            a = O.gen_reads(seed, pairs, L, Rl, name)
-            b = R.gen_reads(seed, pairs, L, Rl, shape)
-            for x, y in zip(a, b):
-                assert np.array_equal(x, y)
+def sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
-def test_cover_helpers_bit_exact(O, R):
-    s, e, q, l = O.gen_reads(3, 5_000, 4_000, 80, "hole")
-    assert np.array_equal(O.coverage(s, e, 4_000), R.input_cover(s, e, 4_000))
-    ids = np.arange(0, len(s), 7, dtype=np.uint64)
-    mask = np.zeros(len(s), np.uint8); mask[ids] = 1
-    assert np.array_equal(O.coverage(s, e, 4_000, mask), R.filtered_cover(s, e, 4_000, ids))
+SHAPE_NAMES = ["uniform", "low_sides", "hole", "zero_sides"]
 
 
-def test_filter_matches_read_bam(O, R):
-    bed, tsv = O.artic_scheme()
-    a0, a1 = O.parse_amplicons(bed, tsv)
-    s, e, q, l = O.gen_reads_amplicon(77, 15_000, 30_000, a0, a1)
-    for ml, mq, ub, ut in [(90, 30, True, True), (90, 30, True, False), (0, 0, True, True),
-                           (120, 50, False, False)]:
-        ref = R.read_bam(s, e, q, l, 30_000, ml, mq, bed if ub else None, tsv if ut else None)
-        x0, x1 = O.parse_amplicons(bed, tsv if ut else None)
-        pp, kept = O.filter_pairs(s, e, q, l, ml, mq, x0 if ub else None, x1 if ub else None)
-        mask = np.repeat(pp, 2).astype(bool)
-        assert kept == len(ref["start"])
-        assert np.array_equal(np.nonzero(mask)[0], ref["bam_id"])
-        assert np.array_equal(s[mask], ref["start"]) and np.array_equal(e[mask], ref["end"])
-        assert np.array_equal(np.nonzero(~mask)[0], ref["filtered_out"])
+@pytest.fixture(scope="module")
+def hostlib(pkg):
+    from genome_downsampler_b200 import hostlib
+    hostlib.load()
+    return hostlib
 
 
-def test_find_pairs_bitmap_equals_reference_set(O, R):
-    s, e, q, l = O.gen_reads(5, 300, 900, 40)
-    rng = np.random.default_rng(0)
-    ids = np.sort(rng.choice(len(s), 150, replace=False)).astype(np.uint64)
-    ref = R.find_pairs(s, e, 900, ids)
-    bm = np.zeros((len(s) + 31) // 32, np.uint32)
+def test_generators_bit_exact(hostlib, golden):
+    # the C++ host mirror of reads_gen.cpp, every stored stream and all four columns
+    for name, g in sorted(golden["generators"].items()):
+        n = 2 * g["pairs"]
+        s = np.empty(n, np.uint32); e = np.empty(n, np.uint32)
+        q = np.empty(n, np.uint8); l = np.empty(n, np.uint32)
+        hostlib.gen_reads_into(g["seed"], g["pairs"], g["L"], g["R"], s, e, q, l,
+                               shape=SHAPE_NAMES[g["shape"]])
+        assert [sha(s), sha(e), sha(q.astype(np.uint32)), sha(l)] == \
+            [g["start"], g["end"], g["quality"], g["seq_len"]], name
+
+
+def test_cover_helpers_bit_exact(O, golden):
+    # the exact per-read coverage (not coverage_fast) against BamApi::find_input_cover
+    for name in ("small_uniform", "small_hole", "c3"):
+        g = golden["generators"][name]
+        s, e, q, l = O.gen_reads(g["seed"], g["pairs"], g["L"], g["R"], SHAPE_NAMES[g["shape"]])
+        cov = O.coverage(s, e, g["L"])
+        assert sha(cov) == g["cover"] and cov[:8].tolist() == g["cover_head"], name
+        assert int(cov.sum()) == g["cover_sum"], name
+
+
+def test_filter_matches_read_bam(hostlib, golden, tmp_path):
+    # the host BAM reader's pair filter (BamApi(input_filepath, config)) on a BAM of the stored
+    # input against the reference's BamApi::read_bam
+    gf = golden["filter"]
+    bedp, tsvp, path = tmp_path / "scheme.bed", tmp_path / "pairs.tsv", tmp_path / "in.bam"
+    bedp.write_text(gf["bed"]); tsvp.write_text(gf["tsv"])
+    a0, a1 = hostlib.artic_amplicons(gf["L"])
+    n = 2 * gf["pairs"]
+    s = np.empty(n, np.uint32); e = np.empty(n, np.uint32)
+    q = np.empty(n, np.uint8); l = np.empty(n, np.uint32)
+    hostlib.gen_reads_amplicon_into(gf["seed"], gf["pairs"], gf["L"], a0, a1, s, e, q, l)
+    hostlib.write_synthetic_bam(path, gf["L"], s, e, q, l, coordinate_sorted=False, threads=2)
+    for name, c in sorted(gf["cases"].items()):
+        b = hostlib.BamFile(path, min_len=c["min_len"], min_mapq=c["min_mapq"],
+                            bed=bedp if c["use_bed"] else None,
+                            tsv=tsvp if c["use_bed"] and c["use_tsv"] else None, threads=2)
+        got, out = b.reads(), b.filtered_out()
+        b.close()
+        assert len(got["bam_id"]) == c["n_kept"], name
+        assert sha(got["bam_id"]) == c["bam_id"] and got["bam_id"][:10].tolist() == c["first_ids"], name
+        assert sha(got["start"].astype(np.uint32)) == c["start"], name
+        assert sha(got["end"].astype(np.uint32)) == c["end"], name
+        assert sha(out) == c["filtered_out"], name
+
+
+def test_find_pairs_bitmap_equals_reference_set(O, golden):
+    ids = golden["small16"]["filtered_cover_ids"]
+    bm = np.zeros(1, np.uint32)
     for i in ids:
-        bm[int(i) >> 5] |= np.uint32(1 << (int(i) & 31))
-    got = np.nonzero(O.bitmap_to_mask(O.find_pairs_bitmap(bm, len(s)), len(s)))[0]
-    assert sorted(ref.tolist()) == got.tolist()
+        bm[0] |= np.uint32(1 << int(i))
+    got = np.nonzero(O.bitmap_to_mask(O.find_pairs_bitmap(bm, 16), 16))[0]
+    assert sorted(golden["small16"]["find_pairs"]) == got.tolist()
 
 
-def test_reference_coverage_tester_accepts_oracle_solvers(O, R):
-    # CoverageTester::test (5 cases, asserts live) through qmcp::Solver
+def test_reference_coverage_tester_accepts_oracle_solvers(O, coverage_tester):
+    # CoverageTester::test (5 cases) through qmcp::Solver
     def sync(M, L, s, e):
         bm, st = O.sync_solve(s, e, [L], [0, len(s)], M, params=PRM)
         return np.nonzero(O.bitmap_to_mask(bm, len(s)))[0]
-    assert R.run_coverage_tests(sync) == 5
+    assert coverage_tester(sync) == 5
