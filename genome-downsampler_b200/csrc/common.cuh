@@ -92,10 +92,16 @@ struct KScope {
     }
 };
 
-// Grow-only device buffer (arena slot).  Reused across gds_solve calls.
+// Grow-only device buffer (arena slot).  Reused across gds_solve calls, freed with its owner.
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     template <typename T>
     T* get(size_t n) {
         size_t bytes = n * sizeof(T);
@@ -120,11 +126,6 @@ struct DevBuf {
     template <typename T>
     T* as() const {
         return reinterpret_cast<T*>(p);
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
     }
 };
 

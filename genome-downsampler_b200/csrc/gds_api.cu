@@ -54,25 +54,13 @@ struct gds_ctx {
     DevBuf unc, adj, fmult, dead;  // forced reads out, cuts in (graph.cuh)
     DevBuf dhist, dlay, b_slot, ident, dwork;  // direct (sort-free) bundle path
     DevBuf kstat, pbund, cand, dctl, in_src, dem_v, fb_list, in1, lab_g, taken;
-    int sweep_smem_set = 0;
-    int mf2_smem_set[3] = {0, 0, 0};
+    unsigned sweep_smem_set = 0;  // bit i: the sweep launch shape i has its shared memory set up
+    int mf2_smem_set[2] = {0, 0};
     unsigned direct_attr = 0;                  // bytes of dynamic smem the direct kernels are set up for
     int mf_smem_set[4] = {0, 0, 0, 0};  // dynamic shared memory the launch shapes are set up for
     bool atomic_rank = false;  // shared-memory atomics rank in lane order on this device (probed)
     Profiler prof;
 
-    void release_all() {
-        DevBuf* all[] = {&in_start, &in_end, &in_mapq, &in_len, &in_raw, &off_d, &reflen_d, &base_d, &foff_d,
-                         &amp_s, &amp_e, &pair_pass, &flag32, &fS, &fE, &small, &keysA, &keysB,
-                         &valsA, &valsB, &tile_counts, &radix.hist, &radix.scan.l1, &radix.scan.l2,
-                         &scan.l1, &scan.l2, &b_first, &b_key, &b_t, &bund, &diff,
-                         &outdeg, &indeg, &excl, &tkA, &tkB, &tvA, &tvB, &node_rec, &n_dsnap, &comp_start, &comp_end, &comp_sidx,
-                         &comp_lo, &comp_hi, &qF, &qT, &qN, &qH, &work_counter, &comp_stats,
-                         &bitmap, &cov_tmp, &dem_tmp, &vdiff, &vexcl, &vs_d, &cross_idx, &cross_tc,
-                         &odiff, &oexcl, &cut_nodes, &tile_off_d, &head_bits, &dhist, &dlay, &b_slot,
-                         &ident, &dwork, &kstat, &pbund, &cand, &dctl, &in_src, &dem_v, &fb_list, &in1, &lab_g, &taken, &unc, &adj, &fmult, &dead};
-        for (DevBuf* b : all) b->release();
-    }
 };
 
 namespace {
@@ -165,11 +153,6 @@ void launch_maxflow(gds_ctx* c, const MfGraph& mg,
             shape = i;
             break;
         }
-    // GDS_MF_SHAPE=0..3: measurement knob (the schedule does not depend on the launch shape)
-    if (const char* e = getenv("GDS_MF_SHAPE"))
-        if (e[0] >= '0' && e[0] <= '3' && !e[1]) shape = e[0] - '0';
-    if (const char* e = getenv("GDS_MF_SMEM_LABELS"))  // =0: labels stay in global memory
-        if (e[0] == '0') max_comp_nodes = 0;
     switch (shape) {
         case 0: launch_maxflow_shape<0>(c, mg, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, max_comp_nodes, comp_list, comp_list_n, n_comp_dev, mft, lab_g); break;
         case 1: launch_maxflow_shape<1>(c, mg, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, max_comp_nodes, comp_list, comp_list_n, n_comp_dev, mft, lab_g); break;
@@ -239,7 +222,7 @@ uint32_t default_seg_len(uint32_t n_samples, const uint32_t* ref_len) {
 struct Mf2Plan {
     bool on = false;
     bool classic_ok = false;  // components outside the express schedule may run in k_maxflow_sm too
-    int smem = 0, per_sm = 1, shape = 1;
+    int smem = 0, per_sm = 1;  // two CTAs per SM run 256 threads each, one runs 512
     uint32_t qcap = 0;
     bool optr = false;
 };
@@ -291,19 +274,9 @@ Mf2Plan plan_maxflow_sm(uint32_t n_comp, uint32_t max_comp_nodes, bool express_p
     pl.classic_ok = !(env && !strcmp(env, "global")) &&
                     (forced || (unsigned long long)n_comp * 2 <= 3ull * kNumSMs * per_sm);
     if (!pl.classic_ok && !express_possible) return pl;
-    // 1024 threads would cap the kernel at 64 registers and make it spill: local memory is what this
-    // kernel must not touch (maxflow_sm.cuh), so it is a measurement knob only
-    int shape = per_sm >= 2 ? 0 : 1;
-    if (const char* e = getenv("GDS_MF2_THREADS")) {
-        if (!strcmp(e, "256")) shape = 0;
-        if (!strcmp(e, "512")) shape = 1;
-        if (!strcmp(e, "1024")) shape = 2;
-    }
-    if (shape != 0) per_sm = 1;
     pl.on = true;
     pl.smem = (int)((smem_ll + 15) & ~15ll);
     pl.per_sm = per_sm;
-    pl.shape = shape;
     pl.qcap = qcap;
     pl.optr = optr;
     return pl;
@@ -315,30 +288,26 @@ void launch_maxflow_sm(gds_ctx* c, const Mf2Plan& pl, const Mf2Graph& g, const u
                        CompStats* cstats, unsigned long long alg_bytes, uint32_t* fb_list,
                        uint32_t* fb_count, const uint32_t* n_comp_dev, MfTotals* mft) {
     KScope ks("maxflow", alg_bytes, c->stream);
-    switch (pl.shape) {
-        case 0: launch_mf2_shape<256, 0>(c, g, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, pl.smem, pl.qcap, fb_list, fb_count, pl.optr, pl.per_sm, n_comp_dev, mft); break;
-        case 1: launch_mf2_shape<512, 1>(c, g, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, pl.smem, pl.qcap, fb_list, fb_count, pl.optr, pl.per_sm, n_comp_dev, mft); break;
-        default: launch_mf2_shape<1024, 2>(c, g, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, pl.smem, pl.qcap, fb_list, fb_count, pl.optr, pl.per_sm, n_comp_dev, mft); break;
-    }
+    if (pl.per_sm >= 2)
+        launch_mf2_shape<256, 0>(c, g, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, pl.smem, pl.qcap, fb_list, fb_count, pl.optr, pl.per_sm, n_comp_dev, mft);
+    else
+        launch_mf2_shape<512, 1>(c, g, comp_lo, comp_hi, n_comp, wc, qF, qT, qN, qH, sp, cstats, pl.smem, pl.qcap, fb_list, fb_count, pl.optr, pl.per_sm, n_comp_dev, mft);
     GDS_KERNEL_CHECK();
 }
 
 // K3' (sweep.cuh): the minimum-cardinality solve.  One warp per component.
-template <int W, int CAP, bool WARP>
+template <int W, int CAP, bool WARP, int SLOT>
 void launch_sweep_shape(gds_ctx* c, const SweepGraph& g, const uint32_t* comp_lo, const uint32_t* comp_hi,
                         uint32_t n_comp, const uint32_t* n_comp_dev, uint32_t M, uint32_t* wc,
                         unsigned long long* fail) {
-    const int smem = kSweepWarps * (2 * W + 4 * CAP + 2 * 34 + 2 * 32) * 4;
+    constexpr int smem = kSweepWarps * (2 * W + 4 * CAP + 2 * 34 + 2 * 32) * 4;
     const int grid = std::max(1, std::min<int>(div_up(n_comp, kSweepWarps), kNumSMs * 8));
-    if (WARP) {
-        auto kern = k_sweep_warp<W, CAP>;
+    auto kern = WARP ? k_sweep_warp<W, CAP> : k_sweep<W, CAP>;
+    if (!(c->sweep_smem_set & (1u << SLOT))) {
         GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        kern<<<grid, kSweepWarps * 32, smem, c->stream>>>(g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail);
-    } else {
-        auto kern = k_sweep<W, CAP>;
-        GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        kern<<<grid, kSweepWarps * 32, smem, c->stream>>>(g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail);
+        c->sweep_smem_set |= 1u << SLOT;
     }
+    kern<<<grid, kSweepWarps * 32, smem, c->stream>>>(g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail);
 }
 
 void launch_sweep(gds_ctx* c, const SweepGraph& g, const uint32_t* comp_lo, const uint32_t* comp_hi,
@@ -350,20 +319,19 @@ void launch_sweep(gds_ctx* c, const SweepGraph& g, const uint32_t* comp_lo, cons
     // arrivals per position -> the warp-synchronous walk adds them in parallel
     const int w = maxlen < 256 ? 0 : maxlen < 1024 ? 1 : 2;
     switch (w * 2 + (one_len ? 0 : 1)) {
-        case 0: launch_sweep_shape<256, 64, false>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
-        case 1: launch_sweep_shape<256, 1024, true>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
-        case 2: launch_sweep_shape<1024, 64, false>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
-        case 3: launch_sweep_shape<1024, 1024, true>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
-        case 4: launch_sweep_shape<4096, 64, false>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
-        default: launch_sweep_shape<4096, 1024, true>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
+        case 0: launch_sweep_shape<256, 64, false, 0>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
+        case 1: launch_sweep_shape<256, 1024, true, 1>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
+        case 2: launch_sweep_shape<1024, 64, false, 2>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
+        case 3: launch_sweep_shape<1024, 1024, true, 3>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
+        case 4: launch_sweep_shape<4096, 64, false, 4>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
+        default: launch_sweep_shape<4096, 1024, true, 5>(c, g, comp_lo, comp_hi, n_comp, n_comp_dev, M, wc, fail); break;
     }
     GDS_KERNEL_CHECK();
 }
 
 template <typename K>
 void build_bundles(gds_ctx* c, const uint32_t* S, const uint32_t* E, const VLayout& vl,
-                   const uint32_t* cross_idx, size_t N, const TileMap& tm, const TileMap& tm_small,
-                   bool local_keys,
+                   const uint32_t* cross_idx, size_t N, const TileMap& tm, bool local_keys,
                    uint32_t n_nodes, int keybits, int lenbits, uint32_t minlen, int32_t* odiff,
                    const uint32_t* fused_ref_len, uint32_t* stats, uint32_t hint_min,
                    uint32_t hint_max, uint32_t& B_out, uint32_t*& sorted_idx_out, int& passes_out) {
@@ -377,14 +345,12 @@ void build_bundles(gds_ctx* c, const uint32_t* S, const uint32_t* E, const VLayo
     if (local_keys) {
         ReadKeys<K, true> rk{S, E, vl, cross_idx, N, lenbits, minlen, fused_ref_len, stats,
                              hint_min, hint_max};
-        where = radix_sort_pairs<K, ReadKeys<K, true>>(kA, vA, kB, vB, tm, tm_small, keybits,
-                                                       c->radix, st, c->atomic_rank, &passes_out,
-                                                       &rk);
+        where = radix_sort_pairs<K, ReadKeys<K, true>>(kA, vA, kB, vB, tm, keybits, c->radix, st,
+                                                       c->atomic_rank, &passes_out, &rk);
     } else {
         ReadKeys<K, false> rk{S, E, vl, cross_idx, N, lenbits, minlen, nullptr, stats, 0, 0};
-        where = radix_sort_pairs<K, ReadKeys<K, false>>(kA, vA, kB, vB, tm, tm_small, keybits,
-                                                        c->radix, st, c->atomic_rank, &passes_out,
-                                                        &rk);
+        where = radix_sort_pairs<K, ReadKeys<K, false>>(kA, vA, kB, vB, tm, keybits, c->radix, st,
+                                                        c->atomic_rank, &passes_out, &rk);
     }
     const K* keys = where ? kB : kA;
     sorted_idx_out = where ? vB : vA;
@@ -731,15 +697,6 @@ void direct_select(gds_ctx* c, const DirectPlan& dp, const uint32_t* S, const ui
     if (dp.lazy) GDS_CUDA(cudaMemcpyAsync(stats + kStatCtl, ctl, 16, cudaMemcpyDeviceToDevice, st));
 }
 
-// 0 = choose, 1 = always the radix sort, 2 = the direct histogram whenever eligible
-int bundle_mode(const gds_params* prm) {
-    if (const char* e = getenv("GDS_BUNDLE")) {
-        if (!strcmp(e, "sort")) return 1;
-        if (!strcmp(e, "direct")) return 2;
-    }
-    return prm ? (int)prm->bundle_mode : 0;
-}
-
 }  // namespace
 
 extern "C" int gds_abi_version(void) { return GDS_ABI_VERSION; }
@@ -771,7 +728,6 @@ extern "C" void gds_destroy(gds_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    c->release_all();
     c->prof.release();
     for (int i = 0; i < EV_COUNT; ++i)
         if (c->ev[i]) cudaEventDestroy(c->ev[i]);
@@ -1192,7 +1148,8 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
             GDS_CUDA(cudaMemsetAsync(odiff, 0, ((size_t)n_onodes + 1) * 4, st));
         }
         // how K2 finds the bundles: shared-memory histogram, global-memory histogram, radix sort
-        const int bmode = bundle_mode(prm);
+        // 0 = choose, 1 = always the radix sort, 2 = the direct histogram whenever eligible
+        const int bmode = prm ? (int)prm->bundle_mode : 0;
         const bool use_direct =
             N > 0 && !split && bmode != 1 && direct_eligible(rd, ns, minlen, maxlen, S, E);
         const bool use_gdirect = N > 0 && !use_direct && bmode != 1 &&
@@ -1263,35 +1220,28 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
                     throw InputFail{GDS_ERR_ARG, 1, "reads outside the len_min/len_max hints"};
             }
             const uint32_t* fused_ref = (fused_validation && local_keys) ? reflen_d : nullptr;
-            TileMap tm{nullptr, nullptr, 1, tiles_for(n_items), n_items, (uint32_t)kRsTile};
-            TileMap tm_small{nullptr, nullptr, 1, tiles_for(n_items, kRsTileSmall), n_items,
-                             (uint32_t)kRsTileSmall};
+            TileMap tm{nullptr, nullptr, 1, tiles_for(n_items), n_items};
             int keybits = nodebits + lenbits;
             if (local_keys && ns > 1) {
-                std::vector<uint32_t> toff(2 * (ns + 1), 0);  // big tiles, then small tiles
-                uint32_t* tb = toff.data();
-                uint32_t* ts = toff.data() + ns + 1;
+                std::vector<uint32_t> toff(ns + 1, 0);
                 uint32_t maxvn = 1;
                 for (uint32_t k = 0; k < ns; ++k) {
                     const uint64_t nk = foff_host[k + 1] - foff_host[k];
-                    tb[k + 1] = tb[k] + tiles_for(nk);
-                    ts[k + 1] = ts[k] + tiles_for(nk, kRsTileSmall);
+                    toff[k + 1] = toff[k] + tiles_for(nk);
                     maxvn = std::max(maxvn, rd->ref_len[k] + 1);
                 }
-                uint32_t* toff_d = c->tile_off_d.get<uint32_t>(2 * (ns + 1));
+                uint32_t* toff_d = c->tile_off_d.get<uint32_t>(ns + 1);
                 GDS_CUDA(cudaMemcpyAsync(toff_d, toff.data(), toff.size() * 4, cudaMemcpyHostToDevice, st));
-                tm = TileMap{toff_d, foff_dev, ns, tb[ns], n_items, (uint32_t)kRsTile};
-                tm_small = TileMap{toff_d + ns + 1, foff_dev, ns, ts[ns], n_items,
-                                   (uint32_t)kRsTileSmall};
+                tm = TileMap{toff_d, foff_dev, ns, toff[ns], n_items};
                 keybits = bits_for(maxvn - 1) + lenbits;
             }
             out->key_bits = keybits;
             if (keybits <= 32)
-                build_bundles<uint32_t>(c, S, E, vl, cross_idx, N, tm, tm_small, local_keys, n_nodes,
+                build_bundles<uint32_t>(c, S, E, vl, cross_idx, N, tm, local_keys, n_nodes,
                                         keybits, lenbits, minlen, odiff, fused_ref, stats, minlen,
                                         maxlen, B, sorted_idx, sort_passes);
             else
-                build_bundles<unsigned long long>(c, S, E, vl, cross_idx, N, tm, tm_small, local_keys,
+                build_bundles<unsigned long long>(c, S, E, vl, cross_idx, N, tm, local_keys,
                                                   n_nodes, keybits, lenbits, minlen, odiff,
                                                   fused_ref, stats, minlen, maxlen, B, sorted_idx,
                                                   sort_passes);
@@ -1336,9 +1286,8 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
         // with M = 100 (configs 1, 2, 5) the classic schedule on the uncut graph needs no more
         // rounds than hops, and the three extra passes over nodes and bundles would cost config 5
         // 0.25 ms of 5.75 (measured); gds_params.schedule = 2 applies them regardless.
-        bool forced_cuts = !(flags & GDS_NO_SOLVE) && algorithm == 0 && schedule != 1 &&
+        const bool forced_cuts = !(flags & GDS_NO_SOLVE) && algorithm == 0 && schedule != 1 &&
                            (schedule >= 2 || max_coverage >= kExpressMinSupply);
-        if (const char* e = getenv("GDS_EXPRESS")) forced_cuts = forced_cuts && atoi(e) != 0;
         int32_t* adj = nullptr;
         uint32_t* fmult = nullptr;
         uint8_t* dead = nullptr;  // nodes without a live bundle of their own (express rule U4)
@@ -1430,11 +1379,9 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
             uint32_t* tvB = c->tvB.get<uint32_t>(B);
             GDS_CUDA(cudaMemcpyAsync(tkA, c->b_t.as<uint32_t>(), (size_t)B * 4,
                                      cudaMemcpyDeviceToDevice, st));
-            TileMap btm{nullptr, nullptr, 1, tiles_for(B), B, (uint32_t)kRsTile};
-            TileMap btm_small{nullptr, nullptr, 1, tiles_for(B, kRsTileSmall), B,
-                              (uint32_t)kRsTileSmall};
-            int w = radix_sort_pairs<uint32_t>(tkA, tvA, tkB, tvB, btm, btm_small, nodebits, c->radix,
-                                               st, c->atomic_rank);
+            TileMap btm{nullptr, nullptr, 1, tiles_for(B), B};
+            int w = radix_sort_pairs<uint32_t>(tkA, tvA, tkB, tvB, btm, nodebits, c->radix, st,
+                                               c->atomic_rank);
             in_bid = w ? tvB : tvA;
         }
         if (!out_dev) {
@@ -1454,7 +1401,6 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
         // the express schedule (maxflow_sm.cuh): components with a supply of kExpressMinSupply or
         // more — none when M is below that, and then nothing about the launch changes
         uint32_t express_on = schedule == 1 ? 0u : schedule == 2 ? 2u : 1u;  // (3: the usual supply rule)
-        if (const char* e = getenv("GDS_EXPRESS")) express_on = (uint32_t)atoi(e);  // measurement knob
         if (!forced_cuts || (express_on == 1 && max_coverage < kExpressMinSupply)) express_on = 0;
         const bool express_possible = express_on != 0;
         const Mf2Plan mf2 = do_solve && algorithm == 0
@@ -1497,12 +1443,8 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
             uint32_t* wc = c->work_counter.get<uint32_t>(4);  // [0] sm kernel, [1] fallback, [2] list size
             GDS_CUDA(cudaMemsetAsync(wc, 0, 16, st));
             const unsigned long long mf_bytes = 36ull * n_nodes + 20ull * B;
-            // compact labels for k_maxflow's relabels (GDS_MF_GLABELS=0: node records, round 1)
-            uint16_t* lab_g = nullptr;
-            {
-                const char* e = getenv("GDS_MF_GLABELS");
-                if (!(e && e[0] == '0')) lab_g = c->lab_g.get<uint16_t>(2 * (size_t)n_nodes + 4);
-            }
+            // compact labels for k_maxflow's relabels
+            uint16_t* lab_g = c->lab_g.get<uint16_t>(2 * (size_t)n_nodes + 4);
             if (mf2.on) {
                 uint32_t* fb_list = c->fb_list.get<uint32_t>(n_comp_cap + 1);
                 Mf2Graph g2{node, c->bund.as<BundleRec>(), in_bid, in_src, out_ptr, in_ptr, dem_v,

@@ -117,12 +117,6 @@ struct ReadKeys {
         if (LOCAL) return (uint32_t)i;
         return i < n_reads ? (uint32_t)i : cross_idx[i - n_reads];
     }
-    // LOCAL keys with 32-bit K are eligible for the TMA-staged first pass (radix_sort.cuh)
-    static constexpr bool kTmaReads = LOCAL && sizeof(K) == 4;
-    const uint32_t* tma_a() const { return S; }
-    const uint32_t* tma_b() const { return E; }
-    int tma_lenbits() const { return lenbits; }
-    uint32_t tma_minlen() const { return minlen; }
 };
 
 // crossing reads -> ascending list of their indices (tile counts -> scan -> write)

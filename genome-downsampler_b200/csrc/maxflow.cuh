@@ -89,21 +89,16 @@ struct CompStats {
 
 // Record loads.  A component is owned by ONE CTA, i.e. one SM: plain (L1-allocating) loads are
 // coherent with the stores and atomics of the other threads of the CTA across __syncthreads, and
-// measured faster than L2-only loads (GDS_MF_LDCG=1 at build time selects the latter).
-#ifdef GDS_MF_LDCG
-#define GDS_MF_LD(p) __ldcg(p)
-#else
-#define GDS_MF_LD(p) (*(p))
-#endif
+// measured faster than L2-only loads (__ldcg).
 __device__ __forceinline__ void ld_node(const NodeRec* p, uint4& lo, uint4& hi) {
     const uint4* q = reinterpret_cast<const uint4*>(p);
-    lo = GDS_MF_LD(q);      // d, stamp, e, eadd
-    hi = GDS_MF_LD(q + 1);  // snk, g, out_ptr, in_ptr
+    lo = q[0];  // d, stamp, e, eadd
+    hi = q[1];  // snk, g, out_ptr, in_ptr
 }
 __device__ __forceinline__ uint4 ld_bundle(const BundleRec* p) {  // t, mult, f, s
-    return GDS_MF_LD(reinterpret_cast<const uint4*>(p));
+    return *reinterpret_cast<const uint4*>(p);
 }
-__device__ __forceinline__ uint32_t ld_u32(const uint32_t* p) { return GDS_MF_LD(p); }
+__device__ __forceinline__ uint32_t ld_u32(const uint32_t* p) { return *p; }
 
 template <uint32_t QCAP>
 struct Queue {
@@ -221,7 +216,7 @@ __device__ uint32_t mf_global_relabel(const MfGraph& G, uint32_t lo, uint32_t hi
             uint4 lo4, hi4;
             ld_node(&G.node[w], lo4, hi4);
             // CSR range ends live in the next record (w + 1 <= n_nodes: the sentinel exists)
-            const uint4 nx_hi = GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
+            const uint4 nx_hi = *(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
             if (w < hi) visit(w + 1);                              // back arc (w+1) -> w: residual
             if (w > lo && (int32_t)hi4.y > 0) visit(w - 1);        // reverse of back arc w -> w-1
             if ((nx_hi.w - hi4.w) + (nx_hi.z - hi4.z) > kHeavyDeg) {
@@ -243,8 +238,8 @@ __device__ uint32_t mf_global_relabel(const MfGraph& G, uint32_t lo, uint32_t hi
             const uint32_t lane = lane_id();
             for (uint32_t h = tid >> 5; h < nH; h += THREADS / 32) {
                 const uint32_t w = warp_mode ? T.get(h) : H.get(h);
-                const uint4 hi4 = GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[w]) + 1);
-                const uint4 nx_hi = GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
+                const uint4 hi4 = *(reinterpret_cast<const uint4*>(&G.node[w]) + 1);
+                const uint4 nx_hi = *(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
                 if (warp_mode && lane == 0) {  // the thread pass was skipped: neighbours here
                     if (w < hi) visit(w + 1);
                     if (w > lo && (int32_t)hi4.y > 0) visit(w - 1);
@@ -420,7 +415,7 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
           const uint32_t* __restrict__ comp_list_n,
           const uint32_t* __restrict__ n_comp_dev /* non-null: the component count lives on the device */,
           MfTotals* __restrict__ totals,
-          uint16_t* __restrict__ lab_g /* [2 * n_nodes + 2] or null: compact 16-bit labels in GLOBAL
+          uint16_t* __restrict__ lab_g /* [2 * n_nodes + 2]: compact 16-bit labels in GLOBAL
               memory for the relabel BFS of components whose labels get no shared memory — the BFS
               then claims 16 nodes per sector instead of one 32-byte record per node */) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -442,7 +437,7 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
         // global array (base 2*lo: 4-byte aligned, components never overlap)
         uint16_t* lab_base = lab_smem;
         uint32_t lcap = lab_cap;
-        if (ncomp > lcap && lab_g && ncomp < 0xfff0u) {
+        if (ncomp > lcap && ncomp < 0xfff0u) {
             lab_base = lab_g + 2 * (size_t)lo;
             lcap = 0xfff0u;
         }
@@ -532,7 +527,7 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
                 uint4 lo4, hi4, r_lo, r_hi;
                 ld_node(&G.node[v], lo4, hi4);
                 ld_node(&G.node[v + 1], r_lo, r_hi);  // neighbours' sectors come with the own one
-                const uint4 l_lo = v > lo ? GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[v - 1]))
+                const uint4 l_lo = v > lo ? *reinterpret_cast<const uint4*>(&G.node[v - 1])
                                           : make_uint4(kLabelInf, 0, 0, 0);  // d, stamp of v-1
                 const uint32_t dv = lo4.x;
                 G.d_snap[v] = dv;  // re-sync the snapshot of a node relabelled last round
@@ -618,7 +613,7 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
                     uint4 lo4, hi4, r_lo, r_hi;  // every lane loads the same sectors (broadcast)
                     ld_node(&G.node[v], lo4, hi4);
                     ld_node(&G.node[v + 1], r_lo, r_hi);
-                    const uint4 l_lo = v > lo ? GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[v - 1]))
+                    const uint4 l_lo = v > lo ? *reinterpret_cast<const uint4*>(&G.node[v - 1])
                                               : make_uint4(kLabelInf, 0, 0, 0);
                     const uint32_t dv = lo4.x;
                     if (warp_mode) {  // what the skipped thread pass does first
@@ -734,7 +729,7 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
                 const uint32_t dw = lo4.x;
                 bool frozen = dw >= kLabelInf;
                 if (in_front && left > 0 && !frozen) {
-                    const uint4 r_hi = GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
+                    const uint4 r_hi = *(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
                     if ((r_hi.z - hi4.z) + (r_hi.w - hi4.w) > kHeavyDeg) {
                         q_append(H, &sh.nH, w);  // the min over many bundles: warp pass below
                     } else {
@@ -774,8 +769,8 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
                 const uint32_t nH = sh.nH, lane = lane_id();
                 for (uint32_t h = tid >> 5; h < nH; h += THREADS / 32) {
                     const uint32_t w = H.get(h);
-                    const uint4 hi4 = GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[w]) + 1);
-                    const uint4 r_hi = GDS_MF_LD(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
+                    const uint4 hi4 = *(reinterpret_cast<const uint4*>(&G.node[w]) + 1);
+                    const uint4 r_hi = *(reinterpret_cast<const uint4*>(&G.node[w + 1]) + 1);
                     uint32_t mn = kLabelInf;
                     if ((int32_t)hi4.x > 0) mn = 0;
                     for (uint32_t b = hi4.z + lane; b < r_hi.z; b += 32) {

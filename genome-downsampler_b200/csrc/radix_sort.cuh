@@ -28,7 +28,6 @@ constexpr int kRsThreads = 512;
 constexpr int kRsWarps = kRsThreads / 32;
 constexpr int kRsItems = 16;
 constexpr int kRsTile = kRsThreads * kRsItems;  // 8192 keys per tile
-constexpr int kRsTileSmall = kRsTile / 2;
 
 // Where the tiles are.  n_groups == 1: items [0, n_items) in tiles of kRsTile.  Otherwise group g
 // owns items [item_off[g], item_off[g+1]) and tiles [tile_off[g], tile_off[g+1]).
@@ -38,7 +37,6 @@ struct TileMap {
     uint32_t n_groups;
     uint32_t n_tiles;
     size_t n_items;
-    uint32_t tile;  // items per tile: kRsTile, or kRsTileSmall for the two-CTA TMA scatter
 };
 
 struct TilePos {
@@ -54,8 +52,8 @@ struct TilePos {
 __device__ __forceinline__ TilePos locate_tile(const TileMap& tm, uint32_t tile) {
     TilePos p;
     if (tm.n_groups == 1) {
-        p.first = (size_t)tile * tm.tile;
-        p.n_valid = (uint32_t)min((size_t)tm.tile, tm.n_items - p.first);
+        p.first = (size_t)tile * kRsTile;
+        p.n_valid = (uint32_t)min((size_t)kRsTile, tm.n_items - p.first);
         p.hist_base = 0;
         p.tiles_g = tm.n_tiles;
         p.tile_in_g = tile;
@@ -72,8 +70,8 @@ __device__ __forceinline__ TilePos locate_tile(const TileMap& tm, uint32_t tile)
     const uint64_t i0 = tm.item_off[lo], i1 = tm.item_off[lo + 1];
     p.tile_in_g = tile - t0;
     p.tiles_g = tm.tile_off[lo + 1] - t0;
-    p.first = (size_t)i0 + (size_t)p.tile_in_g * tm.tile;
-    p.n_valid = (uint32_t)min((uint64_t)tm.tile, i1 - p.first);
+    p.first = (size_t)i0 + (size_t)p.tile_in_g * kRsTile;
+    p.n_valid = (uint32_t)min((uint64_t)kRsTile, i1 - p.first);
     p.hist_base = 256u * t0;
     p.group = lo;
     return p;
@@ -94,15 +92,9 @@ struct ArrayKeys {
     __device__ __forceinline__ bool checks() const { return false; }
     __device__ __forceinline__ uint32_t check(Raw, uint32_t) const { return 0; }
     __device__ __forceinline__ uint32_t* check_stats() const { return nullptr; }
-    // not a (start, end) source: the TMA first-pass kernel does not apply
-    static constexpr bool kTmaReads = false;
-    const uint32_t* tma_a() const { return nullptr; }
-    const uint32_t* tma_b() const { return nullptr; }
-    int tma_lenbits() const { return 0; }
-    uint32_t tma_minlen() const { return 0; }
 };
 
-template <typename K, typename KS, int ITEMS>
+template <typename K, typename KS>
 __global__ void __launch_bounds__(kRsThreads)
 k_rs_hist(KS ks, TileMap tm, int shift, uint32_t* __restrict__ tile_hist) {
     __shared__ uint32_t h[kRsWarps][256];  // per-warp counts: conflicts only inside a warp
@@ -110,16 +102,16 @@ k_rs_hist(KS ks, TileMap tm, int shift, uint32_t* __restrict__ tile_hist) {
     const TilePos tp = locate_tile(tm, blockIdx.x);
     __syncthreads();
     const uint32_t warp = threadIdx.x >> 5;
-    typename KS::Raw raw[ITEMS];
+    typename KS::Raw raw[kRsItems];
 #pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
+    for (int k = 0; k < kRsItems; ++k) {
         uint32_t j = (uint32_t)k * kRsThreads + threadIdx.x;
         // out-of-range lanes re-read the tile's first item: the load stays unconditional
         raw[k] = ks.load(tp.first + (j < tp.n_valid ? j : 0u));
     }
     uint32_t bad = 0;  // input validation fused into the first pass (low half: range, high: hints)
 #pragma unroll
-    for (int k = 0; k < ITEMS; ++k) {
+    for (int k = 0; k < kRsItems; ++k) {
         uint32_t j = (uint32_t)k * kRsThreads + threadIdx.x;
         // lanes past the tile's end get the first item's index too: make() may index side arrays
         // (the crossing-read list of the global key source) with it
@@ -250,9 +242,9 @@ k_rs_scatter(KS ks, const uint32_t* __restrict__ vals_in, K* __restrict__ keys_o
         sm.gbase[threadIdx.x] = tile_off_scanned[(size_t)tp.hist_base +
                                                  (size_t)threadIdx.x * tp.tiles_g + tp.tile_in_g];
 
-    // warp w owns the contiguous chunk [w*32*ITEMS, (w+1)*32*ITEMS) of the tile; row k covers 32
-    // consecutive keys, so (warp, row, lane) order == input order.  Loads are batched 8 rows at a
-    // time (register budget) and never predicated: short tiles re-read their first item.
+    // warp w owns the contiguous chunk [w*32*kRsItems, (w+1)*32*kRsItems) of the tile; row k
+    // covers 32 consecutive keys, so (warp, row, lane) order == input order.  Loads are batched 8
+    // rows at a time (register budget) and never predicated: short tiles re-read their first item.
     const uint32_t wofs = warp * 32 * kRsItems + lane;
     const bool full = tp.n_valid == (uint32_t)kRsTile;
     const size_t gfirst = tp.first + wofs;
@@ -374,290 +366,17 @@ k_rs_scatter(KS ks, const uint32_t* __restrict__ vals_in, K* __restrict__ keys_o
     }
 }
 
-// ------------------------------------------------------------------------------------------
-// Persistent scatter with TMA-staged input (32-bit keys).  The per-tile scatter above is bound by
-// memory-level parallelism: each CTA exposes four dependent DRAM round trips per tile and only
-// ~32 KB are in flight per SM.  Here one CTA per SM walks its tiles; thread 0 prefetches the NEXT
-// tile's two input arrays into shared memory with 1-D bulk copies (cp.async.bulk, completion on an
-// mbarrier) while all warps rank / reorder / write the current tile out of registers, so a full
-// tile (64 KB) is always in flight without holding registers.
-//   MODE 0: A = keys, B = values          (later passes)
-//   MODE 1: A = keys, value = item index   (first pass over an existing key array)
-//   MODE 2: A = start, B = end of the reads; key = (start << lenbits) | (len - minlen),
-//           value = item index             (first pass of the arc sort, LOCAL keys)
-constexpr int kRpRows = 8;  // items per thread
-
-template <int THREADS>
-struct RpSmem {
-    static constexpr int kTile = THREADS * kRpRows;
-    uint32_t stA[kTile + 8];  // + slack for 16-byte source alignment
-    uint32_t stB[kTile + 8];
-    uint32_t skey[kTile];
-    uint32_t sval[kTile];
-    uint32_t wh[THREADS / 32][128];  // two 16-bit counters per word: digits 2p (low), 2p+1 (high)
-    uint32_t gbase[256];
-    uint32_t wsum[4];
-    unsigned long long mbar;
-};
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-    return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
-                 "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, uint32_t bytes,
-                                            unsigned long long* bar) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-            "r"(smem_u32(dst)),
-        "l"(src), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra LAB_DONE;\n"
-        "bra LAB_WAIT;\n"
-        "LAB_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-
-// element offset that makes (ptr + first - off) 16-byte aligned, and the byte count to copy
-__device__ __forceinline__ uint32_t tma_align(const uint32_t* ptr, size_t first, uint32_t n,
-                                              uint32_t& bytes) {
-    uint32_t off = (uint32_t)((reinterpret_cast<uintptr_t>(ptr + first) & 15u) >> 2);
-    bytes = ((off + n) * 4u + 15u) & ~15u;
-    return off;
-}
-
-template <int MODE, int THREADS, int MIN_CTAS, bool ATOMIC_RANK>
-__global__ void __launch_bounds__(THREADS, MIN_CTAS)
-k_rs_scatter_tma(const uint32_t* __restrict__ inA, const uint32_t* __restrict__ inB,
-                 uint32_t* __restrict__ keys_out, uint32_t* __restrict__ vals_out, TileMap tm,
-                 int shift, int nbits, const uint32_t* __restrict__ tile_off_scanned, int lenbits,
-                 uint32_t minlen) {
-    extern __shared__ __align__(128) unsigned char rp_smem_raw[];
-    constexpr int kRpThreads = THREADS;
-    constexpr int kRpWarps = THREADS / 32;
-    constexpr int kTile = THREADS * kRpRows;
-    RpSmem<THREADS>& sm = *reinterpret_cast<RpSmem<THREADS>*>(rp_smem_raw);
-    const uint32_t tid = threadIdx.x, warp = tid >> 5, lane = lane_id();
-    constexpr bool kHasB = MODE != 1;
-
-    if (tid == 0) mbar_init(&sm.mbar, 1);
-    __syncthreads();
-
-    uint32_t tile = blockIdx.x;
-    if (tile >= tm.n_tiles) return;
-    TilePos tp = locate_tile(tm, tile);
-    uint32_t bytesA = 0, bytesB = 0;
-    uint32_t offA = tma_align(inA, tp.first, tp.n_valid, bytesA);
-    uint32_t offB = kHasB ? tma_align(inB, tp.first, tp.n_valid, bytesB) : 0;
-    if (tid == 0) {
-        mbar_expect_tx(&sm.mbar, bytesA + bytesB);
-        tma_load_1d(sm.stA, inA + tp.first - offA, bytesA, &sm.mbar);
-        if (kHasB) tma_load_1d(sm.stB, inB + tp.first - offB, bytesB, &sm.mbar);
-    }
-    uint32_t g_cur = 0;
-    if (tid < 256)
-        g_cur = tile_off_scanned[(size_t)tp.hist_base + (size_t)tid * tp.tiles_g + tp.tile_in_g];
-    const uint32_t wofs = warp * 32 * kRpRows + lane;
-    uint32_t parity = 0;
-
-    for (;;) {
-        // ---- phase A: the staged tile -> registers; counters cleared
-        for (int i = tid; i < kRpWarps * 128; i += kRpThreads) (&sm.wh[0][0])[i] = 0;
-        if (tid < 256) sm.gbase[tid] = g_cur;
-        mbar_wait(&sm.mbar, parity);
-        parity ^= 1;
-        const bool full = tp.n_valid == (uint32_t)kTile;
-        uint32_t key[kRpRows], val[kRpRows];
-#pragma unroll
-        for (int k = 0; k < kRpRows; ++k) {
-            const uint32_t j = wofs + (uint32_t)k * 32;
-            const uint32_t a = sm.stA[offA + j];
-            const uint32_t b = kHasB ? sm.stB[offB + j] : 0u;
-            if (MODE == 2) {
-                key[k] = (a << lenbits) | (b - a + 1 - minlen);
-                val[k] = (uint32_t)(tp.first + j);
-            } else if (MODE == 1) {
-                key[k] = a;
-                val[k] = (uint32_t)(tp.first + j);
-            } else {
-                key[k] = a;
-                val[k] = b;
-            }
-        }
-        __syncthreads();  // S1: stage consumed, counters cleared
-
-        // ---- prefetch the next tile into the (now free) stage
-        const uint32_t next = tile + gridDim.x;
-        const bool has_next = next < tm.n_tiles;
-        const TilePos tp_cur = tp;
-        uint32_t offA_n = 0, offB_n = 0;
-        if (has_next) {
-            tp = locate_tile(tm, next);
-            offA_n = tma_align(inA, tp.first, tp.n_valid, bytesA);
-            offB_n = kHasB ? tma_align(inB, tp.first, tp.n_valid, bytesB) : 0;
-            if (tid == 0) {
-                fence_proxy_async();
-                mbar_expect_tx(&sm.mbar, bytesA + bytesB);
-                tma_load_1d(sm.stA, inA + tp.first - offA_n, bytesA, &sm.mbar);
-                if (kHasB) tma_load_1d(sm.stB, inB + tp.first - offB_n, bytesB, &sm.mbar);
-            }
-            if (tid < 256)
-                g_cur = tile_off_scanned[(size_t)tp.hist_base + (size_t)tid * tp.tiles_g +
-                                         tp.tile_in_g];
-        }
-
-        // ---- stable ranks (ballot peers, one packed shared atomic per peer group)
-        uint32_t rank[kRpRows];
-        if (ATOMIC_RANK) {
-#pragma unroll
-            for (int k = 0; k < kRpRows; ++k) {
-                const uint32_t d = (key[k] >> shift) & 255u;
-                const uint32_t sh16 = (d & 1u) * 16u;
-                rank[k] = 0;
-                if (full || wofs + (uint32_t)k * 32 < tp_cur.n_valid)
-                    rank[k] = (atomicAdd(&sm.wh[warp][d >> 1], 1u << sh16) >> sh16) & 0xffffu;
-            }
-        } else {
-            uint32_t peers[kRpRows];
-#pragma unroll
-            for (int k = 0; k < kRpRows; ++k) {
-                const uint32_t d = (key[k] >> shift) & 255u;
-                const uint32_t vm =
-                    full ? 0xffffffffu
-                         : __ballot_sync(0xffffffffu, wofs + (uint32_t)k * 32 < tp_cur.n_valid);
-                peers[k] = match_digit(d, vm, nbits);
-            }
-#pragma unroll
-            for (int k = 0; k < kRpRows; ++k) {
-                const uint32_t d = (key[k] >> shift) & 255u;
-                const uint32_t sh16 = (d & 1u) * 16u;
-                const uint32_t before = __popc(peers[k] & lanemask_lt());
-                const bool valid = full || wofs + (uint32_t)k * 32 < tp_cur.n_valid;
-                uint32_t prev = 0;
-                if (valid && before == 0)
-                    prev = (atomicAdd(&sm.wh[warp][d >> 1], (uint32_t)__popc(peers[k]) << sh16) >>
-                            sh16) & 0xffffu;
-                prev = __shfl_sync(0xffffffffu, prev,
-                                   __ffs(peers[k] | (valid ? 0u : 1u << lane)) - 1);
-                rank[k] = prev + before;
-            }
-        }
-        __syncthreads();  // S2
-
-        // ---- first slot of every (warp, digit): 128 threads own a digit pair each
-        uint32_t tot0 = 0, tot1 = 0;
-        if (tid < 128) {
-#pragma unroll 8
-            for (int w = 0; w < kRpWarps; ++w) {
-                const uint32_t c = sm.wh[w][tid];
-                tot0 += c & 0xffffu;
-                tot1 += c >> 16;
-            }
-            const uint32_t both = tot0 + tot1;
-            const uint32_t incl = warp_incl_scan(both);
-            if (lane == 31) sm.wsum[warp] = incl;
-            tot1 = incl - both;  // warp-local exclusive start of the pair (reuse the register)
-        }
-        __syncthreads();  // S3
-        if (tid < 128) {
-            uint32_t run0 = tot1;
-#pragma unroll
-            for (int w = 0; w < 4; ++w) run0 += (w < (int)warp) ? sm.wsum[w] : 0u;
-            uint32_t run1 = run0 + tot0;
-            sm.gbase[2 * tid] -= run0;
-            sm.gbase[2 * tid + 1] -= run1;
-#pragma unroll 8
-            for (int w = 0; w < kRpWarps; ++w) {
-                const uint32_t c = sm.wh[w][tid];
-                sm.wh[w][tid] = run0 | (run1 << 16);
-                run0 += c & 0xffffu;
-                run1 += c >> 16;
-            }
-        }
-        __syncthreads();  // S4
-
-        // ---- reorder the tile by digit in shared memory
-#pragma unroll
-        for (int k = 0; k < kRpRows; ++k) {
-            if (full || wofs + (uint32_t)k * 32 < tp_cur.n_valid) {
-                const uint32_t d = (key[k] >> shift) & 255u;
-                const uint32_t p = ((sm.wh[warp][d >> 1] >> ((d & 1u) * 16u)) & 0xffffu) + rank[k];
-                sm.skey[p] = key[k];
-                sm.sval[p] = val[k];
-            }
-        }
-        __syncthreads();  // S5
-
-        // ---- every digit run goes out as one contiguous segment
-#pragma unroll 4
-        for (uint32_t j = tid; j < tp_cur.n_valid; j += kRpThreads) {
-            const uint32_t kk = sm.skey[j];
-            const uint32_t dst = sm.gbase[(kk >> shift) & 255u] + j;
-            keys_out[dst] = kk;
-            vals_out[dst] = sm.sval[j];
-        }
-        if (!has_next) break;
-        tile = next;
-        offA = offA_n;
-        offB = offB_n;
-        __syncthreads();  // S6: skey/sval/wh/gbase free again
-    }
-}
-
 struct RadixTemp {
     DevBuf hist;
     ScanTemp scan;
 };
 
-inline uint32_t tiles_for(size_t n, uint32_t tile = kRsTile) {
-    return (uint32_t)((n + tile - 1) / tile);
-}
+inline uint32_t tiles_for(size_t n) { return (uint32_t)((n + kRsTile - 1) / kRsTile); }
 
-// One scatter launch of the TMA-staged kernel in the shape the tile size asks for:
-// kRsTile -> 1024 threads x 1 CTA/SM, kRsTileSmall -> 512 threads x 2 CTAs/SM.
-template <int MODE>
-inline void launch_scatter_tma(const TileMap& tm, const uint32_t* a, const uint32_t* b,
-                               uint32_t* kout, uint32_t* vout, int shift, int nbits,
-                               const uint32_t* hist, int lenbits, uint32_t minlen, bool atomic_rank,
-                               cudaStream_t st) {
-    auto go = [&](auto kern, int threads, int smem, uint32_t per_sm) {
-        GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        int grid = (int)std::min<uint32_t>(tm.n_tiles, per_sm * (uint32_t)kNumSMs);
-        kern<<<grid, threads, smem, st>>>(a, b, kout, vout, tm, shift, nbits, hist, lenbits, minlen);
-    };
-    if (tm.tile == (uint32_t)kRsTile) {
-        if (atomic_rank) go(k_rs_scatter_tma<MODE, 1024, 1, true>, 1024, (int)sizeof(RpSmem<1024>), 1);
-        else go(k_rs_scatter_tma<MODE, 1024, 1, false>, 1024, (int)sizeof(RpSmem<1024>), 1);
-    } else {
-        if (atomic_rank) go(k_rs_scatter_tma<MODE, 512, 2, true>, 512, (int)sizeof(RpSmem<512>), 2);
-        else go(k_rs_scatter_tma<MODE, 512, 2, false>, 512, (int)sizeof(RpSmem<512>), 2);
-    }
-}
-
-// One scatter launch of the register-staged kernel.
 template <typename K, typename KS>
-inline void launch_scatter_reg(const KS& ks, const uint32_t* vals_in, K* kout, uint32_t* vout,
-                               const TileMap& t, int shift, int nbits, const uint32_t* hist,
-                               bool atomic_rank, cudaStream_t st) {
+inline void launch_scatter(const KS& ks, const uint32_t* vals_in, K* kout, uint32_t* vout,
+                           const TileMap& t, int shift, int nbits, const uint32_t* hist,
+                           bool atomic_rank, cudaStream_t st) {
     constexpr int kMinCtas = sizeof(K) == 4 ? 2 : 1;
     constexpr int smem = (int)sizeof(RsSmem<K>);
     auto go = [&](auto kern) {
@@ -673,42 +392,20 @@ inline void launch_scatter_reg(const KS& ks, const uint32_t* vals_in, K* kout, u
     }
 }
 
-template <typename K, typename KS>
-inline void launch_hist(const KS& ks, const TileMap& tm, int shift, uint32_t* hist, cudaStream_t st) {
-    if (tm.tile == (uint32_t)kRsTile)
-        k_rs_hist<K, KS, kRsItems><<<tm.n_tiles, kRsThreads, 0, st>>>(ks, tm, shift, hist);
-    else
-        k_rs_hist<K, KS, kRsItems / 2><<<tm.n_tiles, kRsThreads, 0, st>>>(ks, tm, shift, hist);
-}
-
-// Sorts the pairs by the low `bits` bits of the key inside every group.  `tm` tiles the items in
-// kRsTile, `tm_small` (same groups) in kRsTileSmall.  Buffers ping-pong; returns 0 if the result
-// is in (keys_a, vals_a), 1 if in (keys_b, vals_b).  The first pass takes key and value from
-// *first_ks when it is non-null, else from keys_a with value = item index.
-//
-// Which scatter kernel runs which pass was chosen by measurement on B200 (profiles/):
-//   'R' register-staged, 2 CTAs x 512 threads, tile 8192   — fastest for every pass (default)
-//   '1' TMA-staged persistent, 1 CTA x 1024 threads, tile 8192
-//   '2' TMA-staged persistent, 2 CTAs x 512 threads, tile 4096
-// GDS_SORT_MODE=<first><later> overrides (experiments); 64-bit keys always use 'R'.
+// Sorts the pairs by the low `bits` bits of the key inside every group.  Buffers ping-pong; returns
+// 0 if the result is in (keys_a, vals_a), 1 if in (keys_b, vals_b).  The first pass takes key and
+// value from *first_ks when it is non-null, else from keys_a with value = item index.
 template <typename K, typename KS0 = ArrayKeys<K>>
 inline int radix_sort_pairs(K* keys_a, uint32_t* vals_a, K* keys_b, uint32_t* vals_b,
-                            const TileMap& tm, const TileMap& tm_small, int bits, RadixTemp& tmp,
-                            cudaStream_t st, bool atomic_rank, int* passes_out = nullptr,
+                            const TileMap& tm, int bits, RadixTemp& tmp, cudaStream_t st,
+                            bool atomic_rank, int* passes_out = nullptr,
                             const KS0* first_ks = nullptr) {
     int passes = (bits + 7) / 8;
     if (passes == 0) passes = 1;  // still need vals materialised
     if (passes_out) *passes_out = passes;
     const size_t n = tm.n_items;
     if (n == 0 || tm.n_tiles == 0) return 0;
-    uint32_t* hist = tmp.hist.get<uint32_t>((size_t)256 * std::max(tm.n_tiles, tm_small.n_tiles));
-    static const char* mode_env = getenv("GDS_SORT_MODE");
-    char first_mode = 'R', later_mode = 'R';
-    if (mode_env && mode_env[0] && mode_env[1]) {
-        first_mode = mode_env[0];
-        later_mode = mode_env[1];
-    }
-    if (sizeof(K) != 4) first_mode = later_mode = 'R';
+    uint32_t* hist = tmp.hist.get<uint32_t>((size_t)256 * tm.n_tiles);
     int cur = 0;
     for (int p = 0; p < passes; ++p) {
         K* kin = cur ? keys_b : keys_a;
@@ -718,50 +415,31 @@ inline int radix_sort_pairs(K* keys_a, uint32_t* vals_a, K* keys_b, uint32_t* va
         int shift = 8 * p;
         const int nbits = std::max(1, std::min(8, bits - shift));  // significant digit bits
         if (p == 0 && first_ks) {
-            const char m = KS0::kTmaReads ? first_mode : 'R';
-            const TileMap& t = m == '2' ? tm_small : tm;
             {
                 KScope ks("rs_hist_reads", 8ull * n, st);
-                launch_hist<K, KS0>(*first_ks, t, shift, hist, st);
+                k_rs_hist<K, KS0><<<tm.n_tiles, kRsThreads, 0, st>>>(*first_ks, tm, shift, hist);
                 GDS_KERNEL_CHECK();
             }
-            exclusive_scan_u32(hist, hist, (size_t)256 * t.n_tiles, tmp.scan, st);
+            exclusive_scan_u32(hist, hist, (size_t)256 * tm.n_tiles, tmp.scan, st);
             {
                 KScope ks("rs_scatter_reads", (8ull + sizeof(K) + 4) * n, st);
-                if (m == 'R')
-                    launch_scatter_reg<K, KS0>(*first_ks, nullptr, kout, vout, t, shift, nbits, hist,
-                                               atomic_rank, st);
-                else
-                    launch_scatter_tma<2>(t, first_ks->tma_a(), first_ks->tma_b(),
-                                          reinterpret_cast<uint32_t*>(kout), vout, shift, nbits, hist,
-                                          first_ks->tma_lenbits(), first_ks->tma_minlen(),
-                                          atomic_rank, st);
+                launch_scatter<K, KS0>(*first_ks, nullptr, kout, vout, tm, shift, nbits, hist,
+                                       atomic_rank, st);
                 GDS_KERNEL_CHECK();
             }
         } else {
             ArrayKeys<K> ak{kin};
             const uint32_t* vsrc = p == 0 ? nullptr : vin;
-            const char m = p == 0 ? first_mode : later_mode;
-            const TileMap& t = m == '2' ? tm_small : tm;
             {
                 KScope ks("rs_hist", sizeof(K) * (unsigned long long)n, st);
-                launch_hist<K, ArrayKeys<K>>(ak, t, shift, hist, st);
+                k_rs_hist<K, ArrayKeys<K>><<<tm.n_tiles, kRsThreads, 0, st>>>(ak, tm, shift, hist);
                 GDS_KERNEL_CHECK();
             }
-            exclusive_scan_u32(hist, hist, (size_t)256 * t.n_tiles, tmp.scan, st);
+            exclusive_scan_u32(hist, hist, (size_t)256 * tm.n_tiles, tmp.scan, st);
             {
                 KScope ks("rs_scatter", (2ull * sizeof(K) + (vsrc ? 8 : 4)) * n, st);
-                if (m != 'R' && vsrc)
-                    launch_scatter_tma<0>(t, reinterpret_cast<const uint32_t*>(kin), vsrc,
-                                          reinterpret_cast<uint32_t*>(kout), vout, shift, nbits, hist,
-                                          0, 0, atomic_rank, st);
-                else if (m != 'R')
-                    launch_scatter_tma<1>(t, reinterpret_cast<const uint32_t*>(kin), nullptr,
-                                          reinterpret_cast<uint32_t*>(kout), vout, shift, nbits, hist,
-                                          0, 0, atomic_rank, st);
-                else
-                    launch_scatter_reg<K, ArrayKeys<K>>(ak, vsrc, kout, vout, t, shift, nbits, hist,
-                                                        atomic_rank, st);
+                launch_scatter<K, ArrayKeys<K>>(ak, vsrc, kout, vout, tm, shift, nbits, hist,
+                                                atomic_rank, st);
                 GDS_KERNEL_CHECK();
             }
         }

@@ -1,8 +1,8 @@
 // scan.cuh — device-wide exclusive prefix sum over uint32 (wrap-around add, so it also serves
 // int32 difference arrays).  One pass with decoupled look-back (each tile publishes its aggregate,
 // then its inclusive prefix, in one 64-bit status word; a tile's first warp walks back over its
-// predecessors' words): the data is read once and written once, 8 bytes per element, where the
-// hierarchical reduce-then-scan below it (kept for one-tile inputs and as GDS_SCAN=hier) moves 16.
+// predecessors' words): the data is read once and written once, 8 bytes per element.  Inputs of
+// one k_scan_tiles tile or less are scanned by a single block.
 // Integer addition is associative, so the result does not depend on which tiles were ready when.
 #pragma once
 #include "common.cuh"
@@ -42,11 +42,11 @@ __device__ __forceinline__ uint32_t block_excl_scan(uint32_t v, uint32_t* total)
     return r;
 }
 
+// n <= kScanTile, one block
 __global__ void __launch_bounds__(kScanThreads)
-k_scan_tiles(const uint32_t* in, uint32_t* out /* may alias in: in-place scans */,
-             uint32_t* __restrict__ tile_sums, size_t n) {
+k_scan_tiles(const uint32_t* in, uint32_t* out /* may alias in: in-place scans */, size_t n) {
     __shared__ uint32_t total;
-    size_t base = (size_t)blockIdx.x * kScanTile + (size_t)threadIdx.x * kScanItems;
+    const size_t base = (size_t)threadIdx.x * kScanItems;
     uint32_t v[kScanItems];
     uint32_t s = 0;
 #pragma unroll
@@ -60,16 +60,6 @@ k_scan_tiles(const uint32_t* in, uint32_t* out /* may alias in: in-place scans *
         if (base + k < n) out[base + k] = ex;
         ex += v[k];
     }
-    if (threadIdx.x == 0 && tile_sums) tile_sums[blockIdx.x] = total;
-}
-
-__global__ void __launch_bounds__(kScanThreads)
-k_scan_add(uint32_t* __restrict__ out, const uint32_t* __restrict__ tile_offs, size_t n) {
-    uint32_t off = tile_offs[blockIdx.x];
-    size_t base = (size_t)blockIdx.x * kScanTile + (size_t)threadIdx.x * kScanItems;
-#pragma unroll
-    for (int k = 0; k < kScanItems; ++k)
-        if (base + k < n) out[base + k] += off;
 }
 
 // Up to three equally long arrays scanned by one launch (the node arrays of the graph build).
@@ -236,30 +226,23 @@ k_scan_lookback(ScanArrays a, uint32_t n_arr, size_t n, uint32_t n_tiles,
 }
 
 struct ScanTemp {
-    DevBuf l1, l2;
     DevBuf status, ticket;
     size_t status_cap = 0;
     uint32_t epoch = 0;
-    int mode = -1;  // 0 = one pass, 1 = hierarchical (GDS_SCAN=hier: measurement knob)
 };
 
-inline void exclusive_scan_u32(const uint32_t* in, uint32_t* out, size_t n, ScanTemp& tmp,
-                               cudaStream_t st);
+inline void scan_one_tile(const uint32_t* in, uint32_t* out, size_t n, cudaStream_t st) {
+    KScope ks("scan_u32", 8ull * n, st);
+    k_scan_tiles<<<1, kScanThreads, 0, st>>>(in, out, n);
+    GDS_KERNEL_CHECK();
+}
 
-// k equally long arrays in one launch; falls back to one hierarchical scan each for short arrays
+// k equally long arrays in one launch; arrays of one tile are scanned one by one
 inline void exclusive_scan_u32_multi(const ScanArrays& a, int n_arr, size_t n, ScanTemp& tmp,
                                      cudaStream_t st) {
     if (n == 0 || n_arr <= 0) return;
-    if (tmp.mode < 0) {
-        const char* e = getenv("GDS_SCAN");
-        tmp.mode = (e && e[0] == 'h') ? 1 : 0;
-    }
-    const size_t t1 = (n + kScanTile - 1) / kScanTile;
-    if (t1 == 1 || tmp.mode == 1 || t1 * n_arr > 0x7fffffffull) {
-        const int keep = tmp.mode;
-        tmp.mode = 1;
-        for (int k = 0; k < n_arr; ++k) exclusive_scan_u32(a.in[k], a.out[k], n, tmp, st);
-        tmp.mode = keep;
+    if (n <= (size_t)kScanTile) {
+        for (int k = 0; k < n_arr; ++k) scan_one_tile(a.in[k], a.out[k], n, st);
         return;
     }
     KScope ks("scan_u32", 8ull * n * n_arr, st);
@@ -278,42 +261,12 @@ inline void exclusive_scan_u32_multi(const ScanArrays& a, int n_arr, size_t n, S
     GDS_KERNEL_CHECK();
 }
 
-// out may alias in.  total (optional, device pointer) receives nothing here: callers that need
-// the grand total read out[n-1] + in[n-1] themselves or scan n+1 elements with a trailing zero.
+// out may alias in.  Callers that need the grand total read out[n-1] + in[n-1] themselves or scan
+// n+1 elements with a trailing zero.
 inline void exclusive_scan_u32(const uint32_t* in, uint32_t* out, size_t n, ScanTemp& tmp,
                                cudaStream_t st) {
-    if (n == 0) return;
-    size_t t1 = (n + kScanTile - 1) / kScanTile;
-    if (t1 > 1 && tmp.mode != 1) {
-        ScanArrays a{{in, nullptr, nullptr}, {out, nullptr, nullptr}};
-        exclusive_scan_u32_multi(a, 1, n, tmp, st);
-        return;
-    }
-    KScope ks("scan_u32", 8ull * n, st);  // the whole hierarchical scan counts as one unit
-    if (t1 == 1) {
-        k_scan_tiles<<<1, kScanThreads, 0, st>>>(in, out, nullptr, n);
-        GDS_KERNEL_CHECK();
-        return;
-    }
-    uint32_t* s1 = tmp.l1.get<uint32_t>(t1);
-    k_scan_tiles<<<(unsigned)t1, kScanThreads, 0, st>>>(in, out, s1, n);
-    GDS_KERNEL_CHECK();
-    size_t t2 = (t1 + kScanTile - 1) / kScanTile;
-    if (t2 == 1) {
-        k_scan_tiles<<<1, kScanThreads, 0, st>>>(s1, s1, nullptr, t1);
-        GDS_KERNEL_CHECK();
-    } else {
-        uint32_t* s2 = tmp.l2.get<uint32_t>(t2);
-        k_scan_tiles<<<(unsigned)t2, kScanThreads, 0, st>>>(s1, s1, s2, t1);
-        GDS_KERNEL_CHECK();
-        // t2 <= 4096 for n <= 2^36
-        k_scan_tiles<<<1, kScanThreads, 0, st>>>(s2, s2, nullptr, t2);
-        GDS_KERNEL_CHECK();
-        k_scan_add<<<(unsigned)t2, kScanThreads, 0, st>>>(s1, s2, t1);
-        GDS_KERNEL_CHECK();
-    }
-    k_scan_add<<<(unsigned)t1, kScanThreads, 0, st>>>(out, s1, n);
-    GDS_KERNEL_CHECK();
+    ScanArrays a{{in, nullptr, nullptr}, {out, nullptr, nullptr}};
+    exclusive_scan_u32_multi(a, 1, n, tmp, st);
 }
 
 }  // namespace gds

@@ -13,7 +13,7 @@ timeout 900 python bench.py --impl reference > $O/${T}_BENCH_reference.json 2> $
 for w in c4 c1 c2 ref_uniform ref_low_sides ref_hole ref_zero_sides; do
   timeout 600 python bench.py --workload $w --no-cpu-baseline > $O/${T}_bench_$w.json 2> $O/${T}_bench_$w.err; echo "$w rc=$?"
 done
-GDS_EXPRESS=0 timeout 600 python bench.py --workload c4 --no-cpu-baseline > $O/${T}_bench_c4_classic.json 2>/dev/null; echo "c4 classic rc=$?"
+timeout 600 python bench.py --workload c4 --schedule 1 --no-cpu-baseline > $O/${T}_bench_c4_classic.json 2>/dev/null; echo "c4 classic rc=$?"
 for w in c1 c4; do
   timeout 600 python bench.py --workload $w --algorithm mcp --no-cpu-baseline > $O/${T}_bench_mcp_$w.json 2> $O/${T}_bench_mcp_$w.err; echo "mcp $w rc=$?"
 done
