@@ -6,6 +6,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace gds {
@@ -26,21 +27,15 @@ struct CudaFail {
         if (_e != cudaSuccess) throw gds::CudaFail{_e, #call, __FILE__, __LINE__}; \
     } while (0)
 
-// follows every kernel launch: checks the launch and counts it (gds_result.kernel_launches)
-#define GDS_KERNEL_CHECK()            \
-    do {                              \
-        gds::count_launch();          \
-        GDS_CUDA(cudaGetLastError()); \
-    } while (0)
+// kernels this thread has launched; gds_result.kernel_launches is its growth over one call
 inline unsigned long long& launch_counter() {
     static thread_local unsigned long long n = 0;
     return n;
 }
-inline void count_launch() { ++launch_counter(); }
 
-// Per-launch accounting.  Every kernel launch sits inside a KScope: it always counts the launch
-// and, when profiling is on (GDS_PROFILE_KERNELS), brackets it with CUDA events on the launching
-// stream so bench.py can report per-kernel time and achieved bytes/s measured live.
+// Per-launch accounting.  When profiling is on (GDS_PROFILE_KERNELS), a KScope brackets a launch
+// with CUDA events on the launching stream so bench.py can report per-kernel time and achieved
+// bytes/s measured live.  launch() opens it and counts the launch.
 struct KRec {
     const char* name;
     unsigned long long bytes;
@@ -48,7 +43,6 @@ struct KRec {
 };
 struct Profiler {
     bool on = false;
-    unsigned long long launches = 0;
     std::vector<KRec> recs;
     std::vector<cudaEvent_t> pool;
     size_t used = 0;
@@ -63,7 +57,6 @@ struct Profiler {
     void reset() {
         recs.clear();
         used = 0;
-        launches = 0;
     }
     void release() {
         for (cudaEvent_t e : pool) cudaEventDestroy(e);
@@ -91,6 +84,17 @@ struct KScope {
         if (e1) cudaEventRecord(e1, st);
     }
 };
+
+// Every kernel launch of the solve path: profiled under `name` with its algorithmic `bytes`, counted
+// (gds_result.kernel_launches) and checked.
+template <typename... Params, typename... Args>
+inline void launch(const char* name, unsigned long long bytes, void (*kernel)(Params...), dim3 grid,
+                   dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+    KScope ks(name, bytes, st);
+    kernel<<<grid, block, smem, st>>>(std::forward<Args>(args)...);
+    ++launch_counter();
+    GDS_CUDA(cudaGetLastError());
+}
 
 // Grow-only device buffer (arena slot).  Reused across gds_solve calls, freed with its owner.
 struct DevBuf {

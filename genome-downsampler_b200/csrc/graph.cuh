@@ -463,8 +463,9 @@ k_uncapped_flags(const uint32_t* __restrict__ excl, const int32_t* __restrict__ 
 
 // One thread per NODE: if no uncapped position lies within maxlen of v none of its bundles can be
 // forced — two reads of the prefix count and nothing else (config 4: all but the genome's two ends).
-// Otherwise its out-bundles are tested one by one.  fmult[b] is written for forced bundles only and
-// read back, after K3, by the same test: it needs no clearing.
+// Otherwise its out-bundles are tested one by one.  fmult[b] is written for every bundle of such a
+// node (0 when the bundle is not forced) and read back, after K3, by the same test: it needs no
+// clearing.
 __device__ __forceinline__ bool node_may_be_forced(const uint32_t* __restrict__ unc, uint32_t v,
                                                    uint32_t n_nodes, uint32_t maxlen) {
     return unc[v] != unc[min(v + maxlen, n_nodes)];

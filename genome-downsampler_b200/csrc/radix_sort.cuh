@@ -374,14 +374,16 @@ struct RadixTemp {
 inline uint32_t tiles_for(size_t n) { return (uint32_t)((n + kRsTile - 1) / kRsTile); }
 
 template <typename K, typename KS>
-inline void launch_scatter(const KS& ks, const uint32_t* vals_in, K* kout, uint32_t* vout,
-                           const TileMap& t, int shift, int nbits, const uint32_t* hist,
-                           bool atomic_rank, cudaStream_t st) {
+inline void launch_scatter(const char* name, unsigned long long bytes, const KS& ks,
+                           const uint32_t* vals_in, K* kout, uint32_t* vout, const TileMap& t,
+                           int shift, int nbits, const uint32_t* hist, bool atomic_rank,
+                           cudaStream_t st) {
     constexpr int kMinCtas = sizeof(K) == 4 ? 2 : 1;
     constexpr int smem = (int)sizeof(RsSmem<K>);
     auto go = [&](auto kern) {
         GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        kern<<<t.n_tiles, kRsThreads, smem, st>>>(ks, vals_in, kout, vout, t, shift, nbits, hist);
+        launch(name, bytes, kern, t.n_tiles, kRsThreads, smem, st, ks, vals_in, kout, vout, t, shift,
+               nbits, hist);
     };
     if (vals_in) {
         if (atomic_rank) go(k_rs_scatter<K, KS, true, true, kMinCtas>);
@@ -415,33 +417,19 @@ inline int radix_sort_pairs(K* keys_a, uint32_t* vals_a, K* keys_b, uint32_t* va
         int shift = 8 * p;
         const int nbits = std::max(1, std::min(8, bits - shift));  // significant digit bits
         if (p == 0 && first_ks) {
-            {
-                KScope ks("rs_hist_reads", 8ull * n, st);
-                k_rs_hist<K, KS0><<<tm.n_tiles, kRsThreads, 0, st>>>(*first_ks, tm, shift, hist);
-                GDS_KERNEL_CHECK();
-            }
+            launch("rs_hist_reads", 8ull * n, k_rs_hist<K, KS0>, tm.n_tiles, kRsThreads, 0, st,
+                   *first_ks, tm, shift, hist);
             exclusive_scan_u32(hist, hist, (size_t)256 * tm.n_tiles, tmp.scan, st);
-            {
-                KScope ks("rs_scatter_reads", (8ull + sizeof(K) + 4) * n, st);
-                launch_scatter<K, KS0>(*first_ks, nullptr, kout, vout, tm, shift, nbits, hist,
-                                       atomic_rank, st);
-                GDS_KERNEL_CHECK();
-            }
+            launch_scatter<K, KS0>("rs_scatter_reads", (8ull + sizeof(K) + 4) * n, *first_ks, nullptr,
+                                   kout, vout, tm, shift, nbits, hist, atomic_rank, st);
         } else {
             ArrayKeys<K> ak{kin};
             const uint32_t* vsrc = p == 0 ? nullptr : vin;
-            {
-                KScope ks("rs_hist", sizeof(K) * (unsigned long long)n, st);
-                k_rs_hist<K, ArrayKeys<K>><<<tm.n_tiles, kRsThreads, 0, st>>>(ak, tm, shift, hist);
-                GDS_KERNEL_CHECK();
-            }
+            launch("rs_hist", sizeof(K) * (unsigned long long)n, k_rs_hist<K, ArrayKeys<K>>, tm.n_tiles,
+                   kRsThreads, 0, st, ak, tm, shift, hist);
             exclusive_scan_u32(hist, hist, (size_t)256 * tm.n_tiles, tmp.scan, st);
-            {
-                KScope ks("rs_scatter", (2ull * sizeof(K) + (vsrc ? 8 : 4)) * n, st);
-                launch_scatter<K, ArrayKeys<K>>(ak, vsrc, kout, vout, tm, shift, nbits, hist,
-                                                atomic_rank, st);
-                GDS_KERNEL_CHECK();
-            }
+            launch_scatter<K, ArrayKeys<K>>("rs_scatter", (2ull * sizeof(K) + (vsrc ? 8 : 4)) * n, ak,
+                                            vsrc, kout, vout, tm, shift, nbits, hist, atomic_rank, st);
         }
         cur ^= 1;
     }

@@ -232,9 +232,7 @@ struct ScanTemp {
 };
 
 inline void scan_one_tile(const uint32_t* in, uint32_t* out, size_t n, cudaStream_t st) {
-    KScope ks("scan_u32", 8ull * n, st);
-    k_scan_tiles<<<1, kScanThreads, 0, st>>>(in, out, n);
-    GDS_KERNEL_CHECK();
+    launch("scan_u32", 8ull * n, k_scan_tiles, 1, kScanThreads, 0, st, in, out, n);
 }
 
 // k equally long arrays in one launch; arrays of one tile are scanned one by one
@@ -245,7 +243,6 @@ inline void exclusive_scan_u32_multi(const ScanArrays& a, int n_arr, size_t n, S
         for (int k = 0; k < n_arr; ++k) scan_one_tile(a.in[k], a.out[k], n, st);
         return;
     }
-    KScope ks("scan_u32", 8ull * n * n_arr, st);
     const size_t tl = (n + kLbTile - 1) / kLbTile;
     unsigned long long* status = tmp.status.get<unsigned long long>(tl * n_arr);
     uint32_t* ticket = tmp.ticket.get<uint32_t>(1);
@@ -256,9 +253,8 @@ inline void exclusive_scan_u32_multi(const ScanArrays& a, int n_arr, size_t n, S
         tmp.epoch = 0;
     }
     ++tmp.epoch;
-    k_scan_lookback<<<(unsigned)(tl * n_arr), kLbThreads, 0, st>>>(a, (uint32_t)n_arr, n, (uint32_t)tl,
-                                                                   status, ticket, tmp.epoch);
-    GDS_KERNEL_CHECK();
+    launch("scan_u32", 8ull * n * n_arr, k_scan_lookback, (unsigned)(tl * n_arr), kLbThreads, 0, st, a,
+           (uint32_t)n_arr, n, (uint32_t)tl, status, ticket, tmp.epoch);
 }
 
 // out may alias in.  Callers that need the grand total read out[n-1] + in[n-1] themselves or scan

@@ -762,3 +762,47 @@ def test_minimum_cardinality_sweep(solver, O):
     with _pt.raises(load_package().GdsError):
         solver.solve(np.array([0], np.uint32), np.array([4999], np.uint32), 6000, 1,
                      params=(64, 150, 1, 0, NOSEG, 0, 1))
+
+
+VERDICT_PATHS = {  # bundle path: (reference length, gds_params, length hints?, environment)
+    "sort_hints": (30_000, PRM + (0, 1), True, {}),
+    "sort_no_hints": (30_000, PRM + (0, 1), False, {}),
+    "segmented": (100_000, (64, 150, 1, 0, 8192, 1), True, {}),
+    "direct_sync": (30_000, PRM + (0, 2), True, {"GDS_SYNC": "1"}),
+    "direct_lazy": (30_000, PRM + (0, 2), True, {}),
+    "global_hist": (100_000, (64, 150, 1, 0, 8192, 0), True, {}),
+}
+
+
+@pytest.mark.parametrize("path,kind", [(p, k) for p in VERDICT_PATHS for k in ("range", "hints")
+                                       if k == "range" or VERDICT_PATHS[p][2]])
+def test_input_verdicts_on_every_bundle_path(pkg, solver, O, path, kind):
+    # bad reads fail the call with the exact code and message (with the number of bad reads where
+    # the path counts them), and the context solves the next call as if nothing had happened
+    import os
+    L, prm, hints, env = VERDICT_PATHS[path]
+    s, e, _, _ = O.gen_reads(4100, 20_000, L, 150)
+    idx = np.array([11, 5_000, 39_000])
+    bad_s, bad_e = s.copy(), e.copy()
+    if kind == "range":  # end >= ref_len, length still 150
+        bad_s[idx] = L - 100; bad_e[idx] = L + 49
+        code, what, count = 2, "reads with start > end or end >= ref_len", len(idx)
+    else:  # length 149 under hints of exactly 150
+        bad_e[idx] = bad_s[idx] + 148
+        code, what = 1, "reads outside the len_min/len_max hints"
+        count = 1 if path == "segmented" else len(idx)  # k_validate only reports the bounds there
+    lh = (150, 150) if hints else None
+    os.environ.update(env)
+    try:
+        good = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
+        with pytest.raises(pkg.GdsError) as ei:
+            solver.solve(bad_s, bad_e, L, 40, params=prm, len_hint=lh)
+        again = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
+    finally:
+        for k in env:
+            del os.environ[k]
+    assert ei.value.code == code
+    assert str(ei.value).endswith(": %d %s" % (count, what)), str(ei.value)
+    want_path = {"direct_sync": 1, "direct_lazy": 1, "global_hist": 2}.get(path, 0)
+    assert good.bundle_path == want_path and good.verify_violations == 0
+    assert np.array_equal(again.kept_bitmap, good.kept_bitmap) and again.n_kept == good.n_kept
