@@ -44,6 +44,20 @@ def build_cuda(force=False, verbose=False):
     return LIB
 
 
+def build_kernel_harness(force=False):
+    """tests/kernels/libkernel_harness.so: the scan, radix sort and K5/K6 kernels behind C wrappers
+    for tests/test_kernels.py.  Test infrastructure, never loaded by the package."""
+    kdir = os.path.join(ROOT, "tests", "kernels")
+    src = os.path.join(kdir, "kernel_harness.cu")
+    out = os.path.join(kdir, "libkernel_harness.so")
+    csrc = os.path.join(HERE, "csrc")
+    srcs = [src] + [os.path.join(csrc, f) for f in sorted(os.listdir(csrc))]
+    if not force and not _newer(out, srcs):
+        return out
+    subprocess.check_call([_find_nvcc()] + NVCC_FLAGS + ["-o", out, src])
+    return out
+
+
 def build_host(force=False):
     hdir = os.path.join(HERE, "host")
     if not os.path.isdir(hdir):

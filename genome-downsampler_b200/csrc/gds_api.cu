@@ -6,6 +6,8 @@
 #include <cstddef>
 #include <cstdlib>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <new>
 #include <string>
 #include <thread>
@@ -56,9 +58,7 @@ struct gds_ctx {
     DevBuf dhist, dlay, b_slot, ident, dwork;  // direct (sort-free) bundle path
     DevBuf kstat, pbund, cand, dctl, in_src, dem_v, fb_list, in1, lab_g, taken;
     unsigned sweep_smem_set = 0;  // bit i: the sweep launch shape i has its shared memory set up
-    int mf2_smem_set[2] = {0, 0};
     unsigned direct_attr = 0;                  // bytes of dynamic smem the direct kernels are set up for
-    int mf_smem_set[4] = {0, 0, 0, 0};  // dynamic shared memory the launch shapes are set up for
     bool atomic_rank = false;  // shared-memory atomics rank in lane order on this device (probed)
     Profiler prof;
 
@@ -197,6 +197,21 @@ struct MfArgs {  // k_maxflow
     uint16_t* lab_g;
 };
 
+// The dynamic shared memory a kernel may take is an attribute of the kernel on the device, shared by
+// every gds_ctx (and host thread) there.  It is only ever raised, under one lock: a record kept per
+// context would let a context with small components lower the limit below what another context's
+// next launch needs, and that launch would fail with "invalid argument".
+void raise_smem_limit(const void* kern, int device, int bytes) {
+    static std::mutex mu;
+    static std::map<std::pair<const void*, int>, int> limit;
+    std::lock_guard<std::mutex> lock(mu);
+    int& cur = limit[{kern, device}];
+    if (bytes > cur) {
+        GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        cur = bytes;
+    }
+}
+
 template <int I>
 void launch_maxflow_shape(gds_ctx* c, const MfArgs& a, unsigned long long alg_bytes) {
     constexpr MfShape sh = kMfShapes[I];
@@ -214,10 +229,7 @@ void launch_maxflow_shape(gds_ctx* c, const MfArgs& a, unsigned long long alg_by
             lab_cap = a.max_comp_nodes;
         }
     }
-    if (c->mf_smem_set[I] < smem) {
-        GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        c->mf_smem_set[I] = smem;
-    }
+    raise_smem_limit(reinterpret_cast<const void*>(kern), c->device, smem);
     const K3Args& k = a.k;
     int grid = std::min<uint32_t>(k.n_comp, (uint32_t)kNumSMs * sh.ctas_per_sm);
     launch("maxflow", alg_bytes, kern, grid, sh.threads, smem, c->stream, a.g, k.comp_lo, k.comp_hi,
@@ -335,10 +347,7 @@ void launch_mf2_shape(gds_ctx* c, const Mf2Plan& pl, const Mf2Graph& g, const K3
                       uint32_t* fb_list, uint32_t* fb_count, bool allow_warp,
                       unsigned long long alg_bytes) {
     auto kern = k_maxflow_sm<THREADS>;
-    if (c->mf2_smem_set[SLOT] < pl.smem) {
-        GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
-        c->mf2_smem_set[SLOT] = pl.smem;
-    }
+    raise_smem_limit(reinterpret_cast<const void*>(kern), c->device, pl.smem);
     // with the count on the device n_comp is an estimate (one component per sample or segment); the
     // cuts at cov <= M can make many more (the reference's "low sides" shape: 11 from one sample,
     // which a grid of one CTA solved one after the other).  A CTA without work exits at once.

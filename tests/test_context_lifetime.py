@@ -36,3 +36,34 @@ def test_create_solve_destroy_returns_device_memory(pkg, O):
     torch.cuda.synchronize()
     free_after, _ = torch.cuda.mem_get_info()
     assert abs(free_after - free_before) <= 2 << 20, (free_before, free_after)
+
+
+def test_contexts_on_one_device_leave_each_others_launches_alone(pkg, O):
+    # How much shared memory a kernel may take is a property of the kernel on the device, not of a
+    # context.  Context `a` solves large components first; context `b` then solves small ones, whose
+    # K3 launches need less.  `b` must not lower the limit under `a`: a's next solve of the same input
+    # must run and give the same answer.  Both K3 kernels: the shared-memory one (default) and
+    # k_maxflow (GDS_MF=global).
+    import os
+
+    parts = [O.gen_reads(610 + k, 20_000, 30_000, 150) for k in range(3)]
+    big = (np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts]), [30_000] * 3, 60)
+    big_kw = dict(read_off=np.arange(4, dtype=np.uint64) * 40_000, params=PRM, verify=True)
+    ex = O.SMALL_EXAMPLE
+    small = [(ex["start"], ex["end"], ex["L"], ex["M"]),
+             (np.full(5000, 10, np.uint32), np.full(5000, 60, np.uint32), 100, 17)]
+    for env in ({}, {"GDS_MF": "global"}):
+        os.environ.update(env)
+        a, b = pkg.Solver(0), pkg.Solver(0)
+        try:
+            first = a.solve(*big, **big_kw)
+            for args in small:
+                assert b.solve(*args, params=PRM, verify=True).verify_violations == 0
+            again = a.solve(*big, **big_kw)
+        finally:
+            a.close()
+            b.close()
+            for k in env:
+                del os.environ[k]
+        assert first.rounds_total > 0 and again.verify_violations == 0
+        assert np.array_equal(again.kept_bitmap, first.kept_bitmap) and again.n_kept == first.n_kept
