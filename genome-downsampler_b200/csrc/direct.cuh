@@ -235,9 +235,10 @@ k_direct_bundles(const uint32_t* __restrict__ ghist, uint32_t ktot, DirectLayout
 // k_direct_mark streams the reads once more (start only when there is one read length), in
 // parallel parts like the histogram: code 1 sets the kept bit, code 2 appends the read index to
 // the bundle's segment.  k_direct_partial then ranks each partial bundle's candidates (one warp per
-// bundle; the host sizes the candidate buffer from ctl[1] between the two kernels).  If a partial
-// bundle is huge (adversarial input: millions of identical reads), ctl[2] is raised and the host
-// runs the ordered walk below instead — same kept set, one CTA per sample.
+// bundle).  If the candidates do not fit their buffer, ctl[2] is raised and the host repeats the
+// selection with the buffer grown to ctl[1].  If a partial bundle is huge (adversarial input:
+// millions of identical reads), ctl[2] is raised and the host repeats the selection with the
+// ordered walk below instead — same kept set, one CTA per sample.
 constexpr uint32_t kSatCode = 1, kPartCode = 2;
 constexpr uint32_t kMaxPartialMult = 2048;  // candidates of one bundle ranked by one warp
 // 512 threads x 3 CTAs per SM at 40 registers (one read length): the kernel is bound by neither
@@ -252,15 +253,15 @@ constexpr uint32_t kDmSplit = 3;
 // walk instead), 2 the candidates do not fit cand_cap (the host grows the buffer and repeats the
 // selection), 4 K2 counted bad reads (the call fails; the mark kernels do not re-validate)
 __global__ void __launch_bounds__(256)
-k_direct_classify(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ b_slot, uint32_t B,
+k_direct_classify(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ b_slot,
                   uint32_t* __restrict__ ghist, uint32_t* __restrict__ kstat,
                   uint32_t* __restrict__ pb_off, uint32_t* __restrict__ pb_f,
                   uint32_t* __restrict__ pb_fill, uint32_t* __restrict__ ctl, uint32_t max_mult,
-                  const uint32_t* __restrict__ B_dev /* non-null: bundle count on the device */,
-                  uint32_t cand_cap, const uint32_t* __restrict__ stats) {
+                  const uint32_t* __restrict__ B_dev, uint32_t cand_cap,
+                  const uint32_t* __restrict__ stats) {
     __shared__ uint32_t tot_n, tot_m, base_n, base_m;
     const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (B_dev) B = *B_dev;
+    const uint32_t B = *B_dev;
     if (b == 0 && (stats[2] | stats[3])) atomicOr(&ctl[2], 4u);
     uint32_t mult = 0, f = 0;
     if (b < B) {
@@ -562,11 +563,10 @@ k_direct_partial(const uint32_t* __restrict__ pb_off, const uint32_t* __restrict
 // most once) the candidates of that key are ranked by index.  The walk stops when every quota is
 // used up.
 __global__ void __launch_bounds__(256)
-k_direct_quota(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ b_slot, uint32_t B,
+k_direct_quota(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ b_slot,
                uint32_t* __restrict__ ghist, const uint32_t* __restrict__ B_dev) {
     const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (B_dev) B = *B_dev;
-    if (b < B) ghist[b_slot[b]] = bund[b].f;
+    if (b < *B_dev) ghist[b_slot[b]] = bund[b].f;
 }
 
 __global__ void __launch_bounds__(kDsThreads, 1)

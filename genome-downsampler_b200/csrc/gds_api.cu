@@ -121,18 +121,15 @@ struct Knobs {
     bool mf_sm;             // GDS_MF=sm: k_maxflow_sm whenever it fits
     bool mf_optr;           // GDS_MF_OPTR=0: k_maxflow_sm without the out-CSR cache
     bool mf_warp;           // GDS_MF_WARP=1 (see launch_mf2_shape)
-    bool sync;              // GDS_SYNC=1: the lazy path keeps its readbacks
     bool walk;              // GDS_DIRECT_SELECT=walk: K5 of the histogram path takes the ordered walk
     const char* dump_comp;  // GDS_DUMP_COMP=<file>: per-component K3 records
     static Knobs read() {
         const char* mf = getenv("GDS_MF");
         const char* optr = getenv("GDS_MF_OPTR");
         const char* warp = getenv("GDS_MF_WARP");
-        const char* sync = getenv("GDS_SYNC");
         const char* sel = getenv("GDS_DIRECT_SELECT");
         return Knobs{mf && !strcmp(mf, "global"), mf && !strcmp(mf, "sm"), !optr || optr[0] != '0',
-                     warp && warp[0] == '1', sync && sync[0] == '1', sel && !strcmp(sel, "walk"),
-                     getenv("GDS_DUMP_COMP")};
+                     warp && warp[0] == '1', sel && !strcmp(sel, "walk"), getenv("GDS_DUMP_COMP")};
     }
 };
 
@@ -146,7 +143,7 @@ struct StatsBlock {
     // F* of the virtual network, reads kept, verification violations, F* of the original network,
     // units through the cut nodes, what the minimum-cardinality sweep could not fill or place
     unsigned long long fstar_virtual, n_kept, violations, fstar_orig, through_flow, sweep_fail;
-    uint32_t n_bundles, n_comp;      // lazy mode: the counts stay on the device
+    uint32_t n_bundles, n_comp;      // the counts stay on the device until the final readback
     uint32_t pad1[2];
     uint32_t ctl[4];                 // K5 control words of the histogram path (direct_select)
     uint32_t pad2[4];
@@ -180,12 +177,12 @@ StatsBlock read_input_verdict(gds_ctx* c, const StatsBlock* ds) {
 // What both K3 kernels are given (host side; every launch shape passes it on)
 struct K3Args {
     const uint32_t *comp_lo, *comp_hi;
-    uint32_t n_comp;
+    uint32_t n_comp;  // the host's estimate: it picks the launch shape and the grid
     uint32_t* wc;
     uint32_t *qF, *qT, *qN, *qH;
     SolveParams sp;
     CompStats* cstats;
-    const uint32_t* n_comp_dev;
+    const uint32_t* n_comp_dev;  // the count itself
     MfTotals* mft;
 };
 
@@ -233,8 +230,8 @@ void launch_maxflow_shape(gds_ctx* c, const MfArgs& a, unsigned long long alg_by
     const K3Args& k = a.k;
     int grid = std::min<uint32_t>(k.n_comp, (uint32_t)kNumSMs * sh.ctas_per_sm);
     launch("maxflow", alg_bytes, kern, grid, sh.threads, smem, c->stream, a.g, k.comp_lo, k.comp_hi,
-           k.n_comp, k.wc, k.qF, k.qT, k.qN, k.qH, k.sp, k.cstats, lab_cap, a.comp_list,
-           a.comp_list_n, k.n_comp_dev, k.mft, a.lab_g);
+           k.wc, k.qF, k.qT, k.qN, k.qH, k.sp, k.cstats, lab_cap, a.comp_list, a.comp_list_n,
+           k.n_comp_dev, k.mft, a.lab_g);
 }
 
 void launch_maxflow(gds_ctx* c, const MfArgs& a, unsigned long long alg_bytes) {
@@ -348,21 +345,20 @@ void launch_mf2_shape(gds_ctx* c, const Mf2Plan& pl, const Mf2Graph& g, const K3
                       unsigned long long alg_bytes) {
     auto kern = k_maxflow_sm<THREADS>;
     raise_smem_limit(reinterpret_cast<const void*>(kern), c->device, pl.smem);
-    // with the count on the device n_comp is an estimate (one component per sample or segment); the
-    // cuts at cov <= M can make many more (the reference's "low sides" shape: 11 from one sample,
-    // which a grid of one CTA solved one after the other).  A CTA without work exits at once.
-    const int grid = (int)std::min<uint32_t>(k.n_comp_dev ? 0xffffffffu : k.n_comp,
-                                             (uint32_t)(kNumSMs * pl.per_sm));
+    // one full wave: k.n_comp is an estimate (one component per sample or segment), and the cuts at
+    // cov <= M can make many more (the reference's "low sides" shape: 11 from one sample, which a
+    // grid of one CTA solved one after the other).  A CTA without work exits at once.
+    const int grid = kNumSMs * pl.per_sm;
     launch("maxflow", alg_bytes, kern, grid, THREADS, pl.smem, c->stream, g, k.comp_lo, k.comp_hi,
-           k.n_comp, k.wc, k.qF, k.qT, k.qN, k.qH, k.sp, k.cstats, (uint32_t)pl.smem, pl.qcap,
-           fb_list, fb_count, pl.optr ? 1u : 0u, k.n_comp_dev, k.mft, allow_warp ? 1u : 0u);
+           k.wc, k.qF, k.qT, k.qN, k.qH, k.sp, k.cstats, (uint32_t)pl.smem, pl.qcap, fb_list,
+           fb_count, pl.optr ? 1u : 0u, k.n_comp_dev, k.mft, allow_warp ? 1u : 0u);
 }
 
 // K3' (sweep.cuh): the minimum-cardinality solve.  One warp per component.
 struct SweepArgs {
     SweepGraph g;
     const uint32_t *comp_lo, *comp_hi;
-    uint32_t n_comp;
+    uint32_t n_comp;  // the host's estimate, for the grid
     const uint32_t* n_comp_dev;
     uint32_t M;
     uint32_t* wc;
@@ -379,7 +375,7 @@ void launch_sweep_shape(gds_ctx* c, const SweepArgs& a, unsigned long long alg_b
         c->sweep_smem_set |= 1u << SLOT;
     }
     launch("sweep", alg_bytes, kern, grid, kSweepWarps * 32, smem, c->stream, a.g, a.comp_lo,
-           a.comp_hi, a.n_comp, a.n_comp_dev, a.M, a.wc, a.fail);
+           a.comp_hi, a.n_comp_dev, a.M, a.wc, a.fail);
 }
 
 void launch_sweep(gds_ctx* c, const SweepArgs& a, uint32_t maxlen, bool one_len,
@@ -405,10 +401,6 @@ struct DirectPlan {
     uint32_t* in_bid = nullptr;  // identity in-CSR (single read length), else null
     bool global = false;         // counters in global memory (several lengths / segmented reference)
     GDirectLayout gl{};
-    // lazy: no readback between the kernels — B is an upper bound on the host, the exact count
-    // lives in *B_dev, and input errors are looked at with the final readback
-    bool lazy = false;
-    const uint32_t* B_dev = nullptr;
 };
 
 // How the virtual node space is laid out: references longer than two segments are cut into
@@ -423,7 +415,7 @@ struct SegPlan {
     uint32_t n_nodes;
     uint32_t max_comp_nodes;  // no component is larger than a whole unsegmented sample or one segment
     // one component per sample or segment (zero-coverage gaps add more, empty samples take some
-    // away): the host's ESTIMATE of the component count in lazy mode
+    // away): the host's ESTIMATE of the component count, which stays on the device
     uint32_t comp_estimate;
 };
 
@@ -474,7 +466,7 @@ struct SolveCall {
     uint32_t* oexcl;
     // K2
     DirectPlan direct;
-    uint32_t B;
+    uint32_t B;  // exact when the host needs it (radix sorts over the bundles), else a bound
     uint32_t* sorted_idx;
     int sort_passes;
     // nodes and components
@@ -486,8 +478,7 @@ struct SolveCall {
     bool forced_cuts;
     uint32_t* fmult;
     uint8_t* dead;
-    uint32_t n_comp, n_comp_cap;
-    const uint32_t* n_comp_dev;
+    uint32_t n_comp_cap;  // a bound; the count is ds->n_comp
     uint32_t *comp_lo, *comp_hi, *in_bid;
     CompStats* cstats;
     // K5 and the final readback
@@ -549,8 +540,9 @@ void build_bundles(gds_ctx* c, SolveCall& sc, const TileMap& tm, const uint32_t*
     launch("heads_count", (sizeof(K) * 8ull + 1ull) * n_items / 8, k_heads_count<K>, n_tiles,
            kHeadThreads, 0, st, keys, tm, tc, head_bits);
     exclusive_scan_u32(tc, tc, n_tiles + 1, c->scan, st);
+    GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_bundles, tc + n_tiles, 4, cudaMemcpyDeviceToDevice, st));
     uint32_t B = 0;
-    d2h_sync(c, &B, tc + n_tiles, 1);
+    d2h_sync(c, &B, tc + n_tiles, 1);  // the sort path sizes and launches by the exact count
     sc.B = B;
     if (fused_ref_len) read_input_verdict(c, sc.ds);  // validation fused into the first histogram pass
     uint32_t* b_first = c->b_first.get<uint32_t>(B + 1);
@@ -624,11 +616,10 @@ struct BundleOut {
 };
 
 // What both histogram paths do once plan.ghist holds the counts: count the non-empty keys per
-// tile, scan, the bundle count sc.B (lazy: it stays on the device, b_bound sizes the buffers), the
-// bundle buffers and the cleared degree arrays.  own_diff: the bundle kernel writes the whole
-// difference array itself.
+// tile, scan, the bundle count (on the device; b_bound sizes the buffers), the bundle buffers and
+// the cleared degree arrays.  own_diff: the bundle kernel writes the whole difference array itself.
 BundleOut histogram_bundles(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint64_t b_bound,
-                            bool own_diff, uint64_t* n_cross) {
+                            bool own_diff) {
     cudaStream_t st = sc.st;
     const uint32_t ktot = plan.ktot;
     const uint32_t n_tiles = (uint32_t)div_up(ktot, kDkTile);
@@ -636,16 +627,13 @@ BundleOut histogram_bundles(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint64_
     GDS_CUDA(cudaMemsetAsync(tc + n_tiles, 0, sizeof(uint32_t), st));
     launch("direct_count", 4ull * ktot, k_direct_count, n_tiles, kDkThreads, 0, st, plan.ghist, ktot, tc);
     exclusive_scan_u32(tc, tc, n_tiles + 1, c->scan, st);
-    uint32_t B = 0;
-    if (plan.lazy) {  // the count stays on the device; size everything by its bound
-        GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_bundles, tc + n_tiles, 4, cudaMemcpyDeviceToDevice, st));
-        plan.B_dev = &sc.ds->n_bundles;
-        B = (uint32_t)std::min<uint64_t>(ktot, b_bound);
-        if (n_cross) *n_cross = 0;  // known with the final readback
-    } else {
+    GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_bundles, tc + n_tiles, 4, cudaMemcpyDeviceToDevice, st));
+    uint32_t B = (uint32_t)std::min<uint64_t>(ktot, b_bound);
+    if (sc.minlen != sc.maxlen) {
+        // several read lengths: the in-CSR order comes from a radix sort of the bundles (build_nodes),
+        // which needs their exact number; the input verdict comes with the same synchronisation
         d2h_sync(c, &B, tc + n_tiles, 1);
-        const StatsBlock h = read_input_verdict(c, sc.ds);
-        if (n_cross) *n_cross = h.n_cross;
+        read_input_verdict(c, sc.ds);
     }
     sc.B = B;
     BundleOut o{n_tiles, tc, c->bund.get<BundleRec>(B + 1), c->b_t.get<uint32_t>(B + 1),
@@ -707,7 +695,7 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
     plan.kmax = kmax;
     plan.n_items = n_items;
     // one read length: k_direct_bundles writes the difference array of every node itself
-    const BundleOut o = histogram_bundles(c, sc, plan, N, nlen == 1, nullptr);
+    const BundleOut o = histogram_bundles(c, sc, plan, N, nlen == 1);
     if (sc.B)
         launch("direct_bundles", 4ull * ktot + 40ull * sc.B, k_direct_bundles, o.n_tiles, kDkThreads, 0,
                st, ghist, ktot, dl, o.tc, o.bund, o.b_t, o.b_slot, o.ident, o.d.diff, o.d.outdeg,
@@ -716,7 +704,7 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
 
 // The same with the counters in global memory (direct.cuh: k_gdirect_*): any layout whose key space
 // (virtual nodes x read lengths) stays L2-sized.
-void build_bundles_gdirect(gds_ctx* c, SolveCall& sc, uint64_t& n_cross) {
+void build_bundles_gdirect(gds_ctx* c, SolveCall& sc) {
     cudaStream_t st = sc.st;
     DirectPlan& plan = sc.direct;
     const uint64_t N = sc.N;
@@ -732,7 +720,7 @@ void build_bundles_gdirect(gds_ctx* c, SolveCall& sc, uint64_t& n_cross) {
     plan.ghist = ghist;
     plan.ktot = ktot;
     // a read crossing a cut counts twice
-    const BundleOut o = histogram_bundles(c, sc, plan, 2 * N, false, &n_cross);
+    const BundleOut o = histogram_bundles(c, sc, plan, 2 * N, false);
     if (sc.B)
         launch("gdirect_bundles", 4ull * ktot + 40ull * sc.B, k_gdirect_bundles, o.n_tiles, kDkThreads,
                0, st, ghist, ktot, gl, o.tc, o.bund, o.b_t, o.b_slot, o.ident, o.d.diff, o.d.outdeg,
@@ -741,25 +729,25 @@ void build_bundles_gdirect(gds_ctx* c, SolveCall& sc, uint64_t& n_cross) {
 
 // K5 on the direct path (direct.cuh): classify the bundles, mark the reads of saturated bundles in
 // one parallel streaming pass, rank the candidates of partial bundles; the ordered walk is the
-// fallback when the candidates do not fit (or GDS_DIRECT_SELECT=walk asks for it).
-// force_walk: the ordered walk right away (the lazy path's second attempt after ctl flag 1).
-// Lazy mode (dp.lazy): nothing is read back here.  The candidate buffer keeps the size it has
-// (never below N/8 slots); k_direct_classify raises ctl flag 2 when the candidates do not fit and
-// flag 1 for a partial bundle too large for one warp, the mark / ranking kernels then do nothing,
-// and gds_solve — which sees the flags with its one final readback — repeats the selection.
+// fallback when a partial bundle is too large for one warp (or GDS_DIRECT_SELECT=walk asks for it).
+// Nothing is read back here.  The candidate buffer keeps the size it has (never below N/8 slots or
+// cand_need); k_direct_classify raises ctl flag 2 when the candidates do not fit and flag 1 for a
+// partial bundle too large for one warp, the mark / ranking kernels then do nothing, and
+// select_reads — which sees the flags with the final readback — repeats the selection: with a
+// larger buffer, or with the ordered walk right away (force_walk).
 void direct_select(gds_ctx* c, SolveCall& sc, bool force_walk, size_t cand_need) {
     cudaStream_t st = sc.st;
     const DirectPlan& dp = sc.direct;
     const uint32_t B = sc.B;
+    const uint32_t* B_dev = &sc.ds->n_bundles;
     const size_t N = sc.N;
     uint32_t* bm = sc.bm;
     unsigned long long* totals = sc.totals();
     BundleRec* bund = c->bund.as<BundleRec>();
     uint32_t* b_slot = c->b_slot.as<uint32_t>();
-    bool walk = !dp.global && (force_walk || sc.knobs.walk);
     uint32_t* ctl = c->dctl.get<uint32_t>(4);
     GDS_CUDA(cudaMemsetAsync(ctl, 0, 16, st));
-    if (!walk) {
+    if (dp.global || !(force_walk || sc.knobs.walk)) {
         uint32_t* kstat = c->kstat.get<uint32_t>(dp.ktot / 16 + 1);
         uint32_t* pb = c->pbund.get<uint32_t>(3 * ((size_t)B + 1));
         uint32_t* fill = pb + 2 * ((size_t)B + 1);
@@ -768,57 +756,42 @@ void direct_select(gds_ctx* c, SolveCall& sc, bool force_walk, size_t cand_need)
         // and regrowing the arena is expensive
         size_t cand_cap = std::max<size_t>({cand_need, N / 8, c->cand.cap / 4, (size_t)1});
         cand_cap = std::min<size_t>(cand_cap, 0xffffffffu);
-        uint32_t* cand = dp.lazy ? c->cand.get<uint32_t>(cand_cap) : nullptr;
+        uint32_t* cand = c->cand.get<uint32_t>(cand_cap);
         // a partial bundle beyond kMaxPartialMult reads sends the shared-memory path to the
         // ordered walk; the global path has no walk and lets one warp grind through it
         launch("direct_classify", 20ull * B, k_direct_classify, div_up(B, 256), 256, 0, st, bund,
-               b_slot, B, dp.ghist, kstat, pb, pb + B + 1, fill, ctl,
-               dp.global ? 0xffffffffu : kMaxPartialMult, dp.B_dev,
-               dp.lazy ? (uint32_t)cand_cap : 0xffffffffu, sc.stats());
-        uint32_t hctl[4] = {1, 0, 0, 0};  // lazy: the ranking kernel is launched unconditionally
-        if (!dp.lazy) {
-            d2h_sync(c, hctl, ctl, 4);  // candidate buffer sized exactly
-            sc.out->partial_bundles = hctl[0];
-            sc.out->partial_candidates = hctl[1];
-            walk = (hctl[2] & 1u) != 0;
-            if (!walk) cand = c->cand.get<uint32_t>(std::max<size_t>((size_t)hctl[1] + 1, N / 8));
+               b_slot, dp.ghist, kstat, pb, pb + B + 1, fill, ctl,
+               dp.global ? 0xffffffffu : kMaxPartialMult, B_dev, (uint32_t)cand_cap, sc.stats());
+        const unsigned long long per_read = (dp.global || dp.dl.nlen > 1) ? 8 : 4;
+        if (dp.global) {
+            launch("gdirect_mark", per_read * N + dp.ktot / 4 + 8ull * N / 32, k_gdirect_mark,
+                   div_up((long long)N, kGdTile), kGdThreads, 0, st, sc.S, sc.E, N, dp.gl, dp.ghist,
+                   kstat, pb, fill, cand, bm, totals, ctl);
+        } else {
+            uint32_t* wc = c->dwork.as<uint32_t>() + 1;
+            GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
+            const int grid = (int)std::min<uint32_t>(
+                dp.n_items * kDmSplit, (uint32_t)kNumSMs * (dp.dl.nlen == 1 ? kDmCtasPerSm : 2));
+            launch("direct_mark", per_read * N + dp.ktot / 4 + 8ull * N / 32,
+                   dp.dl.nlen == 1 ? k_direct_mark<true> : k_direct_mark<false>, grid, kDmThreads,
+                   kDmQueueBytes + dp.kmax, st, sc.S, sc.E, dp.dl, dp.n_items, wc, dp.ghist, kstat, pb,
+                   fill, cand, ctl, bm, totals);
         }
-        if (!walk) {
-            const unsigned long long per_read = (dp.global || dp.dl.nlen > 1) ? 8 : 4;
-            if (dp.global) {
-                launch("gdirect_mark", per_read * N + dp.ktot / 4 + 8ull * N / 32, k_gdirect_mark,
-                       div_up((long long)N, kGdTile), kGdThreads, 0, st, sc.S, sc.E, N, dp.gl,
-                       dp.ghist, kstat, pb, fill, cand, bm, totals, ctl);
-            } else {
-                uint32_t* wc = c->dwork.as<uint32_t>() + 1;
-                GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
-                const int grid = (int)std::min<uint32_t>(
-                    dp.n_items * kDmSplit, (uint32_t)kNumSMs * (dp.dl.nlen == 1 ? kDmCtasPerSm : 2));
-                launch("direct_mark", per_read * N + dp.ktot / 4 + 8ull * N / 32,
-                       dp.dl.nlen == 1 ? k_direct_mark<true> : k_direct_mark<false>, grid, kDmThreads,
-                       kDmQueueBytes + dp.kmax, st, sc.S, sc.E, dp.dl, dp.n_items, wc, dp.ghist, kstat,
-                       pb, fill, cand, ctl, bm, totals);
-            }
-            // segments of a long reference (global path): ~10 reads per bundle, half a warp each
-            if (hctl[0])
-                launch("direct_partial",
-                       dp.lazy ? 16ull * (N / 64) : 16ull * hctl[0] + 4ull * hctl[1],
-                       dp.global ? k_direct_partial<true> : k_direct_partial<false>, kNumSMs * 32, 256,
-                       0, st, pb, pb + B + 1, fill, cand, ctl, bm, totals);
-            if (dp.lazy)
-                GDS_CUDA(cudaMemcpyAsync(sc.ds->ctl, ctl, 16, cudaMemcpyDeviceToDevice, st));
-            return;
-        }
+        // segments of a long reference (global path): ~10 reads per bundle, half a warp each
+        launch("direct_partial", 16ull * (N / 64),
+               dp.global ? k_direct_partial<true> : k_direct_partial<false>, kNumSMs * 32, 256, 0, st,
+               pb, pb + B + 1, fill, cand, ctl, bm, totals);
+    } else {
+        // ordered walk: one CTA per sample, quota per key in shared memory
+        launch("direct_quota", 24ull * B, k_direct_quota, div_up(B, 256), 256, 0, st, bund, b_slot,
+               dp.ghist, B_dev);
+        uint32_t* wc = c->dwork.as<uint32_t>() + 1;
+        GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
+        launch("direct_walk", 4ull * dp.ktot + 8ull * N / 32, k_direct_select,
+               (int)std::min<uint32_t>(sc.ns, (uint32_t)kNumSMs), kDsThreads, dp.kmax * 4, st, sc.S,
+               sc.E, dp.dl, wc, dp.ghist, bm, totals);
     }
-    // ordered walk: one CTA per sample, quota per key in shared memory
-    launch("direct_quota", 24ull * B, k_direct_quota, div_up(B, 256), 256, 0, st, bund, b_slot, B,
-           dp.ghist, dp.B_dev);
-    uint32_t* wc = c->dwork.as<uint32_t>() + 1;
-    GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
-    launch("direct_walk", 4ull * dp.ktot + 8ull * N / 32, k_direct_select,
-           (int)std::min<uint32_t>(sc.ns, (uint32_t)kNumSMs), kDsThreads, dp.kmax * 4, st, sc.S, sc.E,
-           dp.dl, wc, dp.ghist, bm, totals);
-    if (dp.lazy) GDS_CUDA(cudaMemcpyAsync(sc.ds->ctl, ctl, 16, cudaMemcpyDeviceToDevice, st));
+    GDS_CUDA(cudaMemcpyAsync(sc.ds->ctl, ctl, 16, cudaMemcpyDeviceToDevice, st));
 }
 
 }  // namespace
@@ -1280,21 +1253,13 @@ void find_bundles(gds_ctx* c, SolveCall& sc) {
         if (n_items >= (1ull << 32) - 64)
             throw CallFail{GDS_ERR_RANGE, "more than 2^32 arc items after segmentation"};
     }
-    out->n_arc_items = n_items;
-    // Lazy mode: one read length (the in-CSR is the identity, no second sort to size) on a
-    // histogram path, caller-provided length hints (no validation readback): nothing is read
-    // back until the end of the call, so the ~25 launches queue up behind each other instead
-    // of waiting for the host five times.  GDS_SYNC=1 keeps the readbacks (measurements).
-    sc.direct.lazy = (use_direct || use_gdirect) && sc.fused_validation && sc.minlen == sc.maxlen &&
-                     !sc.flt && !sc.knobs.sync;
+    out->n_arc_items = n_items;  // (global histogram: N + n_cross, with the final readback)
     if (use_direct) {
         build_bundles_direct(c, sc);
         out->key_bits = bits_for(sc.direct.kmax - 1);
         out->bundle_path = 1;
     } else if (use_gdirect) {
-        uint64_t n_cross = 0;
-        build_bundles_gdirect(c, sc, n_cross);
-        out->n_arc_items = N + n_cross;
+        build_bundles_gdirect(c, sc);
         out->key_bits = bits_for((uint64_t)sc.direct.ktot - 1);
         out->bundle_path = 2;
     } else if (N > 0) {
@@ -1306,7 +1271,6 @@ void find_bundles(gds_ctx* c, SolveCall& sc) {
         c->bund.get<BundleRec>(1);
     }
     sc.deg = Degrees{c->diff.as<int32_t>(), c->outdeg.as<uint32_t>(), c->indeg.as<uint32_t>()};
-    out->n_bundles = sc.B;
     out->sort_passes = sc.sort_passes;
 }
 
@@ -1376,23 +1340,14 @@ void build_nodes(gds_ctx* c, SolveCall& sc) {
     }
     uint32_t* sidx = c->comp_sidx.get<uint32_t>(n_nodes + 1);
     exclusive_scan_u32(cstart, sidx, n_nodes + 1, c->scan, st);
-    const bool lazy = sc.direct.lazy;
-    if (lazy) {
-        // the count stays on the device; on the host an estimate picks the K3 kernel and the
-        // grid, and the arrays are sized by the bound
-        GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_comp, sidx + n_nodes, 4, cudaMemcpyDeviceToDevice, st));
-        sc.n_comp_dev = &sc.ds->n_comp;
-        sc.n_comp = sc.plan.comp_estimate;
-    } else {
-        d2h_sync(c, &sc.n_comp, sidx + n_nodes, 1);  // also fences hvs/hcuts uploads
-    }
-    out->n_components = sc.n_comp;
-    sc.n_comp_cap = lazy ? n_nodes / 2 + 1 : sc.n_comp;
+    // the count stays on the device; on the host SegPlan::comp_estimate picks the K3 kernel and the
+    // grid, and the arrays are sized by the bound (a component has >= 2 nodes)
+    GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_comp, sidx + n_nodes, 4, cudaMemcpyDeviceToDevice, st));
+    sc.n_comp_cap = n_nodes / 2 + 1;
     sc.comp_lo = c->comp_lo.get<uint32_t>(sc.n_comp_cap + 1);
     sc.comp_hi = c->comp_hi.get<uint32_t>(sc.n_comp_cap + 1);
-    if (sc.n_comp)
-        launch("comp_write", 16ull * n_nodes, k_comp_write, div_up(n_nodes, 256), 256, 0, st, cstart,
-               cend, sidx, n_nodes, sc.comp_lo, sc.comp_hi);
+    launch("comp_write", 16ull * n_nodes, k_comp_write, div_up(n_nodes, 256), 256, 0, st, cstart, cend,
+           sidx, n_nodes, sc.comp_lo, sc.comp_hi);
     // in-CSR: bundle ids ordered by (end node, bundle id) = stable sort of ids by b_t
     sc.in_bid = sc.direct.in_bid;  // single read length: bundle order is end order too
     if (B && !sc.in_bid) {
@@ -1416,9 +1371,9 @@ void build_nodes(gds_ctx* c, SolveCall& sc) {
 
 // K3: max flow (k_maxflow_sm and/or k_maxflow), or the sweep of the minimum-cardinality solve
 void solve_flow(gds_ctx* c, SolveCall& sc) {
-    const uint32_t n_nodes = sc.plan.n_nodes, B = sc.B, n_comp = sc.n_comp;
+    const uint32_t n_nodes = sc.plan.n_nodes, B = sc.B, n_comp = sc.plan.comp_estimate;
     const uint32_t max_comp_nodes = sc.plan.max_comp_nodes;
-    const uint32_t* n_comp_dev = sc.n_comp_dev;
+    const uint32_t* n_comp_dev = &sc.ds->n_comp;
     cudaStream_t st = sc.st;
     BundleRec* bund = c->bund.as<BundleRec>();
     const Degrees& d = sc.deg;
@@ -1435,12 +1390,12 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
     uint32_t* in1 = c->in1.get<uint32_t>((size_t)n_nodes + 1);
     GDS_CUDA(cudaMemsetAsync(in1, 0xff, ((size_t)n_nodes + 1) * 4, st));
     if (B)
-        launch("in_src", 24ull * B, k_in_src, div_up(B, 256), 256, 0, st, bund, sc.in_bid, d.indeg, B,
-               in_src, mf2.on ? sc.node : nullptr, sc.direct.B_dev, in1);
+        launch("in_src", 24ull * B, k_in_src, div_up(B, 256), 256, 0, st, bund, sc.in_bid, d.indeg,
+               &sc.ds->n_bundles, in_src, mf2.on ? sc.node : nullptr, in1);
     // per-component records only for the diagnostics dump; gds_result's counters are summed on
     // the device (MfTotals)
     sc.cstats = sc.knobs.dump_comp ? c->comp_stats.get<CompStats>(sc.n_comp_cap + 1) : nullptr;
-    if (sc.do_solve && n_comp && sc.algorithm == 1) {
+    if (sc.do_solve && sc.algorithm == 1) {
         // K3': greedy interval multicover, one warp per component, then bundle flows
         uint32_t* wc = c->work_counter.get<uint32_t>(4);
         GDS_CUDA(cudaMemsetAsync(wc, 0, 16, st));
@@ -1453,12 +1408,14 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
             launch("sweep_distribute", 12ull * n_nodes + 24ull * B, k_sweep_distribute,
                    div_up((long long)n_nodes, 256), 256, 0, st, taken, d.indeg, sc.in_bid, bund, n_nodes,
                    &sc.ds->sweep_fail);
-    } else if (sc.do_solve && n_comp) {
+    } else if (sc.do_solve) {
         uint32_t* wc = c->work_counter.get<uint32_t>(4);  // [0] sm kernel, [1] fallback, [2] list size
         GDS_CUDA(cudaMemsetAsync(wc, 0, 16, st));
-        K3Args k{sc.comp_lo, sc.comp_hi, n_comp, wc, c->qF.get<uint32_t>(n_nodes),
-                 c->qT.get<uint32_t>(n_nodes), c->qN.get<uint32_t>(n_nodes),
-                 c->qH.get<uint32_t>(n_nodes), sc.sp, sc.cstats, n_comp_dev, &sc.ds->mf};
+        // k_maxflow gets at least one wave: the estimate may be low
+        K3Args k{sc.comp_lo, sc.comp_hi, std::max<uint32_t>(n_comp, kNumSMs), wc,
+                 c->qF.get<uint32_t>(n_nodes), c->qT.get<uint32_t>(n_nodes),
+                 c->qN.get<uint32_t>(n_nodes), c->qH.get<uint32_t>(n_nodes), sc.sp, sc.cstats,
+                 n_comp_dev, &sc.ds->mf};
         const unsigned long long mf_bytes = 36ull * n_nodes + 20ull * B;
         // compact labels for k_maxflow's relabels
         uint16_t* lab_g = c->lab_g.get<uint16_t>(2 * (size_t)n_nodes + 4);
@@ -1469,14 +1426,10 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
                               sc.vs_d, sc.ns, express_on, mf2.classic_ok ? 1u : 0u, sc.dead};
             (mf2.per_sm >= 2 ? launch_mf2_shape<256, 0> : launch_mf2_shape<512, 1>)(
                 c, mf2, g2, k, fb_list, wc + 2, sc.knobs.mf_warp, mf_bytes);
-            // whatever the shared-memory kernel could not take (grid: at most one wave)
-            // (with the count on the device the list may be longer than the estimate says)
-            k.n_comp = mf2.classic_ok && !n_comp_dev ? std::min<uint32_t>(n_comp, kNumSMs)
-                                                     : std::max<uint32_t>(n_comp, kNumSMs);
+            // whatever the shared-memory kernel could not take
             k.wc = wc + 1;
             launch_maxflow(c, MfArgs{mg, k, max_comp_nodes, fb_list, wc + 2, lab_g}, 0);
         } else {
-            k.n_comp = n_comp_dev ? std::max<uint32_t>(n_comp, kNumSMs) : n_comp;
             launch_maxflow(c, MfArgs{mg, k, max_comp_nodes, nullptr, nullptr, lab_g}, mf_bytes);
         }
     }
@@ -1486,14 +1439,14 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
     GDS_CUDA(cudaEventRecord(c->ev[EV_MAXFLOW], st));
 }
 
-// K5 (selection), K6 (verification) and the final readback.  One pass in the normal case.  In lazy
-// mode the selection may have to be repeated once: the final readback is the first time the host
-// sees that the candidates of the partial bundles did not fit their buffer (it grows) or that a
-// partial bundle needs the ordered walk.
+// K5 (selection), K6 (verification) and the final readback.  One pass in the normal case.  On a
+// histogram path the selection may have to be repeated once: the final readback is the first time
+// the host sees that the candidates of the partial bundles did not fit their buffer (it grows) or
+// that a partial bundle needs the ordered walk.
 void select_reads(gds_ctx* c, SolveCall& sc) {
     const uint32_t B = sc.B, n_onodes = sc.n_onodes;
     const uint64_t N = sc.N;
-    const bool split = sc.plan.split, lazy = sc.direct.lazy;
+    const bool split = sc.plan.split;
     cudaStream_t st = sc.st;
     gds_result* out = sc.out;
     unsigned long long* totals = sc.totals();
@@ -1535,22 +1488,18 @@ void select_reads(gds_ctx* c, SolveCall& sc) {
         if (!attempt) GDS_CUDA(cudaEventRecord(c->ev[EV_VERIFY], st));
 
         if (sc.do_solve && !sc.out_dev) deliver(c, out->kept_bitmap, bm, n_words, false);
-        d2h_sync(c, &h, sc.ds, 1);  // THE readback of a lazy call
-        if (!lazy) break;
+        d2h_sync(c, &h, sc.ds, 1);
         input_verdict(h);
         const uint32_t cflags = sc.do_solve && B && sc.direct.on ? h.ctl[2] : 0;
         if (attempt || !(cflags & 3u)) break;
         force_walk = (cflags & 1u) != 0;  // ordered walk (shared-memory path)
         cand_need = (size_t)h.ctl[1] + 1;  // or the buffer the candidates need
     }
-    if (lazy) {
-        out->n_bundles = h.n_bundles;
-        sc.n_comp = h.n_comp;
-        out->n_components = sc.n_comp;
-        out->partial_bundles = h.ctl[0];
-        out->partial_candidates = h.ctl[1];
-        if (sc.direct.global) out->n_arc_items = N + h.n_cross;
-    }
+    out->n_bundles = h.n_bundles;
+    out->n_components = h.n_comp;
+    out->partial_bundles = h.ctl[0];
+    out->partial_candidates = h.ctl[1];
+    if (sc.direct.global) out->n_arc_items = N + h.n_cross;
 }
 
 // The result: flow and counters from the final readback, stage times, convergence
@@ -1558,7 +1507,7 @@ int finish(gds_ctx* c, SolveCall& sc, unsigned long long launches0) {
     gds_result* out = sc.out;
     const StatsBlock& h = sc.hstat;
     const bool split = sc.plan.split;
-    const uint32_t n_comp = sc.n_comp;
+    const uint32_t n_comp = h.n_comp;
     // fstar_virtual = source capacity of the (virtual) network the kernel solved; when references
     // were segmented the closed-form F* of the ORIGINAL network is fstar_orig and through_flow
     // units pass straight through the cut nodes once the segment flows are stitched together

@@ -413,14 +413,13 @@ k_node_finalize(const uint32_t* __restrict__ excl, const int32_t* __restrict__ d
 // first one a cancel tries — next to its other fields, so a push needs no in-CSR lookup
 __global__ void __launch_bounds__(256)
 k_in_src(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ in_bid,
-         const uint32_t* __restrict__ in_ptr, uint32_t B, uint32_t* __restrict__ in_src,
+         const uint32_t* __restrict__ in_ptr, const uint32_t* __restrict__ B_dev,
+         uint32_t* __restrict__ in_src,
          NodeRec* __restrict__ node /* null: k_maxflow only, the records keep {d, stamp, e, eadd} */,
-         const uint32_t* __restrict__ B_dev /* non-null: the bundle count lives on the device */,
          uint32_t* __restrict__ in1 /* [n_nodes], preset to 0xffffffff: start node of a node's only
                                        in-arc, 0xfffffffe when it has several */) {
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (B_dev) B = *B_dev;
-    if (k >= B) return;
+    if (k >= *B_dev) return;
     const uint32_t b = in_bid[k];
     const uint4 r = reinterpret_cast<const uint4*>(bund)[b];  // t, mult, f, s
     // a forced bundle (capacity 0 while K3 runs) is no arc of the residual graph: the relabels that

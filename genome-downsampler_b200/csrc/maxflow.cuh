@@ -408,12 +408,11 @@ __device__ uint32_t mf_first_relabel(const MfGraph& G, uint32_t lo, uint32_t hi,
 template <int THREADS, uint32_t QCAP, int MIN_CTAS>
 __global__ void __launch_bounds__(THREADS, MIN_CTAS)
 k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __restrict__ comp_hi,
-          uint32_t n_comp, uint32_t* work_counter, uint32_t* qF_g, uint32_t* qT_g, uint32_t* qN_g,
+          uint32_t* work_counter, uint32_t* qF_g, uint32_t* qT_g, uint32_t* qN_g,
           uint32_t* qH_g, SolveParams P, CompStats* __restrict__ stats,
           uint32_t lab_cap /* nodes the shared-memory label array behind MfShared holds (0: none) */,
           const uint32_t* __restrict__ comp_list /* null: all components; else the ids to solve */,
-          const uint32_t* __restrict__ comp_list_n,
-          const uint32_t* __restrict__ n_comp_dev /* non-null: the component count lives on the device */,
+          const uint32_t* __restrict__ comp_list_n, const uint32_t* __restrict__ n_comp_dev,
           MfTotals* __restrict__ totals,
           uint16_t* __restrict__ lab_g /* [2 * n_nodes + 2]: compact 16-bit labels in GLOBAL
               memory for the relabel BFS of components whose labels get no shared memory — the BFS
@@ -422,8 +421,8 @@ k_maxflow(MfGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __res
     MfShared<QCAP>& sh = *reinterpret_cast<MfShared<QCAP>*>(smem_raw);
     uint16_t* lab_smem = reinterpret_cast<uint16_t*>(smem_raw + sizeof(MfShared<QCAP>));
     const uint32_t tid = threadIdx.x;
-    if (n_comp_dev) n_comp = *n_comp_dev;
-    if (comp_list) n_comp = *comp_list_n;  // the components k_maxflow_sm left for this kernel
+    // all components, or those k_maxflow_sm left for this kernel
+    const uint32_t n_comp = comp_list ? *comp_list_n : *n_comp_dev;
 
     for (;;) {
         if (tid == 0) sh.comp = atomicAdd(work_counter, 1u);

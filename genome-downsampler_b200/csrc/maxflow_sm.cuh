@@ -634,10 +634,10 @@ __device__ __forceinline__ uint32_t mf2_bfs(Mf2Shared& sh, bool first, unsigned 
 template <int THREADS>
 __global__ void __launch_bounds__(THREADS, THREADS == 256 ? 2 : 1)
 k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __restrict__ comp_hi,
-             uint32_t n_comp, uint32_t* work_counter, uint32_t* qF_g, uint32_t* qT_g, uint32_t* qN_g,
+             uint32_t* work_counter, uint32_t* qF_g, uint32_t* qT_g, uint32_t* qN_g,
              uint32_t* qH_g, SolveParams P, CompStats* __restrict__ stats, uint32_t smem_bytes,
              uint32_t qcap, uint32_t* __restrict__ fb_list, uint32_t* fb_count, uint32_t allow_optr,
-             const uint32_t* __restrict__ n_comp_dev /* non-null: the count lives on the device */,
+             const uint32_t* __restrict__ n_comp_dev,
              MfTotals* __restrict__ totals, uint32_t allow_warp) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Mf2Shared& sh = *reinterpret_cast<Mf2Shared*>(smem_raw);
@@ -646,7 +646,7 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
     const uint32_t node_cap_bytes = smem_bytes - kMf2HeaderBytes - 16u * qcap;
     const uint32_t tid = threadIdx.x;
     const uint32_t lane = lane_id();
-    if (n_comp_dev) n_comp = *n_comp_dev;
+    const uint32_t n_comp = *n_comp_dev;
 
     for (;;) {
         if (tid == 0) sh.comp = atomicAdd(work_counter, 1u);

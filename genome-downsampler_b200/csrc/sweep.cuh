@@ -53,7 +53,7 @@ __device__ __forceinline__ void cp_async_wait_all() {
 template <int W, int CAP>
 __global__ void __launch_bounds__(kSweepWarps * 32)
 k_sweep(SweepGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __restrict__ comp_hi,
-        uint32_t n_comp, const uint32_t* __restrict__ n_comp_dev, uint32_t M, uint32_t* work_counter,
+        const uint32_t* __restrict__ n_comp_dev, uint32_t M, uint32_t* work_counter,
         unsigned long long* __restrict__ fail /* += positions whose pool ran dry (never) */) {
     extern __shared__ __align__(16) unsigned char sw_raw[];
     const uint32_t warp = threadIdx.x >> 5, lane = lane_id();
@@ -64,7 +64,7 @@ k_sweep(SweepGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __re
     uint2* stage = reinterpret_cast<uint2*>(pend + W);
     uint32_t* rows = reinterpret_cast<uint32_t*>(stage + 2 * CAP);
     uint32_t* needs = rows + 2 * 34;
-    if (n_comp_dev) n_comp = *n_comp_dev;
+    const uint32_t n_comp = *n_comp_dev;
     for (;;) {
         uint32_t c = 0;
         if (lane == 0) c = atomicAdd(work_counter, 1u);
@@ -155,7 +155,7 @@ k_sweep(SweepGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __re
 template <int W, int CAP>
 __global__ void __launch_bounds__(kSweepWarps * 32)
 k_sweep_warp(SweepGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t* __restrict__ comp_hi,
-        uint32_t n_comp, const uint32_t* __restrict__ n_comp_dev, uint32_t M, uint32_t* work_counter,
+        const uint32_t* __restrict__ n_comp_dev, uint32_t M, uint32_t* work_counter,
         unsigned long long* __restrict__ fail /* += positions whose pool ran dry (never) */) {
     extern __shared__ __align__(16) unsigned char sw_raw[];
     const uint32_t warp = threadIdx.x >> 5, lane = lane_id();
@@ -163,7 +163,7 @@ k_sweep_warp(SweepGraph G, const uint32_t* __restrict__ comp_lo, const uint32_t*
     uint32_t* pool = reinterpret_cast<uint32_t*>(sw_raw) + (size_t)warp * (2 * W + 4 * CAP);
     uint32_t* pend = pool + W;
     uint2* stage = reinterpret_cast<uint2*>(pend + W);
-    if (n_comp_dev) n_comp = *n_comp_dev;
+    const uint32_t n_comp = *n_comp_dev;
     for (;;) {
         uint32_t c = 0;
         if (lane == 0) c = atomicAdd(work_counter, 1u);

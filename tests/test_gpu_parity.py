@@ -559,8 +559,7 @@ def test_maxflow_kernels_agree(solver, O):
                             verify=True)
         c = _solve_with_env(solver, {"GDS_MF_OPTR": "0"}, s, e, Ls, M, read_off=off, params=prm)
         # heavy components stay in the shared-memory kernel (its warp passes) instead of k_maxflow
-        d = _solve_with_env(solver, {"GDS_MF_WARP": "1", "GDS_SYNC": "1"}, s, e, Ls, M, read_off=off,
-                            params=prm)
+        d = _solve_with_env(solver, {"GDS_MF_WARP": "1"}, s, e, Ls, M, read_off=off, params=prm)
         for key in COUNTERS:
             assert a[key] == b[key] == c[key] == d[key], key
         assert np.array_equal(a.kept_bitmap, d.kept_bitmap)
@@ -764,13 +763,15 @@ def test_minimum_cardinality_sweep(solver, O):
                      params=(64, 150, 1, 0, NOSEG, 0, 1))
 
 
-VERDICT_PATHS = {  # bundle path: (reference length, gds_params, length hints?, environment)
-    "sort_hints": (30_000, PRM + (0, 1), True, {}),
-    "sort_no_hints": (30_000, PRM + (0, 1), False, {}),
-    "segmented": (100_000, (64, 150, 1, 0, 8192, 1), True, {}),
-    "direct_sync": (30_000, PRM + (0, 2), True, {"GDS_SYNC": "1"}),
-    "direct_lazy": (30_000, PRM + (0, 2), True, {}),
-    "global_hist": (100_000, (64, 150, 1, 0, 8192, 0), True, {}),
+VERDICT_PATHS = {  # bundle path: (reference length, gds_params, length hints)
+    "sort_hints": (30_000, PRM + (0, 1), (150, 150)),
+    "sort_no_hints": (30_000, PRM + (0, 1), None),
+    "segmented": (100_000, (64, 150, 1, 0, 8192, 1), (150, 150)),
+    # several read lengths: the bundle count is read back for the in-CSR sort, and the verdict with
+    # it (15 001 nodes x 3 lengths fit the shared-memory histogram)
+    "direct_several_lengths": (15_000, PRM + (0, 2), (150, 152)),
+    "direct_one_length": (30_000, PRM + (0, 2), (150, 150)),
+    "global_hist": (100_000, (64, 150, 1, 0, 8192, 0), (150, 150)),
 }
 
 
@@ -779,30 +780,23 @@ VERDICT_PATHS = {  # bundle path: (reference length, gds_params, length hints?, 
 def test_input_verdicts_on_every_bundle_path(pkg, solver, O, path, kind):
     # bad reads fail the call with the exact code and message (with the number of bad reads where
     # the path counts them), and the context solves the next call as if nothing had happened
-    import os
-    L, prm, hints, env = VERDICT_PATHS[path]
+    L, prm, lh = VERDICT_PATHS[path]
     s, e, _, _ = O.gen_reads(4100, 20_000, L, 150)
     idx = np.array([11, 5_000, 39_000])
     bad_s, bad_e = s.copy(), e.copy()
     if kind == "range":  # end >= ref_len, length still 150
         bad_s[idx] = L - 100; bad_e[idx] = L + 49
         code, what, count = 2, "reads with start > end or end >= ref_len", len(idx)
-    else:  # length 149 under hints of exactly 150
+    else:  # length 149, under the shortest hinted length of 150
         bad_e[idx] = bad_s[idx] + 148
         code, what = 1, "reads outside the len_min/len_max hints"
         count = 1 if path == "segmented" else len(idx)  # k_validate only reports the bounds there
-    lh = (150, 150) if hints else None
-    os.environ.update(env)
-    try:
-        good = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
-        with pytest.raises(pkg.GdsError) as ei:
-            solver.solve(bad_s, bad_e, L, 40, params=prm, len_hint=lh)
-        again = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
-    finally:
-        for k in env:
-            del os.environ[k]
+    good = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
+    with pytest.raises(pkg.GdsError) as ei:
+        solver.solve(bad_s, bad_e, L, 40, params=prm, len_hint=lh)
+    again = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
     assert ei.value.code == code
     assert str(ei.value).endswith(": %d %s" % (count, what)), str(ei.value)
-    want_path = {"direct_sync": 1, "direct_lazy": 1, "global_hist": 2}.get(path, 0)
+    want_path = {"direct_several_lengths": 1, "direct_one_length": 1, "global_hist": 2}.get(path, 0)
     assert good.bundle_path == want_path and good.verify_violations == 0
     assert np.array_equal(again.kept_bitmap, good.kept_bitmap) and again.n_kept == good.n_kept

@@ -4,7 +4,7 @@ NumPy reference at the sizes, alignments and key widths where such kernels go wr
 buffer of the harness sits between guard words; every call asserts that they are intact.
 
 End to end: the radix sort's ballot ranking (the fallback for devices where shared-memory atomics
-do not rank in lane order) against the oracle, and both branches of the lazy selection retry."""
+do not rank in lane order) against the oracle, and both branches of the selection retry."""
 import ctypes as C
 import importlib.util
 import os
@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 from conftest import PRM, ROOT
-from test_gpu_parity import COUNTERS, _solve_with_env, assert_parity
+from test_gpu_parity import COUNTERS, assert_parity
 
 gpu = pytest.mark.gpu
 
@@ -587,10 +587,11 @@ def test_ballot_rank_several_read_lengths(solver, ballot_solver, O):
     assert_ballot_matches(O, solver, ballot_solver, s, e, [9_200, 30_000], off, 200, PRM + (0, 1))
 
 
-# ------------------------------------------------------------------ lazy selection retry
-def _lazy_then_sync(pkg, O, s, e, L, M, prm, len_hint):
-    """The lazy call on a fresh context (empty candidate buffer), profiled; then the same call with
-    GDS_SYNC=1 (readbacks between the kernels, not lazy).  Both must match the oracle."""
+# ------------------------------------------------------------------ selection retry
+def _retry_then_unhinted(pkg, O, s, e, L, M, prm, len_hint):
+    """The call on a fresh context (empty candidate buffer), profiled; then the same call again, and
+    once more without the length hints (k_validate finds the bounds, then the same selection).  All
+    must match the oracle."""
     fresh = pkg.Solver(0)
     try:
         fresh.kernel_profile_reset()
@@ -598,29 +599,29 @@ def _lazy_then_sync(pkg, O, s, e, L, M, prm, len_hint):
                         profile=True)
         prof = {k["name"]: k["launches"] for k in fresh.kernel_profile()}
         again = fresh.solve(s, e, L, M, params=prm, verify=True, len_hint=len_hint)
-        sync = _solve_with_env(fresh, {"GDS_SYNC": "1"}, s, e, L, M, params=prm, verify=True,
-                               want_vectors=True, len_hint=len_hint)
+        unhinted = fresh.solve(s, e, L, M, params=prm, verify=True, want_vectors=True)
     finally:
         fresh.close()
     off = np.array([0, len(s)], np.uint64)
     assert_parity(O, r, s, e, [L], off, M, prm[:5])
-    assert_parity(O, sync, s, e, [L], off, M, prm[:5])
+    assert_parity(O, unhinted, s, e, [L], off, M, prm[:5])
     for key in COUNTERS:
-        assert r[key] == sync[key] == again[key], key
-    assert np.array_equal(r.kept_bitmap, sync.kept_bitmap)
+        assert r[key] == unhinted[key] == again[key], key
+    assert np.array_equal(r.kept_bitmap, unhinted.kept_bitmap)
     assert np.array_equal(r.kept_bitmap, again.kept_bitmap)
-    return r, again, sync, prof
+    return r, again, unhinted, prof
 
 
 @gpu
-def test_lazy_retry_grows_the_candidate_buffer(pkg, O):
+def test_selection_retry_grows_the_candidate_buffer(pkg, O):
     # config 4's density (10 reads per start, one length, M = 500: coverage 1500) on a segmented
-    # reference: the global histogram path, lazy.  Most reads sit in partial bundles, more than the
-    # N/8 candidate slots a fresh context starts with: the first selection overflows and is repeated.
+    # reference: the global histogram path.  Most reads sit in partial bundles, more than the N/8
+    # candidate slots a fresh context starts with: the first selection overflows and is repeated.
     L, M = 200_000, 500
     s, e, _, _ = O.gen_reads(4040, 1_000_000, L, 150)
-    r, again, sync, prof = _lazy_then_sync(pkg, O, s, e, L, M, (64, 150, 1, 0, 8192, 0), (150, 150))
-    assert r.bundle_path == 2 and sync.bundle_path == 2
+    r, again, unhinted, prof = _retry_then_unhinted(pkg, O, s, e, L, M, (64, 150, 1, 0, 8192, 0),
+                                                    (150, 150))
+    assert r.bundle_path == 2 and unhinted.bundle_path == 2
     assert r.partial_candidates > r.n_filtered // 8
     assert prof["direct_classify"] == 2, prof  # the selection ran twice
     # the buffer has grown: the same call on the same context selects once
@@ -628,12 +629,12 @@ def test_lazy_retry_grows_the_candidate_buffer(pkg, O):
 
 
 @gpu
-def test_lazy_retry_forces_the_ordered_walk(pkg, O):
+def test_selection_retry_forces_the_ordered_walk(pkg, O):
     # 5000 identical reads, M = 17: one partial bundle of more than 2048 reads is too large for one
-    # warp's ranking, so the lazy call repeats the selection with the ordered walk
+    # warp's ranking, so the call repeats the selection with the ordered walk
     s = np.full(5000, 10, np.uint32)
     e = np.full(5000, 60, np.uint32)
-    r, again, sync, prof = _lazy_then_sync(pkg, O, s, e, 100, 17, PRM + (0, 0), (51, 51))
+    r, again, unhinted, prof = _retry_then_unhinted(pkg, O, s, e, 100, 17, PRM + (0, 0), (51, 51))
     assert r.bundle_path == 1 and r.n_bundles == 1
     assert prof.get("direct_mark") == 1 and prof.get("direct_walk") == 1, prof
     assert pkg.Solver.bitmap_to_indices(r.kept_bitmap, 5000).tolist() == list(range(17))

@@ -18,6 +18,10 @@ def _cases(O):
     batch = dict(start=s, end=e, ref_len=[30_000] * 3, read_off=off)
     sl, el, _, _ = O.gen_reads(620, 120_000, 150_000, 150)
     seg = dict(start=sl, end=el, ref_len=150_000)
+    # reads of 150, 151 and 152 positions: 3 x 15 001 keys fit the shared-memory histogram
+    sv, ev, _, _ = O.gen_reads(640, 40_000, 15_000, 150)
+    ev = np.where(ev + 2 < 15_000, ev + np.arange(len(ev)) % 3, ev).astype(np.uint32)
+    several = dict(start=sv, end=ev, ref_len=15_000)
     bed, tsv = O.artic_scheme()
     a0, a1 = O.parse_amplicons(bed, tsv)
     sf, ef, q, ln = O.gen_reads_amplicon(630, 50_000, 30_000, a0, a1)
@@ -26,8 +30,8 @@ def _cases(O):
     # name: (inputs, M, solve keywords, environment)
     return {
         "radix_sort": (batch, 60, dict(params=PRM + (0, 1)), {}),
-        "direct_lazy": (batch, 60, dict(params=PRM + (0, 2), len_hint=(150, 150)), {}),
-        "direct_sync": (batch, 60, dict(params=PRM + (0, 2), len_hint=(150, 150)), {"GDS_SYNC": "1"}),
+        "direct_one_length": (batch, 60, dict(params=PRM + (0, 2), len_hint=(150, 150)), {}),
+        "direct_several_lengths": (several, 60, dict(params=PRM + (0, 2), len_hint=(150, 152)), {}),
         "global_hist_segmented": (seg, 60, dict(params=(64, 150, 1, 0, 8192, 0)), {}),
         "pair_filter": (filt, 100, dict(params=PRM), {}),
         "direct_walk": (batch, 60, dict(params=PRM + (0, 2)), {"GDS_DIRECT_SELECT": "walk"}),
@@ -37,8 +41,8 @@ def _cases(O):
     }
 
 
-PATHS = ["radix_sort", "direct_lazy", "direct_sync", "global_hist_segmented", "pair_filter",
-         "direct_walk", "maxflow_global", "express", "min_cardinality"]
+PATHS = ["radix_sort", "direct_one_length", "direct_several_lengths", "global_hist_segmented",
+         "pair_filter", "direct_walk", "maxflow_global", "express", "min_cardinality"]
 
 
 @pytest.mark.parametrize("path", PATHS)
@@ -56,7 +60,7 @@ def test_profile_accounts_for_every_launch(solver, O, path):
         for k in env:
             del os.environ[k]
     assert prof.kernel_launches > 0
-    # (the two calls' launch counts may differ: the lazy path repeats its selection once when the
+    # (the two calls' launch counts may differ: a histogram path repeats its selection once when the
     # context's candidate buffer is still smaller than the call needs)
     assert sum(k["launches"] for k in stats) == prof.kernel_launches
     assert all(k["name"] for k in stats)
@@ -65,5 +69,7 @@ def test_profile_accounts_for_every_launch(solver, O, path):
                 "sort_passes", "verify_violations"):
         assert prof[key] == plain[key], key
     assert plain.verify_violations == 0
+    if path.startswith("direct_"):
+        assert plain.bundle_path == 1
     if path == "pair_filter":
         assert np.array_equal(prof.pair_pass, plain.pair_pass)
