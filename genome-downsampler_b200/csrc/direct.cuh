@@ -162,6 +162,9 @@ k_direct_count(const uint32_t* __restrict__ ghist, uint32_t ktot, uint32_t* __re
 
 // Writes what k_bundle_fill writes on the sort path (bundle record, in-CSR key, difference array,
 // CSR degrees) plus the bundle's histogram slot (K5 puts the bundle's flow there).
+// One read length takes k_direct_graph below, except with forced cuts: the forced-bundle test
+// compares the uncapped-position count at a bundle's end, R nodes to the right of a node, which a
+// left-to-right pass does not have yet.  The one_len branch here serves that case.
 __global__ void __launch_bounds__(kDkThreads)
 k_direct_bundles(const uint32_t* __restrict__ ghist, uint32_t ktot, DirectLayout dl,
                  const uint32_t* __restrict__ tile_offs, BundleRec* __restrict__ bund,
@@ -222,6 +225,318 @@ k_direct_bundles(const uint32_t* __restrict__ ghist, uint32_t ktot, DirectLayout
         }
         ++b;
     }
+}
+
+// ---- one read length: the whole flow graph in one pass --------------------------------------------
+// With one read length R and no forced cuts, every node and bundle array K3, K5 and K6 read follows
+// from the histogram h alone.  Node v of sample k is slot j = v - node_base[k] of the sample's region:
+//   diff[v]  = h[j] - h[j-R]         (reads starting at v minus reads ending at v)
+//   out-arc  iff h[j] != 0, in-arc iff h[j-R] != 0   (at most one bundle starts / ends at a node)
+//   the in-CSR order is the bundle order, so the in-arc of v is bundle indeg[v] and starts at v - R.
+// One pass over tiles of the node space carries four exclusive prefixes with the decoupled look-back
+// of scan.cuh (status words tile*4 + 0..3): coverage, bundles starting before v, bundles ending
+// before v, and components starting before v.  The first three are published as soon as the tile
+// has its loads; a component starts where the coverage rises from 0, so that word follows once the
+// tile knows its coverage prefix.  Coverage does not leak from one sample into the next: each
+// sample's diff sums to 0.  Every output is written once, the same as the chain it replaces
+// (direct_count, its scan, direct_bundles, the node scans, node_finalize, the component scan,
+// comp_write and in_src) wrote it.
+// A lane holds 4 x 4 consecutive nodes (4-aligned: the node arrays take 16-byte stores); 4 tiles of
+// 64 registers per thread sit on each SM, so one tile's look-back is covered by the others' loads.
+constexpr int kDgThreads = 256;
+constexpr int kDgRows = 4;
+constexpr int kDgWarpSpan = 32 * 4 * kDgRows;
+constexpr int kDgTile = kDgThreads / 32 * kDgWarpSpan;  // 4096 nodes
+
+struct DirectGraphOut {
+    BundleRec* bund;
+    uint32_t *b_t, *b_slot, *ident, *in_src;
+    int32_t* diff;
+    uint32_t *excl, *outdeg, *indeg;
+    NodeRec* node;
+    uint32_t* d_snap;
+    int32_t* dem_v;
+    uint32_t* in1;
+    uint32_t *comp_lo, *comp_hi;
+    uint32_t* cov_capped;  // null unless the call asks for it
+    int32_t* demand;       // likewise
+    uint32_t *n_bundles, *n_comp;
+    unsigned long long *fstar, *res_supply;
+};
+
+// Histogram slot and sample-local index of nodes v0 .. v0+3 (the four may run into the next
+// sample; past the last node they mean nothing).  Samples k0 .. k1 hold the tile's nodes.
+__device__ __forceinline__ void dg_locate(const DirectLayout& dl, uint32_t k0, uint32_t k1, uint32_t v0,
+                                          uint32_t n_nodes, uint32_t (&slot)[4], uint32_t (&j)[4]) {
+    const uint32_t vs = min(v0, n_nodes - 1);
+    uint32_t lo = k0, hi = k1 + 1;  // node_base[lo] <= vs < node_base[hi]
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (dl.node_base[mid] <= vs) lo = mid;
+        else hi = mid;
+    }
+    uint32_t k = lo, nb = dl.node_base[k], nb1 = dl.node_base[k + 1], kb = dl.kbase[k];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const uint32_t v = v0 + q;
+        if (v >= nb1 && v < n_nodes) {
+            do {
+                ++k;
+            } while (dl.node_base[k + 1] <= v);
+            nb = dl.node_base[k];
+            nb1 = dl.node_base[k + 1];
+            kb = dl.kbase[k];
+        }
+        j[q] = v - nb;
+        slot[q] = kb + j[q];
+    }
+}
+
+// Tiles cover nodes [0, n_nodes]: node n_nodes is the sentinel that closes the CSR ranges.
+__global__ void __launch_bounds__(kDgThreads, 4)
+k_direct_graph(const uint32_t* __restrict__ ghist, DirectLayout dl, uint32_t n_nodes, uint32_t M,
+               uint32_t in_first /* k_maxflow_sm runs: {start, bundle} of the in-arc over {d, stamp} */,
+               DirectGraphOut o, unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket,
+               uint32_t epoch, uint32_t n_tiles) {
+    __shared__ uint32_t s_tile, s_k0, s_k1;
+    __shared__ uint32_t s_prefix[4];
+    __shared__ uint32_t wtot[3][kDgThreads / 32];
+    __shared__ uint4 s_h[kDgTile / 4], s_hin[kDgTile / 4];  // h[j] and h[j-R] of the tile's nodes
+    // a row's bundles (start node, multiplicity, slot) on their way to coalesced stores
+    __shared__ uint32_t s_bv[kDgThreads / 32][128], s_bm[kDgThreads / 32][128], s_bs[kDgThreads / 32][128];
+    const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
+    // tiles are handed out in launch order, so every predecessor of a tile is already running
+    if (threadIdx.x == 0) {
+        const uint32_t t = atomicAdd(ticket, 1u);
+        s_tile = t;
+        s_k0 = find_u32(dl.node_base, dl.ns, min(t * kDgTile, n_nodes - 1));
+        s_k1 = find_u32(dl.node_base, dl.ns, min(t * kDgTile + kDgTile - 1, n_nodes - 1));
+    }
+    __syncthreads();
+    const uint32_t tile = s_tile, k0 = s_k0, k1 = s_k1;
+    const uint32_t R = dl.minlen;
+    const uint32_t wbase = tile * kDgTile + warp * kDgWarpSpan;
+    // this lane's 4 nodes of row r sit at s_h[row(r)] (each thread reads back only what it wrote)
+    auto row = [&](int r) { return warp * (kDgWarpSpan / 4) + r * 32 + lane; };
+    uint32_t hv[4], hin[4];
+    auto fetch = [&](int r) {
+        const uint4 a = s_h[row(r)], b = s_hin[row(r)];
+        hv[0] = a.x; hv[1] = a.y; hv[2] = a.z; hv[3] = a.w;
+        hin[0] = b.x; hin[1] = b.y; hin[2] = b.z; hin[3] = b.w;
+    };
+    {  // loads warp-striped (32 consecutive nodes per load), stored where the row layout reads them
+        uint32_t* sh = reinterpret_cast<uint32_t*>(s_h) + warp * kDgWarpSpan;
+        uint32_t* si = reinterpret_cast<uint32_t*>(s_hin) + warp * kDgWarpSpan;
+        uint32_t lo = k0, hi = k1 + 1;  // the sample of the warp's first node
+        const uint32_t vs = min(wbase, n_nodes - 1);
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (dl.node_base[mid] <= vs) lo = mid;
+            else hi = mid;
+        }
+        uint32_t k = lo, nb = dl.node_base[k], nb1 = dl.node_base[k + 1], kb = dl.kbase[k];
+        if (wbase + kDgWarpSpan <= nb1) {  // the warp's nodes lie in one sample (and before the end)
+            const uint32_t j0 = wbase - nb + lane;
+            const uint32_t* h = ghist + kb + j0;
+#pragma unroll
+            for (int m = 0; m < kDgWarpSpan / 32; ++m) {
+                sh[m * 32 + lane] = h[m * 32];
+                si[m * 32 + lane] = j0 + m * 32 >= R ? h[m * 32 - (int)R] : 0u;
+            }
+        } else {
+#pragma unroll 4
+            for (int m = 0; m < kDgWarpSpan / 32; ++m) {
+                const uint32_t v = wbase + m * 32 + lane;
+                uint32_t x = 0, y = 0;
+                if (v < n_nodes) {
+                    while (v >= nb1) {  // nodes only grow with m
+                        ++k;
+                        nb = dl.node_base[k];
+                        nb1 = dl.node_base[k + 1];
+                        kb = dl.kbase[k];
+                    }
+                    const uint32_t j = v - nb;
+                    x = ghist[kb + j];
+                    y = j >= R ? ghist[kb + j - R] : 0u;
+                }
+                sh[m * 32 + lane] = x;
+                si[m * 32 + lane] = y;
+            }
+        }
+        __syncwarp();
+    }
+    // lane offsets within the warp, row by row: coverage, and (out-arcs | in-arcs << 16)
+    uint32_t rd[kDgRows], ro[kDgRows], wd = 0, wo = 0;
+#pragma unroll
+    for (int r = 0; r < kDgRows; ++r) {
+        fetch(r);
+        uint32_t sd = 0, so = 0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            sd += hv[q] - hin[q];
+            so += (hv[q] != 0 ? 1u : 0u) + (hin[q] != 0 ? 0x10000u : 0u);
+        }
+        const uint32_t id = warp_incl_scan(sd), io = warp_incl_scan(so);
+        rd[r] = wd + id - sd;
+        ro[r] = wo + io - so;
+        wd += __shfl_sync(0xffffffffu, id, 31);
+        wo += __shfl_sync(0xffffffffu, io, 31);
+    }
+    if (lane == 0) {
+        wtot[0][warp] = wd;
+        wtot[1][warp] = wo;
+    }
+    __syncthreads();
+    uint32_t offd = 0, offo = 0, totd = 0, toto = 0;
+#pragma unroll
+    for (int w = 0; w < kDgThreads / 32; ++w) {
+        const uint32_t td = wtot[0][w], to = wtot[1][w];
+        offd += w < (int)warp ? td : 0u;
+        offo += w < (int)warp ? to : 0u;
+        totd += td;
+        toto += to;
+    }
+    if (warp < 3) {
+        const uint32_t total = warp == 0 ? totd : warp == 1 ? (toto & 0xffffu) : (toto >> 16);
+        const uint32_t p = lookback_prefix(status, tile * 4 + warp, 4, tile == 0, total, epoch);
+        if (lane == 0) s_prefix[warp] = p;
+    }
+    __syncthreads();
+    const uint32_t pd = s_prefix[0] + offd;
+    const uint32_t po = s_prefix[1] + (offo & 0xffffu), pi = s_prefix[2] + (offo >> 16);
+    // components start where the coverage rises from 0 (past the last node it stays 0)
+    uint32_t rc[kDgRows], wc = 0;
+#pragma unroll
+    for (int r = 0; r < kDgRows; ++r) {
+        fetch(r);
+        uint32_t cov = pd + rd[r], sc = 0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const uint32_t covR = cov + hv[q] - hin[q];
+            sc += (cov == 0 && covR != 0) ? 1u : 0u;
+            cov = covR;
+        }
+        const uint32_t ic = warp_incl_scan(sc);
+        rc[r] = wc + ic - sc;
+        wc += __shfl_sync(0xffffffffu, ic, 31);
+    }
+    if (lane == 0) wtot[2][warp] = wc;
+    __syncthreads();
+    uint32_t offc = 0, totc = 0;
+#pragma unroll
+    for (int w = 0; w < kDgThreads / 32; ++w) {
+        const uint32_t t = wtot[2][w];
+        offc += w < (int)warp ? t : 0u;
+        totc += t;
+    }
+    if (warp == 3) {
+        const uint32_t p = lookback_prefix(status, tile * 4 + 3, 4, tile == 0, totc, epoch);
+        if (lane == 0) s_prefix[3] = p;
+    }
+    __syncthreads();
+    const uint32_t pc = s_prefix[3] + offc;
+    unsigned long long src = 0;
+    // (one row at a time: unrolled, the rows' stores would need 96 registers)
+    auto pick = [](const uint32_t (&a)[kDgRows], int r) {
+        uint32_t x = a[0];
+#pragma unroll
+        for (int i = 1; i < kDgRows; ++i) x = r == i ? a[i] : x;
+        return x;
+    };
+#pragma unroll 1
+    for (int r = 0; r < kDgRows; ++r) {
+        fetch(r);
+        const uint32_t v0 = wbase + r * 128 + lane * 4;
+        const uint32_t rdr = pick(rd, r), ror = pick(ro, r), rcr = pick(rc, r);
+        const uint32_t cov0 = pd + rdr, b0 = po + (ror & 0xffffu), ib0 = pi + (ror >> 16);
+        // the node arrays, one at a time (16-byte stores; the end of the last tile one by one)
+        auto put = [&](uint32_t* a, uint32_t x0, uint32_t x1, uint32_t x2, uint32_t x3, uint32_t last) {
+            if (v0 + 3 < n_nodes) {
+                *reinterpret_cast<uint4*>(a + v0) = make_uint4(x0, x1, x2, x3);
+            } else {
+                if (v0 <= last) a[v0] = x0;
+                if (v0 + 1 <= last) a[v0 + 1] = x1;
+                if (v0 + 2 <= last) a[v0 + 2] = x2;
+                if (v0 + 3 <= last) a[v0 + 3] = x3;
+            }
+        };
+        const uint32_t d0 = hv[0] - hin[0], d1 = hv[1] - hin[1], d2 = hv[2] - hin[2],
+                       d3 = hv[3] - hin[3];
+        const uint32_t c1 = cov0 + d0, c2 = c1 + d1, c3 = c2 + d2, c4 = c3 + d3;  // covR of each node
+        put(reinterpret_cast<uint32_t*>(o.diff), d0, d1, d2, d3, n_nodes);
+        put(o.excl, cov0, c1, c2, c3, n_nodes);
+        auto dem = [&](uint32_t l, uint32_t rr) { return (uint32_t)((int32_t)min(l, M) - (int32_t)min(rr, M)); };
+        put(reinterpret_cast<uint32_t*>(o.dem_v), dem(cov0, c1), dem(c1, c2), dem(c2, c3), dem(c3, c4), n_nodes - 1);
+        auto nz = [&](uint32_t x) { return x != 0 ? 1u : 0u; };
+        const uint32_t o1 = b0 + nz(hv[0]), o2 = o1 + nz(hv[1]), o3 = o2 + nz(hv[2]);
+        put(o.outdeg, b0, o1, o2, o3, n_nodes);
+        const uint32_t i1 = ib0 + nz(hin[0]), i2 = i1 + nz(hin[1]), i3 = i2 + nz(hin[2]);
+        put(o.indeg, ib0, i1, i2, i3, n_nodes);
+        // start node of the node's only in-arc
+        auto src_of = [&](uint32_t hi, uint32_t v) { return hi ? v - R : 0xffffffffu; };
+        put(o.in1, src_of(hin[0], v0), src_of(hin[1], v0 + 1), src_of(hin[2], v0 + 2),
+            src_of(hin[3], v0 + 3), n_nodes);
+        put(o.d_snap, kLabelInf, kLabelInf, kLabelInf, kLabelInf, n_nodes - 1);
+        // per node: the record, the components, the bundle
+        uint32_t slot[4], j[4];
+        dg_locate(dl, k0, k1, v0, n_nodes, slot, j);
+        uint32_t cov = cov0, b = b0, ib = ib0, cs = pc + rcr;
+        const uint32_t rb = __shfl_sync(0xffffffffu, b0, 0);  // the row's first bundle
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const uint32_t v = v0 + q, h = hv[q], hi = hin[q];
+            const uint32_t covR = cov + h - hi;
+            const int32_t dm = (int32_t)min(cov, M) - (int32_t)min(covR, M);
+            const bool start = cov == 0 && covR != 0;
+            if (v < n_nodes) {
+                uint4* nr = reinterpret_cast<uint4*>(&o.node[v]);
+                const bool inf = !(in_first && hi);
+                nr[0] = make_uint4(inf ? kLabelInf : v - R, inf ? 0u : ib, (uint32_t)(dm < 0 ? -dm : 0), 0u);
+                nr[1] = make_uint4((uint32_t)(dm > 0 ? dm : 0), 0u, b, ib);
+                if (o.cov_capped) o.cov_capped[v] = min(covR, M);
+                if (o.demand) o.demand[v] = dm;
+                if (dm < 0) src += (unsigned long long)(-dm);
+                // components are disjoint runs: the end at v closes the one opened last
+                if (start) o.comp_lo[cs] = v;
+                if (cov != 0 && covR == 0) o.comp_hi[cs - 1] = v;
+                if (h) {
+                    s_bv[warp][b - rb] = v;
+                    s_bm[warp][b - rb] = h;
+                    s_bs[warp][b - rb] = slot[q];
+                }
+            } else if (v == n_nodes) {  // sentinel record; the counts stay on the device
+                uint4* nr = reinterpret_cast<uint4*>(&o.node[v]);
+                nr[0] = make_uint4(0u, 0u, 0u, 0u);
+                nr[1] = make_uint4(0u, 0u, b, ib);
+                *o.n_bundles = b;
+                *o.n_comp = cs;
+            }
+            cs += start ? 1u : 0u;
+            b += h != 0 ? 1u : 0u;
+            ib += hi != 0 ? 1u : 0u;
+            cov = covR;
+        }
+        // the row's bundles are consecutive: written by consecutive lanes (one lane per bundle and
+        // its own 4-node group scattered every store over 16-32 sectors)
+        const uint32_t nrow = __shfl_sync(0xffffffffu, b, 31) - rb;
+        __syncwarp();
+        for (uint32_t x = lane; x < nrow; x += 32) {
+            const uint32_t bb = rb + x, v = s_bv[warp][x];
+            reinterpret_cast<uint4*>(o.bund)[bb] = make_uint4(v + R, s_bm[warp][x], 0u, v);  // {t, mult, f, s}
+            o.b_t[bb] = v + R;
+            o.b_slot[bb] = s_bs[warp][x];
+            o.ident[bb] = bb;
+            o.in_src[bb] = v;
+        }
+        __syncwarp();
+    }
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) src += __shfl_xor_sync(0xffffffffu, src, s);
+    if (lane == 0 && src) {
+        atomicAdd(o.fstar, src);
+        atomicAdd(o.res_supply, src);
+    }
+    if (threadIdx.x == 0 && tile == n_tiles - 1) *ticket = 0;  // every ticket is out by now
 }
 
 // ---- K5 direct ---------------------------------------------------------------------------------

@@ -464,8 +464,13 @@ struct SolveCall {
     int nodebits;
     int32_t* odiff;
     uint32_t* oexcl;
+    // what K3 will run, decided before the graph is built (plan_solve)
+    bool forced_cuts;
+    uint32_t express_on;
+    Mf2Plan mf2;
     // K2
     DirectPlan direct;
+    bool direct_graph;  // k_direct_graph builds the nodes, components and in-arcs (one read length)
     uint32_t B;  // exact when the host needs it (radix sorts over the bundles), else a bound
     uint32_t* sorted_idx;
     int sort_passes;
@@ -475,7 +480,6 @@ struct SolveCall {
     NodeRec* node;
     uint32_t* d_snap;
     int32_t* dem_v;
-    bool forced_cuts;
     uint32_t* fmult;
     uint8_t* dead;
     uint32_t n_comp_cap;  // a bound; the count is ds->n_comp
@@ -496,10 +500,15 @@ StatsBlock validate_reads(gds_ctx* c, const SolveCall& sc) {
     return read_input_verdict(c, sc.ds);
 }
 
-// K2's per-node outputs, cleared: the difference array of the coverage and the out/in degrees
+// K2's per-node outputs: the difference array of the coverage and the out/in degrees
+Degrees degree_buffers(gds_ctx* c, uint32_t n_nodes) {
+    return Degrees{c->diff.get<int32_t>(n_nodes + 1), c->outdeg.get<uint32_t>(n_nodes + 1),
+                   c->indeg.get<uint32_t>(n_nodes + 1)};
+}
+
+// ... cleared
 Degrees alloc_degrees(gds_ctx* c, cudaStream_t st, uint32_t n_nodes, bool clear_diff = true) {
-    const Degrees d{c->diff.get<int32_t>(n_nodes + 1), c->outdeg.get<uint32_t>(n_nodes + 1),
-                    c->indeg.get<uint32_t>(n_nodes + 1)};
+    const Degrees d = degree_buffers(c, n_nodes);
     if (clear_diff) GDS_CUDA(cudaMemsetAsync(d.diff, 0, (n_nodes + 1) * sizeof(int32_t), st));
     else GDS_CUDA(cudaMemsetAsync(d.diff + n_nodes, 0, sizeof(int32_t), st));
     GDS_CUDA(cudaMemsetAsync(d.outdeg, 0, (n_nodes + 1) * sizeof(uint32_t), st));
@@ -615,6 +624,18 @@ struct BundleOut {
     Degrees d;
 };
 
+// The bundle buffers of a histogram path, sized for B bundles; the identity in-CSR when there is
+// one read length
+void bundle_buffers(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint32_t B, BundleOut& o) {
+    sc.B = B;
+    o.bund = c->bund.get<BundleRec>(B + 1);
+    o.b_t = c->b_t.get<uint32_t>(B + 1);
+    o.b_slot = c->b_slot.get<uint32_t>(B + 1);
+    o.ident = sc.minlen == sc.maxlen ? c->ident.get<uint32_t>(B + 1) : nullptr;
+    plan.on = true;
+    plan.in_bid = o.ident;
+}
+
 // What both histogram paths do once plan.ghist holds the counts: count the non-empty keys per
 // tile, scan, the bundle count (on the device; b_bound sizes the buffers), the bundle buffers and
 // the cleared degree arrays.  own_diff: the bundle kernel writes the whole difference array itself.
@@ -635,13 +656,9 @@ BundleOut histogram_bundles(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint64_
         d2h_sync(c, &B, tc + n_tiles, 1);
         read_input_verdict(c, sc.ds);
     }
-    sc.B = B;
-    BundleOut o{n_tiles, tc, c->bund.get<BundleRec>(B + 1), c->b_t.get<uint32_t>(B + 1),
-                c->b_slot.get<uint32_t>(B + 1),
-                sc.minlen == sc.maxlen ? c->ident.get<uint32_t>(B + 1) : nullptr};
+    BundleOut o{n_tiles, tc};
+    bundle_buffers(c, sc, plan, B, o);
     o.d = alloc_degrees(c, st, sc.plan.n_nodes, !(own_diff && B));
-    plan.on = true;
-    plan.in_bid = o.ident;
     return o;
 }
 
@@ -694,6 +711,12 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
     plan.ktot = ktot;
     plan.kmax = kmax;
     plan.n_items = n_items;
+    if (sc.direct_graph) {  // k_direct_graph (build_nodes) writes the bundles and every node array
+        BundleOut o{};
+        bundle_buffers(c, sc, plan, (uint32_t)std::min<uint64_t>(ktot, N), o);
+        degree_buffers(c, sc.plan.n_nodes);
+        return;
+    }
     // one read length: k_direct_bundles writes the difference array of every node itself
     const BundleOut o = histogram_bundles(c, sc, plan, N, nlen == 1);
     if (sc.B)
@@ -1211,6 +1234,29 @@ SegPlan plan_segments(const gds_reads* rd, const gds_params* prm, const std::vec
     return pl;
 }
 
+// What K3 runs, from the call's arguments and the segment plan alone: the graph build writes the
+// node records in the form the chosen kernel reads.
+void plan_solve(SolveCall& sc) {
+    // Forced reads out, cuts in (graph.cuh, DESIGN.md §4): bundles that cover a position with
+    // cov <= M get capacity 0 for the solve and their fixed flow goes into the demand; components
+    // are cut at every such position.  Not for the minimum-cardinality sweep (it walks all
+    // bundles itself) and not with gds_params.schedule = 1 (round 1's graph and schedule).
+    // ... and not below the supply at which the express schedule starts (kExpressMinSupply):
+    // with M = 100 (configs 1, 2, 5) the classic schedule on the uncut graph needs no more
+    // rounds than hops, and the three extra passes over nodes and bundles would cost config 5
+    // 0.25 ms of 5.75 (measured); gds_params.schedule = 2 applies them regardless.
+    sc.forced_cuts = sc.do_solve && sc.algorithm == 0 && sc.schedule != 1 &&
+                     (sc.schedule >= 2 || sc.M >= kExpressMinSupply);
+    // the express schedule (maxflow_sm.cuh): components with a supply of kExpressMinSupply or
+    // more — none when M is below that, and then nothing about the launch changes
+    uint32_t express_on = sc.schedule == 1 ? 0u : sc.schedule == 2 ? 2u : 1u;  // (3: the usual supply rule)
+    if (!sc.forced_cuts || (express_on == 1 && sc.M < kExpressMinSupply)) express_on = 0;
+    sc.express_on = express_on;
+    sc.mf2 = sc.do_solve && sc.algorithm == 0
+                 ? plan_maxflow_sm(sc.plan.comp_estimate, sc.plan.max_comp_nodes, express_on != 0, sc.knobs)
+                 : Mf2Plan{};
+}
+
 // K2: the bundles (arcs of equal start, end and length) and the node degrees.  Shared-memory
 // histogram, global-memory histogram or radix sort.
 void find_bundles(gds_ctx* c, SolveCall& sc) {
@@ -1235,6 +1281,7 @@ void find_bundles(gds_ctx* c, SolveCall& sc) {
                             direct_eligible(sc.rd, ns, sc.minlen, sc.maxlen, sc.S, sc.E);
     const bool use_gdirect = N > 0 && !use_direct && bmode != 1 &&
                              (uint64_t)n_nodes * ((uint64_t)sc.maxlen - sc.minlen + 1) <= kGDirectMaxKeys;
+    sc.direct_graph = use_direct && sc.minlen == sc.maxlen && !sc.forced_cuts;
     size_t n_items = N;
     uint32_t* cross_idx = nullptr;
     if (pl.split && N > 0 && !use_gdirect) {  // right parts of the reads that cross a cut
@@ -1274,41 +1321,23 @@ void find_bundles(gds_ctx* c, SolveCall& sc) {
     out->sort_passes = sc.sort_passes;
 }
 
-// Coverage and CSR row starts, the forced cuts, the node records, the components and the in-CSR
-void build_nodes(gds_ctx* c, SolveCall& sc) {
+// The graph build of every path but k_direct_graph's: scans, forced cuts, node records, components,
+// in-CSR order
+void build_nodes_chain(gds_ctx* c, SolveCall& sc, uint32_t* cov_dev, int32_t* dem_dev) {
     const uint32_t n_nodes = sc.plan.n_nodes, n_onodes = sc.n_onodes, B = sc.B, M = sc.M;
     const bool split = sc.plan.split;
     cudaStream_t st = sc.st;
-    gds_result* out = sc.out;
     unsigned long long* totals = sc.totals();
     const Degrees& d = sc.deg;
-    uint32_t* excl = sc.excl = c->excl.get<uint32_t>(n_nodes + 1);
+    uint32_t* excl = sc.excl;
     {  // coverage from the difference array and both CSR row starts: one launch
         ScanArrays sa{{reinterpret_cast<const uint32_t*>(d.diff), d.outdeg, d.indeg}, {excl, d.outdeg, d.indeg}};
         exclusive_scan_u32_multi(sa, 3, n_nodes + 1, c->scan, st);
     }
-    sc.node = c->node_rec.get<NodeRec>((size_t)n_nodes + 1);
-    sc.d_snap = c->n_dsnap.get<uint32_t>(n_nodes);
-    sc.dem_v = c->dem_v.get<int32_t>((size_t)n_nodes + 1);
     uint32_t* cstart = c->comp_start.get<uint32_t>(n_nodes + 1);
     uint32_t* cend = c->comp_end.get<uint32_t>(n_nodes + 1);
     GDS_CUDA(cudaMemsetAsync(cstart + n_nodes, 0, 4, st));
     GDS_CUDA(cudaMemsetAsync(cend + n_nodes, 0, 4, st));
-    // cov_capped / demand are reported on the ORIGINAL node space
-    uint32_t* cov_dev = nullptr;
-    int32_t* dem_dev = nullptr;
-    if (out->cov_capped) cov_dev = sc.out_dev ? out->cov_capped : c->cov_tmp.get<uint32_t>(n_onodes);
-    if (out->demand) dem_dev = sc.out_dev ? out->demand : c->dem_tmp.get<int32_t>(n_onodes);
-    // Forced reads out, cuts in (graph.cuh, DESIGN.md §4): bundles that cover a position with
-    // cov <= M get capacity 0 for the solve and their fixed flow goes into the demand; components
-    // are cut at every such position.  Not for the minimum-cardinality sweep (it walks all
-    // bundles itself) and not with gds_params.schedule = 1 (round 1's graph and schedule).
-    // ... and not below the supply at which the express schedule starts (kExpressMinSupply):
-    // with M = 100 (configs 1, 2, 5) the classic schedule on the uncut graph needs no more
-    // rounds than hops, and the three extra passes over nodes and bundles would cost config 5
-    // 0.25 ms of 5.75 (measured); gds_params.schedule = 2 applies them regardless.
-    sc.forced_cuts = sc.do_solve && sc.algorithm == 0 && sc.schedule != 1 &&
-                     (sc.schedule >= 2 || M >= kExpressMinSupply);
     int32_t* adj = nullptr;
     if (sc.forced_cuts && B) {
         uint32_t* unc = c->unc.get<uint32_t>((size_t)n_nodes + 1);
@@ -1340,16 +1369,10 @@ void build_nodes(gds_ctx* c, SolveCall& sc) {
     }
     uint32_t* sidx = c->comp_sidx.get<uint32_t>(n_nodes + 1);
     exclusive_scan_u32(cstart, sidx, n_nodes + 1, c->scan, st);
-    // the count stays on the device; on the host SegPlan::comp_estimate picks the K3 kernel and the
-    // grid, and the arrays are sized by the bound (a component has >= 2 nodes)
     GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_comp, sidx + n_nodes, 4, cudaMemcpyDeviceToDevice, st));
-    sc.n_comp_cap = n_nodes / 2 + 1;
-    sc.comp_lo = c->comp_lo.get<uint32_t>(sc.n_comp_cap + 1);
-    sc.comp_hi = c->comp_hi.get<uint32_t>(sc.n_comp_cap + 1);
     launch("comp_write", 16ull * n_nodes, k_comp_write, div_up(n_nodes, 256), 256, 0, st, cstart, cend,
            sidx, n_nodes, sc.comp_lo, sc.comp_hi);
     // in-CSR: bundle ids ordered by (end node, bundle id) = stable sort of ids by b_t
-    sc.in_bid = sc.direct.in_bid;  // single read length: bundle order is end order too
     if (B && !sc.in_bid) {
         uint32_t* tkA = c->tkA.get<uint32_t>(B);
         uint32_t* tkB = c->tkB.get<uint32_t>(B);
@@ -1361,6 +1384,47 @@ void build_nodes(gds_ctx* c, SolveCall& sc) {
         int w = radix_sort_pairs<uint32_t>(tkA, tvA, tkB, tvB, btm, sc.nodebits, c->radix, st,
                                            c->atomic_rank);
         sc.in_bid = w ? tvB : tvA;
+    }
+}
+
+// Coverage and CSR row starts, the forced cuts, the node records, the components and the in-CSR
+void build_nodes(gds_ctx* c, SolveCall& sc) {
+    const uint32_t n_nodes = sc.plan.n_nodes, n_onodes = sc.n_onodes, B = sc.B, M = sc.M;
+    cudaStream_t st = sc.st;
+    gds_result* out = sc.out;
+    unsigned long long* totals = sc.totals();
+    const Degrees& d = sc.deg;
+    uint32_t* excl = sc.excl = c->excl.get<uint32_t>(n_nodes + 1);
+    sc.node = c->node_rec.get<NodeRec>((size_t)n_nodes + 1);
+    sc.d_snap = c->n_dsnap.get<uint32_t>(n_nodes);
+    sc.dem_v = c->dem_v.get<int32_t>((size_t)n_nodes + 1);
+    // cov_capped / demand are reported on the ORIGINAL node space
+    uint32_t* cov_dev = nullptr;
+    int32_t* dem_dev = nullptr;
+    if (out->cov_capped) cov_dev = sc.out_dev ? out->cov_capped : c->cov_tmp.get<uint32_t>(n_onodes);
+    if (out->demand) dem_dev = sc.out_dev ? out->demand : c->dem_tmp.get<int32_t>(n_onodes);
+    // the count stays on the device; on the host SegPlan::comp_estimate picks the K3 kernel and the
+    // grid, and the arrays are sized by the bound (a component has >= 2 nodes)
+    sc.n_comp_cap = n_nodes / 2 + 1;
+    sc.comp_lo = c->comp_lo.get<uint32_t>(sc.n_comp_cap + 1);
+    sc.comp_hi = c->comp_hi.get<uint32_t>(sc.n_comp_cap + 1);
+    sc.in_bid = sc.direct.in_bid;  // single read length: bundle order is end order too
+    if (sc.direct_graph) {
+        // one pass writes what the scans, node_finalize, comp_write and in_src write below
+        // (no split, no forced cuts: virtual == original nodes, cut_at = 0, no adjustment)
+        const uint32_t n_tiles = (uint32_t)div_up((long long)n_nodes + 1, kDgTile);
+        const LookbackWords lw = lookback_words(c->scan, 4ull * n_tiles, st);
+        const DirectGraphOut o{c->bund.as<BundleRec>(), c->b_t.as<uint32_t>(), c->b_slot.as<uint32_t>(),
+                               sc.in_bid, c->in_src.get<uint32_t>((size_t)B + 1), d.diff, excl, d.outdeg,
+                               d.indeg, sc.node, sc.d_snap, sc.dem_v,
+                               c->in1.get<uint32_t>((size_t)n_nodes + 1), sc.comp_lo, sc.comp_hi, cov_dev,
+                               dem_dev, &sc.ds->n_bundles, &sc.ds->n_comp, totals, &sc.ds->res_supply};
+        // (B is the bound)
+        launch("direct_graph", 4ull * sc.direct.ktot + 60ull * n_nodes + 32ull * B, k_direct_graph,
+               n_tiles, kDgThreads, 0, st, sc.direct.ghist, sc.direct.dl, n_nodes, M,
+               sc.mf2.on ? 1u : 0u, o, lw.status, lw.ticket, lw.epoch, n_tiles);
+    } else {
+        build_nodes_chain(c, sc, cov_dev, dem_dev);
     }
     if (!sc.out_dev) {
         deliver(c, out->cov_capped, cov_dev, n_onodes, false);
@@ -1379,19 +1443,16 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
     const Degrees& d = sc.deg;
     if (sc.do_solve && sc.algorithm == 1 && sc.maxlen >= 4096)
         throw CallFail{GDS_ERR_ARG, "algorithm 1 (minimum cardinality) takes reads of up to 4095 positions"};
-    // the express schedule (maxflow_sm.cuh): components with a supply of kExpressMinSupply or
-    // more — none when M is below that, and then nothing about the launch changes
-    uint32_t express_on = sc.schedule == 1 ? 0u : sc.schedule == 2 ? 2u : 1u;  // (3: the usual supply rule)
-    if (!sc.forced_cuts || (express_on == 1 && sc.M < kExpressMinSupply)) express_on = 0;
-    const Mf2Plan mf2 = sc.do_solve && sc.algorithm == 0
-                            ? plan_maxflow_sm(n_comp, max_comp_nodes, express_on != 0, sc.knobs)
-                            : Mf2Plan{};
+    const uint32_t express_on = sc.express_on;
+    const Mf2Plan& mf2 = sc.mf2;
     uint32_t* in_src = c->in_src.get<uint32_t>((size_t)B + 1);
     uint32_t* in1 = c->in1.get<uint32_t>((size_t)n_nodes + 1);
-    GDS_CUDA(cudaMemsetAsync(in1, 0xff, ((size_t)n_nodes + 1) * 4, st));
-    if (B)
-        launch("in_src", 24ull * B, k_in_src, div_up(B, 256), 256, 0, st, bund, sc.in_bid, d.indeg,
-               &sc.ds->n_bundles, in_src, mf2.on ? sc.node : nullptr, in1);
+    if (!sc.direct_graph) {  // (k_direct_graph wrote both)
+        GDS_CUDA(cudaMemsetAsync(in1, 0xff, ((size_t)n_nodes + 1) * 4, st));
+        if (B)
+            launch("in_src", 24ull * B, k_in_src, div_up(B, 256), 256, 0, st, bund, sc.in_bid, d.indeg,
+                   &sc.ds->n_bundles, in_src, mf2.on ? sc.node : nullptr, in1);
+    }
     // per-component records only for the diagnostics dump; gds_result's counters are summed on
     // the device (MfTotals)
     sc.cstats = sc.knobs.dump_comp ? c->comp_stats.get<CompStats>(sc.n_comp_cap + 1) : nullptr;
@@ -1605,6 +1666,7 @@ extern "C" int gds_solve(gds_ctx* c, const gds_reads* rd, const gds_filter* flt,
         read_length_bounds(c, sc);
         sc.plan = plan_segments(rd, prm, sc.base, sc.minlen, sc.maxlen);
         out->seg_len = sc.plan.seg_len;
+        plan_solve(sc);
         find_bundles(c, sc);
         build_nodes(c, sc);
         solve_flow(c, sc);

@@ -74,6 +74,43 @@ __device__ __forceinline__ unsigned long long scan_status(uint32_t epoch, uint32
     return ((unsigned long long)epoch << 34) | ((unsigned long long)flag << 32) | v;
 }
 
+// Decoupled look-back of one value, run by one whole warp of the tile holding ticket tk; the tile
+// before it in the same sequence holds tk - stride.  Publishes the tile's aggregate, adds up the
+// predecessors' words back to the nearest inclusive prefix, publishes the tile's inclusive prefix
+// and returns its exclusive prefix (on every lane).
+__device__ __forceinline__ uint32_t lookback_prefix(unsigned long long* status, uint32_t tk,
+                                                    uint32_t stride, bool first_tile, uint32_t total,
+                                                    uint32_t epoch) {
+    const uint32_t lane = lane_id();
+    volatile unsigned long long* st = status;
+    if (first_tile) {
+        if (lane == 0) st[tk] = scan_status(epoch, 2, total);
+        return 0;
+    }
+    if (lane == 0) st[tk] = scan_status(epoch, 1, total);
+    uint32_t prefix = 0;
+    long long idx = (long long)tk - stride;
+    for (;;) {
+        const long long my = idx - (long long)lane * stride;
+        uint32_t flag = 2, val = 0;  // before the first tile: an inclusive prefix of zero
+        if (my >= 0) {
+            unsigned long long w;
+            do {
+                w = st[my];
+            } while ((uint32_t)(w >> 34) != epoch || ((w >> 32) & 3) == 0);
+            flag = (uint32_t)(w >> 32) & 3;
+            val = (uint32_t)w;
+        }
+        const uint32_t incl = __ballot_sync(0xffffffffu, flag == 2);
+        const int first = __ffs(incl) - 1;  // nearest predecessor that knows its prefix
+        prefix += __reduce_add_sync(0xffffffffu, (first < 0 || (int)lane <= first) ? val : 0u);
+        if (first >= 0) break;
+        idx -= 32ll * stride;
+    }
+    if (lane == 0) st[tk] = scan_status(epoch, 2, prefix + total);
+    return prefix;
+}
+
 // 256 threads x 16 elements per step, kLbSub steps per tile: a tile is 64 KB, read twice (the
 // second time from L2): once to publish its aggregate, once to scan and write.  Six or more tiles
 // per SM are resident, so the wait of one tile for its predecessors is covered by the loads of the
@@ -141,32 +178,8 @@ k_scan_lookback(ScanArrays a, uint32_t n_arr, size_t n, uint32_t n_tiles,
         uint32_t total = 0;
 #pragma unroll
         for (int w = 0; w < kLbThreads / 32; ++w) total += warp_tot[w];
-        uint32_t prefix = 0;
-        volatile unsigned long long* st = status;
-        if (tile == 0) {
-            if (lane == 0) st[tk] = scan_status(epoch, 2, total);
-        } else {
-            if (lane == 0) st[tk] = scan_status(epoch, 1, total);
-            long long idx = (long long)tk - n_arr;  // the tile before this one in the same array
-            for (;;) {
-                const long long my = idx - (long long)lane * n_arr;
-                uint32_t flag = 2, val = 0;  // before the first tile: an inclusive prefix of zero
-                if (my >= 0) {
-                    unsigned long long w;
-                    do {
-                        w = st[my];
-                    } while ((uint32_t)(w >> 34) != epoch || ((w >> 32) & 3) == 0);
-                    flag = (uint32_t)(w >> 32) & 3;
-                    val = (uint32_t)w;
-                }
-                const uint32_t incl = __ballot_sync(0xffffffffu, flag == 2);
-                const int first = __ffs(incl) - 1;  // nearest predecessor that knows its prefix
-                prefix += __reduce_add_sync(0xffffffffu, (first < 0 || (int)lane <= first) ? val : 0u);
-                if (first >= 0) break;
-                idx -= 32ll * n_arr;
-            }
-            if (lane == 0) st[tk] = scan_status(epoch, 2, prefix + total);
-        }
+        // the tile before this one in the same array holds ticket tk - n_arr
+        const uint32_t prefix = lookback_prefix(status, tk, n_arr, tile == 0, total, epoch);
         if (lane == 0) s_prefix = prefix;
     }
     __syncthreads();
@@ -235,6 +248,26 @@ inline void scan_one_tile(const uint32_t* in, uint32_t* out, size_t n, cudaStrea
     launch("scan_u32", 8ull * n, k_scan_tiles, 1, kScanThreads, 0, st, in, out, n);
 }
 
+// The status words and the ticket of one look-back launch, and its epoch.  The ticket is zero
+// between launches (the last tile of a launch resets it).
+struct LookbackWords {
+    unsigned long long* status;
+    uint32_t* ticket;
+    uint32_t epoch;
+};
+
+inline LookbackWords lookback_words(ScanTemp& tmp, size_t n_words, cudaStream_t st) {
+    unsigned long long* status = tmp.status.get<unsigned long long>(n_words);
+    uint32_t* ticket = tmp.ticket.get<uint32_t>(1);
+    if (tmp.status_cap != tmp.status.cap || tmp.epoch >= (1u << 30) - 1) {  // new buffer or epoch wrap
+        GDS_CUDA(cudaMemsetAsync(tmp.status.p, 0, tmp.status.cap, st));
+        GDS_CUDA(cudaMemsetAsync(ticket, 0, 4, st));
+        tmp.status_cap = tmp.status.cap;
+        tmp.epoch = 0;
+    }
+    return LookbackWords{status, ticket, ++tmp.epoch};
+}
+
 // k equally long arrays in one launch; arrays of one tile are scanned one by one
 inline void exclusive_scan_u32_multi(const ScanArrays& a, int n_arr, size_t n, ScanTemp& tmp,
                                      cudaStream_t st) {
@@ -244,17 +277,9 @@ inline void exclusive_scan_u32_multi(const ScanArrays& a, int n_arr, size_t n, S
         return;
     }
     const size_t tl = (n + kLbTile - 1) / kLbTile;
-    unsigned long long* status = tmp.status.get<unsigned long long>(tl * n_arr);
-    uint32_t* ticket = tmp.ticket.get<uint32_t>(1);
-    if (tmp.status_cap != tmp.status.cap || tmp.epoch >= (1u << 30) - 1) {  // new buffer or epoch wrap
-        GDS_CUDA(cudaMemsetAsync(tmp.status.p, 0, tmp.status.cap, st));
-        GDS_CUDA(cudaMemsetAsync(ticket, 0, 4, st));
-        tmp.status_cap = tmp.status.cap;
-        tmp.epoch = 0;
-    }
-    ++tmp.epoch;
+    const LookbackWords lw = lookback_words(tmp, tl * n_arr, st);
     launch("scan_u32", 8ull * n * n_arr, k_scan_lookback, (unsigned)(tl * n_arr), kLbThreads, 0, st, a,
-           (uint32_t)n_arr, n, (uint32_t)tl, status, ticket, tmp.epoch);
+           (uint32_t)n_arr, n, (uint32_t)tl, lw.status, lw.ticket, lw.epoch);
 }
 
 // out may alias in.  Callers that need the grand total read out[n-1] + in[n-1] themselves or scan
