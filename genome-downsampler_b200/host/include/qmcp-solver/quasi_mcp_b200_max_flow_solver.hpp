@@ -21,8 +21,8 @@ class QuasiMcpB200MaxFlowSolver : public Solver {
     std::unique_ptr<Solution> solve(uint32_t max_coverage, bam_api::BamApi& bam_api) override;
     bool uses_quality_of_reads() override { return false; }
 
-    // A batch of independent samples (contigs, runs) in ONE device call: the narrowing loops of all
-    // samples fill one pinned staging area on the host threads, gds_solve gets n_samples = size of
+    // A batch of independent samples (contigs, runs) in ONE device call: one narrowing loop over all
+    // samples fills one pinned staging area on the host threads, gds_solve gets n_samples = size of
     // the batch, and every sample's ascending kept indices come back as its own Solution — what
     // calling solve() on each BamApi in turn returns, minus a device round trip per sample.
     // BamApis with a pending pair filter are solved one by one through solve().
@@ -40,6 +40,15 @@ class QuasiMcpB200MaxFlowSolver : public Solver {
     void set_segment_length(uint32_t positions) { seg_len_ = positions; }
 
    private:
+    // The device call of solve() and solve_batch(): the samples' size_t columns, laid end to end,
+    // are narrowed into the staging buffers and solved in one gds_solve; any failure logs and
+    // exits.  `filter` = the BamApi whose pending filter the device applies (one sample only).
+    // Leaves the report in last_, the kept bitmap in bitmap_ and, filtered, the pair verdicts in
+    // pair_pass_.  Returns the samples' read offsets (n_samples + 1 entries).
+    std::vector<uint64_t> solve_on_device(uint32_t max_coverage,
+                                          const std::vector<const bam_api::SOAPairedReads*>& samples,
+                                          const bam_api::BamApi* filter);
+
     // grow-only page-locked staging buffer (gds_host_alloc): the narrowing loop writes straight
     // into it and the library copies from it at full PCIe speed
     struct Pinned {

@@ -80,22 +80,24 @@ def test_mcp_b200_plugin_returns_the_minimum_cover(hostlib, O):
 def test_plugin_solve_batch_equals_one_by_one(hostlib, O):
     # QuasiMcpB200MaxFlowSolver::solve_batch: ragged samples (different sizes, shapes and read
     # lengths, so the batch travels as 32-bit columns) and a fixed-length batch (compact transport);
-    # every sample's index list equals solve() on that sample alone and the oracle's bitmap
-    parts = [O.gen_reads(300 + k, 20_000 + 37 * k, 30_000, 150, sh)
-             for k, sh in enumerate(["uniform", "hole", "uniform", "low_sides", "uniform"])]
+    # every sample's index list equals solve() on that sample alone and the oracle's bitmap.
+    # The 70 kb batch has no 16-bit starts and is cut into segments; it stays fixed-length, because
+    # the default segment length is rounded to whole reads only when the batch has one read length.
+    def fixed(L):
+        return [O.gen_reads(300 + k, 20_000 + 37 * k, L, 150, sh)[:2]
+                for k, sh in enumerate(["uniform", "hole", "uniform", "low_sides", "uniform"])]
     rng = np.random.default_rng(4)
     s5 = rng.integers(0, 29_000, size=30_001).astype(np.uint32)   # odd count, variable lengths
     e5 = (s5 + rng.integers(80, 200, size=30_001)).astype(np.uint32)
-    for extra in ([], [(s5, e5)]):
-        ps = [(p[0], p[1]) for p in parts] + extra
+    for L, ps in ((30_000, fixed(30_000)), (30_000, fixed(30_000) + [(s5, e5)]), (70_000, fixed(70_000))):
         s = np.concatenate([p[0] for p in ps]); e = np.concatenate([p[1] for p in ps])
         off = np.cumsum([0] + [len(p[0]) for p in ps]).astype(np.uint64)
-        per, counts, secs = hostlib.plugin_solve_batch(s, e, off, 30_000, 60, repeats=2)
+        per, counts, secs = hostlib.plugin_solve_batch(s, e, off, L, 60, repeats=2)
         assert secs > 0 and len(per) == len(ps)
-        bm, st = O.sync_solve(s, e, [30_000] * len(ps), off, 60, params=(64, 150, 1, 0))
+        bm, st = O.sync_solve(s, e, [L] * len(ps), off, 60, params=(64, 150, 1, 0))
         mask = O.bitmap_to_mask(bm, len(s))
         for k, (sk, ek) in enumerate(ps):
-            one = hostlib.plugin_solve("quasi-mcp-b200", sk, ek, 30_000, 60)
+            one = hostlib.plugin_solve("quasi-mcp-b200", sk, ek, L, 60)
             assert np.array_equal(per[k], one) and counts[k] == len(one)
             assert np.array_equal(np.flatnonzero(mask[int(off[k]):int(off[k + 1])]), per[k].astype(np.int64))
 
