@@ -1,14 +1,17 @@
 // direct.cuh — sort-free K2 (bundles) and K5 (selection) for samples whose key space fits in the
 // shared memory of one SM.
 //
-// A bundle is the set of reads with one (start node, length) key (graph.cuh).  When a sample has
-// at most kDirectMaxKeys possible keys (ref_len x #lengths: 30 000 for a 30 kb reference with
-// fixed-length reads: configs 1, 3, 5 of SURVEY §8), its bundle multiplicities are a HISTOGRAM of the
-// reads: one shared-memory atomic per read, every input byte read exactly once at HBM speed
-// (tools/hist_probe.cu: 7.0 TB/s on B200 — the atomic unit keeps up with the loads), instead of
-// the two-pass radix sort's 48 bytes per read.  Restates the same network as the sort path
+// A bundle is the set of reads with one (start node, length) key (graph.cuh).  When all reads of
+// the call have one length, the key is the start node, and when a sample has at most kDirectMaxKeys
+// nodes (30 001 for a 30 kb reference: configs 1, 3, 5 of SURVEY §8) its bundle multiplicities are
+// a HISTOGRAM of the reads: one shared-memory atomic per read, every input byte read exactly once
+// at HBM speed (tools/hist_probe.cu: 7.0 TB/s on B200 — the atomic unit keeps up with the loads),
+// instead of the two-pass radix sort's 48 bytes per read.  Restates the same network as the sort path
 // (quasi_mcp_cpu_max_flow_solver.cpp:30-87 on bundles) — bundle order, node ids, difference array
 // and CSR are identical, so K3 and every parity test see the same graph.
+// Several read lengths take the global-memory histogram at the end of this file: (ref_len + 1) x
+// #lengths counters fit one SM only for short references (a 30 kb sample with two lengths already
+// has 60 002), so no realistic input with several lengths ever fitted here.
 //
 // K5 without a sorted read order: see the K5 section below.
 #pragma once
@@ -34,7 +37,7 @@ struct DirectLayout {
     const uint32_t* node_base; // [ns+1] first node id of sample k
     const uint32_t* kbase;     // [ns+1] first histogram slot of sample k (regions padded to 32)
     const uint32_t* item_off;  // [ns+1] first work item (sample part) of sample k
-    uint32_t ns, nlen, minlen, maxlen;
+    uint32_t ns, minlen;       // minlen: the one read length R
 };
 
 __device__ __forceinline__ uint32_t find_u32(const uint32_t* __restrict__ off, uint32_t n,
@@ -62,7 +65,7 @@ k_direct_hist(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
     const uint32_t tid = threadIdx.x;
     for (uint32_t i = tid; i < kmax; i += kDhThreads) h[i] = 0;
     uint32_t bad_range = 0, bad_hint = 0;
-    const uint32_t nlen = dl.nlen, minlen = dl.minlen, maxlen = dl.maxlen;
+    const uint32_t R = dl.minlen;
     for (;;) {
         if (tid == 0) s_item = atomicAdd(work_counter, 1u);
         __syncthreads();
@@ -81,12 +84,11 @@ k_direct_hist(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
                 ++bad_range;
                 return;
             }
-            const uint32_t len = e - s + 1;
-            if (len < minlen || len > maxlen) {
+            if (e - s + 1 != R) {
                 ++bad_hint;
                 return;
             }
-            atomicAdd(&h[s * nlen + (len - minlen)], 1u);
+            atomicAdd(&h[s], 1u);
         };
         if (a < b) {
             // unaligned head and tail by single loads, the body by 16-byte loads
@@ -161,17 +163,16 @@ k_direct_count(const uint32_t* __restrict__ ghist, uint32_t ktot, uint32_t* __re
 }
 
 // Writes what k_bundle_fill writes on the sort path (bundle record, in-CSR key, difference array,
-// CSR degrees) plus the bundle's histogram slot (K5 puts the bundle's flow there).
-// One read length takes k_direct_graph below, except with forced cuts: the forced-bundle test
-// compares the uncapped-position count at a bundle's end, R nodes to the right of a node, which a
-// left-to-right pass does not have yet.  The one_len branch here serves that case.
+// CSR degrees) plus the bundle's histogram slot (K5 puts the bundle's flow there) and the identity
+// in-CSR.  k_direct_graph below does all of it in one pass, except with forced cuts: the
+// forced-bundle test compares the uncapped-position count at a bundle's end, R nodes to the right of
+// a node, which a left-to-right pass does not have yet.  This kernel serves that case.
 __global__ void __launch_bounds__(kDkThreads)
 k_direct_bundles(const uint32_t* __restrict__ ghist, uint32_t ktot, DirectLayout dl,
                  const uint32_t* __restrict__ tile_offs, BundleRec* __restrict__ bund,
                  uint32_t* __restrict__ b_t, uint32_t* __restrict__ b_slot,
-                 uint32_t* __restrict__ in_bid /* identity when nlen == 1, else null */,
-                 int32_t* __restrict__ diff, uint32_t* __restrict__ outdeg,
-                 uint32_t* __restrict__ indeg) {
+                 uint32_t* __restrict__ in_bid, int32_t* __restrict__ diff,
+                 uint32_t* __restrict__ outdeg, uint32_t* __restrict__ indeg) {
     __shared__ uint32_t total;
     const uint32_t i = (blockIdx.x * kDkThreads + threadIdx.x) * 4;
     uint32_t v[4] = {0, 0, 0, 0};
@@ -184,45 +185,32 @@ k_direct_bundles(const uint32_t* __restrict__ ghist, uint32_t ktot, DirectLayout
     }
     const uint32_t c = (v[0] != 0) + (v[1] != 0) + (v[2] != 0) + (v[3] != 0);
     uint32_t b = block_excl_scan(c, &total) + tile_offs[blockIdx.x];
-    const bool one_len = in_bid != nullptr;
-    if (i >= ktot || (c == 0 && !one_len)) return;
+    if (i >= ktot) return;
     const uint32_t k = find_u32(dl.kbase, dl.ns, i);  // regions are 32-aligned: same k for all 4
     const uint32_t local = i - dl.kbase[k];
     const uint32_t nb = dl.node_base[k];
-    if (one_len) {
-        // one read length: key == start node, so the difference array needs no atomics —
-        // diff[v] = (reads starting at v) - (reads ending before v) = hist[v] - hist[v - len];
-        // every node of the sample is written (the region covers ref_len + 1 slots)
-        const uint32_t L = dl.ref_len[k], len = dl.minlen;
+    // key == start node, so the difference array needs no atomics —
+    // diff[v] = (reads starting at v) - (reads ending before v) = hist[v] - hist[v - len];
+    // every node of the sample is written (the region covers ref_len + 1 slots)
+    const uint32_t L = dl.ref_len[k], len = dl.minlen;
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const uint32_t j = local + q;
-            if (j > L) continue;
-            const uint32_t ends = j >= len ? ghist[i + q - len] : 0u;
-            diff[nb + j] = (int32_t)v[q] - (int32_t)ends;
-        }
-        if (c == 0) return;
+    for (int q = 0; q < 4; ++q) {
+        const uint32_t j = local + q;
+        if (j > L) continue;
+        const uint32_t ends = j >= len ? ghist[i + q - len] : 0u;
+        diff[nb + j] = (int32_t)v[q] - (int32_t)ends;
     }
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
         if (!v[q]) continue;
-        const uint32_t key = local + q;
-        const uint32_t s = nb + key / dl.nlen;
-        const uint32_t t = s + dl.minlen + key % dl.nlen;
-        const uint32_t mult = v[q];
-        reinterpret_cast<uint4*>(bund)[b] = make_uint4(t, mult, 0u, s);
+        const uint32_t s = nb + local + q;
+        const uint32_t t = s + len;
+        reinterpret_cast<uint4*>(bund)[b] = make_uint4(t, v[q], 0u, s);
         b_t[b] = t;
         b_slot[b] = i + q;
-        if (one_len) {  // at most one bundle starts / ends at a node
-            in_bid[b] = b;
-            outdeg[s] = 1u;
-            indeg[t] = 1u;
-        } else {
-            atomicAdd(&diff[s], (int32_t)mult);
-            atomicAdd(&diff[t], -(int32_t)mult);
-            atomicAdd(&outdeg[s], 1u);
-            atomicAdd(&indeg[t], 1u);
-        }
+        in_bid[b] = b;
+        outdeg[s] = 1u;  // at most one bundle starts / ends at a node
+        indeg[t] = 1u;
         ++b;
     }
 }
@@ -547,18 +535,17 @@ k_direct_graph(const uint32_t* __restrict__ ghist, DirectLayout dl, uint32_t n_n
 //   0 < f < mult  "partial": the f lowest of its mult read indices are kept       (code 2)
 // k_direct_classify writes the 2-bit code of every key (16 per word; a 30 kb sample's table is
 // 7.5 KB) and gives every partial bundle a segment of mult slots in a candidate buffer.
-// k_direct_mark streams the reads once more (start only when there is one read length), in
-// parallel parts like the histogram: code 1 sets the kept bit, code 2 appends the read index to
-// the bundle's segment.  k_direct_partial then ranks each partial bundle's candidates (one warp per
+// k_direct_mark streams the reads' starts once more, in parallel parts like the histogram: code 1
+// sets the kept bit, code 2 appends the read index to the bundle's segment.  k_direct_partial then ranks each partial bundle's candidates (one warp per
 // bundle).  If the candidates do not fit their buffer, ctl[2] is raised and the host repeats the
 // selection with the buffer grown to ctl[1].  If a partial bundle is huge (adversarial input:
 // millions of identical reads), ctl[2] is raised and the host repeats the selection with the
 // ordered walk below instead — same kept set, one CTA per sample.
 constexpr uint32_t kSatCode = 1, kPartCode = 2;
 constexpr uint32_t kMaxPartialMult = 2048;  // candidates of one bundle ranked by one warp
-// 512 threads x 3 CTAs per SM at 40 registers (one read length): the kernel is bound by neither
-// issue slots nor HBM but by its stalls per instruction, so more resident warps pay — 1.27 ms with
-// one CTA of 1024 threads (48 registers, half occupancy), 1.14 ms this way (config 5)
+// 512 threads x 3 CTAs per SM at 40 registers: the kernel is bound by neither issue slots nor HBM
+// but by its stalls per instruction, so more resident warps pay — 1.27 ms with one CTA of 1024
+// threads (48 registers, half occupancy), 1.14 ms this way (config 5)
 constexpr int kDmThreads = 512;
 constexpr int kDmCtasPerSm = 3;
 constexpr uint32_t kDmSplit = 3;
@@ -634,10 +621,9 @@ constexpr int kDmUnroll = 4;                                    // 512 reads per
 constexpr uint32_t kDmQueue = 256;                              // entries per warp
 constexpr uint32_t kDmQueueBytes = (kDmThreads / 32) * kDmQueue * 8;
 
-template <bool ONE_LEN>
-__global__ void __launch_bounds__(kDmThreads, ONE_LEN ? kDmCtasPerSm : 2)
-k_direct_mark(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, DirectLayout dl,
-              uint32_t n_items, uint32_t* __restrict__ work_counter,
+__global__ void __launch_bounds__(kDmThreads, kDmCtasPerSm)
+k_direct_mark(const uint32_t* __restrict__ S, DirectLayout dl, uint32_t n_items,
+              uint32_t* __restrict__ work_counter,
               const uint32_t* __restrict__ ghist, const uint32_t* __restrict__ kstat,
               const uint32_t* __restrict__ pb_off, uint32_t* __restrict__ pb_fill,
               uint32_t* __restrict__ cand, const uint32_t* __restrict__ ctl,
@@ -650,7 +636,6 @@ k_direct_mark(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
     __shared__ uint32_t wcnt[kDmThreads / 32];
     if (ctl[2]) return;
     const uint32_t tid = threadIdx.x, lane = lane_id(), warp = threadIdx.x >> 5;
-    const uint32_t nlen = dl.nlen, minlen = dl.minlen;
     constexpr int kU = kDmUnroll;
     uint32_t kept = 0;
     if (lane == 0) wcnt[warp] = 0;
@@ -684,10 +669,8 @@ k_direct_mark(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
             reinterpret_cast<uint4*>(st32)[i] = make_uint4(o[0], o[1], o[2], o[3]);
         }
         __syncthreads();
-        auto key_of = [&](uint32_t s, uint32_t e) {
-            const uint32_t key = ONE_LEN ? s : s * nlen + (e - s + 1 - minlen);
-            return min(key, kk - 1);  // in range on validated input; never read past the table
-        };
+        // the key is the start: in range on validated input; never read past the table
+        auto key_of = [&](uint32_t s) { return min(s, kk - 1); };
         // converged warp: hand the parked reads to their bundles' candidate segments
         auto park = [&](uint32_t key, uint32_t g) {
             const uint32_t pid = ghist[kb + key];
@@ -721,8 +704,7 @@ k_direct_mark(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
                 const uint64_t lo = side ? b4 : a, hi = side ? b : a4;
                 if (tid < hi - lo) {
                     const uint64_t g = lo + tid;
-                    const uint32_t s = S[g];
-                    const uint32_t key = key_of(s, ONE_LEN ? 0u : E[g]);
+                    const uint32_t key = key_of(S[g]);
                     if (hit(g, key, st[key])) {
                         atomicOr(&bitmap[g >> 5], 1u << (g & 31));
                         ++kept;
@@ -730,10 +712,8 @@ k_direct_mark(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
                 }
             }
             const uint4* S4 = reinterpret_cast<const uint4*>(S) + a4 / 4;
-            const uint4* E4 = reinterpret_cast<const uint4*>(E) + a4 / 4;
-            auto mark4 = [&](uint32_t j, const uint4& s, const uint4& e) {
-                const uint32_t k0 = key_of(s.x, e.x), k1 = key_of(s.y, e.y), k2 = key_of(s.z, e.z),
-                               k3 = key_of(s.w, e.w);
+            auto mark4 = [&](uint32_t j, const uint4& s) {
+                const uint32_t k0 = key_of(s.x), k1 = key_of(s.y), k2 = key_of(s.z), k3 = key_of(s.w);
                 const uint32_t c0 = st[k0], c1 = st[k1], c2 = st[k2], c3 = st[k3];
                 if ((c0 | c1 | c2 | c3) == 0) return;  // 94 % of the groups
                 const uint64_t g = a4 + 4ull * j;
@@ -748,19 +728,16 @@ k_direct_mark(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, Di
             // converged): lanes past the end process nothing
             const uint32_t jend = (uint32_t)((b4 - a4) / 4);
             for (uint32_t jw = warp * 32; jw < jend; jw += kU * kDmThreads) {
-                uint4 s[kU], e[kU];
+                uint4 s[kU];
 #pragma unroll
                 for (int u = 0; u < kU; ++u) {
                     const uint32_t j = jw + lane + u * kDmThreads;
-                    if (j < jend) {
-                        s[u] = ld_stream4(S4 + j);
-                        if (!ONE_LEN) e[u] = ld_stream4(E4 + j);
-                    }
+                    if (j < jend) s[u] = ld_stream4(S4 + j);
                 }
 #pragma unroll
                 for (int u = 0; u < kU; ++u) {
                     const uint32_t j = jw + lane + u * kDmThreads;
-                    if (j < jend) mark4(j, s[u], e[u]);
+                    if (j < jend) mark4(j, s[u]);
                 }
                 drain(kDmQueue / 2);
             }
@@ -885,15 +862,14 @@ k_direct_quota(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ 
 }
 
 __global__ void __launch_bounds__(kDsThreads, 1)
-k_direct_select(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, DirectLayout dl,
-                uint32_t* __restrict__ work_counter, const uint32_t* __restrict__ ghist,
-                uint32_t* __restrict__ bitmap, unsigned long long* __restrict__ totals) {
-    extern __shared__ uint32_t quota[];  // per key: flow still to be handed out (as int32)
+k_direct_select(const uint32_t* __restrict__ S, DirectLayout dl, uint32_t* __restrict__ work_counter,
+                const uint32_t* __restrict__ ghist, uint32_t* __restrict__ bitmap,
+                unsigned long long* __restrict__ totals) {
+    extern __shared__ uint32_t quota[];  // per key (start node): flow still to be handed out (as int32)
     __shared__ uint32_t c_key[kDsTile];
     __shared__ uint16_t c_pos[kDsTile];
     __shared__ uint32_t s_k, s_nconf, s_remaining;
     const uint32_t tid = threadIdx.x;
-    const uint32_t nlen = dl.nlen, minlen = dl.minlen;
     constexpr uint32_t kNone = 0xffffffffu;
     for (;;) {
         if (tid == 0) {
@@ -919,14 +895,12 @@ k_direct_select(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, 
         const uint32_t total = s_remaining;
         if (total != 0) {
             const uint32_t n_tiles = (uint32_t)((n_k + kDsTile - 1) / kDsTile);
-            uint32_t ns_[kDsPer], ne_[kDsPer];
+            uint32_t ns_[kDsPer];
             auto fetch = [&](uint32_t t) {
 #pragma unroll
                 for (int q = 0; q < kDsPer; ++q) {
                     const uint64_t idx = (uint64_t)t * kDsTile + q * kDsThreads + tid;
-                    const bool in = idx < n_k;
-                    ns_[q] = in ? ld_stream(S + base + idx) : kNone;
-                    ne_[q] = (in && nlen > 1) ? ld_stream(E + base + idx) : 0u;
+                    ns_[q] = idx < n_k ? ld_stream(S + base + idx) : kNone;
                 }
             };
             fetch(0);
@@ -936,12 +910,7 @@ k_direct_select(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, 
                 bool any = false;
 #pragma unroll
                 for (int q = 0; q < kDsPer; ++q) {
-                    key[q] = kNone;
-                    if (ns_[q] != kNone) {
-                        const uint32_t kq = nlen > 1 ? ns_[q] * nlen + (ne_[q] - ns_[q] + 1 - minlen)
-                                                     : ns_[q];
-                        if (kq < kk) key[q] = kq;
-                    }
+                    key[q] = ns_[q] < kk ? ns_[q] : kNone;
                     cand[q] = key[q] != kNone && (int32_t)quota[key[q]] > 0;
                     any |= cand[q];
                 }
@@ -1005,12 +974,12 @@ k_direct_select(const uint32_t* __restrict__ S, const uint32_t* __restrict__ E, 
 
 
 // ---- the same idea with the histogram in global memory ------------------------------------------
-// When a sample's key space does not fit one SM (several read lengths: config 2) or the reference is
-// cut into segments (config 4), the counters live in global memory instead: up to kGDirectMaxKeys of
-// them (96 MB, resident in the 126 MB L2), one RED.ADD per read (tools/hist_probe.cu: 170 G keys/s)
-// and a second one for the right part of a read that crosses a segment cut.  Keys are the sort
-// path's keys, (virtual fake start id, length) — graph.cuh: ReadKeys / VLayout — so bundles come
-// out in the same order with the same clamping to the segment's node range.
+// When the reads have several lengths (config 2), a sample does not fit one SM, or the reference is
+// cut into segments (config 4), the counters live in global memory instead: up to kGDirectMaxKeys
+// of them (96 MB, resident in the 126 MB L2), one RED.ADD per read (tools/hist_probe.cu: 170 G
+// keys/s) and a second one for the right part of a read that crosses a segment cut.  Keys are the
+// sort path's keys, (virtual fake start id, length) — graph.cuh: ReadKeys / VLayout — so bundles
+// come out in the same order with the same clamping to the segment's node range.
 constexpr unsigned long long kGDirectMaxKeys = 24ull << 20;
 constexpr int kGdThreads = 256;
 constexpr int kGdItems = 8;

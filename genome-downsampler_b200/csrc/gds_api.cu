@@ -391,14 +391,14 @@ void launch_sweep(gds_ctx* c, const SweepArgs& a, uint32_t maxlen, bool one_len,
     kShapes[w * 2 + (one_len ? 0 : 1)](c, a, alg_bytes);
 }
 
-// Sort-free K2 (direct.cuh).  Eligible when no sample is segmented and every sample's key space
-// (ref_len x number of distinct read lengths) fits in one SM's shared memory.
+// Sort-free K2 (direct.cuh).  The shared-memory histogram is eligible when all reads have one
+// length, no sample is segmented and every sample's ref_len + 1 nodes fit in one SM's shared memory.
 struct DirectPlan {
     bool on = false;
     DirectLayout dl{};
     uint32_t* ghist = nullptr;
     uint32_t ktot = 0, kmax = 0, n_items = 0;
-    uint32_t* in_bid = nullptr;  // identity in-CSR (single read length), else null
+    uint32_t* in_bid = nullptr;  // identity in-CSR (one read length), else null
     bool global = false;         // counters in global memory (several lengths / segmented reference)
     GDirectLayout gl{};
 };
@@ -470,7 +470,7 @@ struct SolveCall {
     Mf2Plan mf2;
     // K2
     DirectPlan direct;
-    bool direct_graph;  // k_direct_graph builds the nodes, components and in-arcs (one read length)
+    bool direct_graph;  // k_direct_graph builds the nodes, components and in-arcs (no forced cuts)
     uint32_t B;  // exact when the host needs it (radix sorts over the bundles), else a bound
     uint32_t* sorted_idx;
     int sort_passes;
@@ -602,13 +602,11 @@ void sort_bundles(gds_ctx* c, SolveCall& sc, const uint32_t* cross_idx, size_t n
         build_bundles<unsigned long long>(c, sc, tm, cross_idx, local_keys, keybits, fused_ref);
 }
 
-bool direct_eligible(const gds_reads* rd, uint32_t ns, uint32_t minlen, uint32_t maxlen,
-                     const uint32_t* S, const uint32_t* E) {
+bool direct_eligible(const gds_reads* rd, uint32_t ns, const uint32_t* S, const uint32_t* E) {
     if (((uintptr_t)S | (uintptr_t)E) & 15) return false;  // 16-byte loads
-    const uint64_t nlen = (uint64_t)maxlen - minlen + 1;
     uint64_t tot = 0;
     for (uint32_t k = 0; k < ns; ++k) {
-        const uint64_t kk = ((uint64_t)rd->ref_len[k] + 1) * nlen;  // one slot row per node
+        const uint64_t kk = (uint64_t)rd->ref_len[k] + 1;  // one slot per node
         if (kk > kDirectMaxKeys) return false;
         tot += (kk + 31) & ~31ull;
     }
@@ -625,7 +623,7 @@ struct BundleOut {
 };
 
 // The bundle buffers of a histogram path, sized for B bundles; the identity in-CSR when there is
-// one read length
+// one read length (always on the shared-memory path)
 void bundle_buffers(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint32_t B, BundleOut& o) {
     sc.B = B;
     o.bund = c->bund.get<BundleRec>(B + 1);
@@ -638,9 +636,8 @@ void bundle_buffers(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint32_t B, Bun
 
 // What both histogram paths do once plan.ghist holds the counts: count the non-empty keys per
 // tile, scan, the bundle count (on the device; b_bound sizes the buffers), the bundle buffers and
-// the cleared degree arrays.  own_diff: the bundle kernel writes the whole difference array itself.
-BundleOut histogram_bundles(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint64_t b_bound,
-                            bool own_diff) {
+// the cleared degree arrays (k_direct_bundles writes the whole difference array itself).
+BundleOut histogram_bundles(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint64_t b_bound) {
     cudaStream_t st = sc.st;
     const uint32_t ktot = plan.ktot;
     const uint32_t n_tiles = (uint32_t)div_up(ktot, kDkTile);
@@ -651,23 +648,23 @@ BundleOut histogram_bundles(gds_ctx* c, SolveCall& sc, DirectPlan& plan, uint64_
     GDS_CUDA(cudaMemcpyAsync(&sc.ds->n_bundles, tc + n_tiles, 4, cudaMemcpyDeviceToDevice, st));
     uint32_t B = (uint32_t)std::min<uint64_t>(ktot, b_bound);
     if (sc.minlen != sc.maxlen) {
-        // several read lengths: the in-CSR order comes from a radix sort of the bundles (build_nodes),
-        // which needs their exact number; the input verdict comes with the same synchronisation
+        // several read lengths (global memory): the in-CSR order comes from a radix sort of the
+        // bundles (build_nodes), which needs their exact number; the input verdict comes with the
+        // same synchronisation
         d2h_sync(c, &B, tc + n_tiles, 1);
         read_input_verdict(c, sc.ds);
     }
     BundleOut o{n_tiles, tc};
     bundle_buffers(c, sc, plan, B, o);
-    o.d = alloc_degrees(c, st, sc.plan.n_nodes, !(own_diff && B));
+    o.d = alloc_degrees(c, st, sc.plan.n_nodes, plan.global || !B);
     return o;
 }
 
 void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
     cudaStream_t st = sc.st;
     DirectPlan& plan = sc.direct;
-    const uint32_t ns = sc.ns, minlen = sc.minlen, maxlen = sc.maxlen;
+    const uint32_t ns = sc.ns;
     const uint64_t N = sc.N;
-    const uint32_t nlen = maxlen - minlen + 1;
     // host-side layout: histogram regions and work items (sample parts)
     std::vector<uint32_t> lay(2 * (ns + 1), 0);
     uint32_t* kbase = lay.data();
@@ -675,7 +672,7 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
     const uint64_t part_len = std::max<uint64_t>(65536, (N + 8ull * kNumSMs - 1) / (8ull * kNumSMs));
     uint32_t kmax = 32;
     for (uint32_t k = 0; k < ns; ++k) {
-        const uint32_t kk = ((sc.rd->ref_len[k] + 1) * nlen + 31u) & ~31u;
+        const uint32_t kk = (sc.rd->ref_len[k] + 1 + 31u) & ~31u;
         kmax = std::max(kmax, kk);
         kbase[k + 1] = kbase[k] + kk;
         const uint64_t nk = sc.foff_host[k + 1] - sc.foff_host[k];
@@ -690,16 +687,14 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
     uint32_t* wc = c->dwork.get<uint32_t>(2);
     GDS_CUDA(cudaMemsetAsync(ghist, 0, (size_t)ktot * 4, st));
     GDS_CUDA(cudaMemsetAsync(wc, 0, 8, st));
-    const DirectLayout dl{sc.foff_dev, sc.reflen_d, sc.base_d, lay_d, lay_d + ns + 1, ns, nlen, minlen, maxlen};
+    const DirectLayout dl{sc.foff_dev, sc.reflen_d, sc.base_d, lay_d, lay_d + ns + 1, ns, sc.minlen};
     const unsigned smem = kmax * 4;
     if (smem > c->direct_attr) {
         GDS_CUDA(cudaFuncSetAttribute(k_direct_hist, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)(kDirectMaxKeys * 4)));
         GDS_CUDA(cudaFuncSetAttribute(k_direct_select, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)(kDirectMaxKeys * 4)));
-        GDS_CUDA(cudaFuncSetAttribute(k_direct_mark<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(kDmQueueBytes + kDirectMaxKeys)));
-        GDS_CUDA(cudaFuncSetAttribute(k_direct_mark<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        GDS_CUDA(cudaFuncSetAttribute(k_direct_mark, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)(kDmQueueBytes + kDirectMaxKeys)));
         c->direct_attr = kDirectMaxKeys * 4;
     }
@@ -717,8 +712,7 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
         degree_buffers(c, sc.plan.n_nodes);
         return;
     }
-    // one read length: k_direct_bundles writes the difference array of every node itself
-    const BundleOut o = histogram_bundles(c, sc, plan, N, nlen == 1);
+    const BundleOut o = histogram_bundles(c, sc, plan, N);
     if (sc.B)
         launch("direct_bundles", 4ull * ktot + 40ull * sc.B, k_direct_bundles, o.n_tiles, kDkThreads, 0,
                st, ghist, ktot, dl, o.tc, o.bund, o.b_t, o.b_slot, o.ident, o.d.diff, o.d.outdeg,
@@ -743,7 +737,7 @@ void build_bundles_gdirect(gds_ctx* c, SolveCall& sc) {
     plan.ghist = ghist;
     plan.ktot = ktot;
     // a read crossing a cut counts twice
-    const BundleOut o = histogram_bundles(c, sc, plan, 2 * N, false);
+    const BundleOut o = histogram_bundles(c, sc, plan, 2 * N);
     if (sc.B)
         launch("gdirect_bundles", 4ull * ktot + 40ull * sc.B, k_gdirect_bundles, o.n_tiles, kDkThreads,
                0, st, ghist, ktot, gl, o.tc, o.bund, o.b_t, o.b_slot, o.ident, o.d.diff, o.d.outdeg,
@@ -785,20 +779,17 @@ void direct_select(gds_ctx* c, SolveCall& sc, bool force_walk, size_t cand_need)
         launch("direct_classify", 20ull * B, k_direct_classify, div_up(B, 256), 256, 0, st, bund,
                b_slot, dp.ghist, kstat, pb, pb + B + 1, fill, ctl,
                dp.global ? 0xffffffffu : kMaxPartialMult, B_dev, (uint32_t)cand_cap, sc.stats());
-        const unsigned long long per_read = (dp.global || dp.dl.nlen > 1) ? 8 : 4;
         if (dp.global) {
-            launch("gdirect_mark", per_read * N + dp.ktot / 4 + 8ull * N / 32, k_gdirect_mark,
+            launch("gdirect_mark", 8ull * N + dp.ktot / 4 + 8ull * N / 32, k_gdirect_mark,
                    div_up((long long)N, kGdTile), kGdThreads, 0, st, sc.S, sc.E, N, dp.gl, dp.ghist,
                    kstat, pb, fill, cand, bm, totals, ctl);
         } else {
             uint32_t* wc = c->dwork.as<uint32_t>() + 1;
             GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
-            const int grid = (int)std::min<uint32_t>(
-                dp.n_items * kDmSplit, (uint32_t)kNumSMs * (dp.dl.nlen == 1 ? kDmCtasPerSm : 2));
-            launch("direct_mark", per_read * N + dp.ktot / 4 + 8ull * N / 32,
-                   dp.dl.nlen == 1 ? k_direct_mark<true> : k_direct_mark<false>, grid, kDmThreads,
-                   kDmQueueBytes + dp.kmax, st, sc.S, sc.E, dp.dl, dp.n_items, wc, dp.ghist, kstat, pb,
-                   fill, cand, ctl, bm, totals);
+            const int grid = (int)std::min<uint32_t>(dp.n_items * kDmSplit, (uint32_t)kNumSMs * kDmCtasPerSm);
+            launch("direct_mark", 4ull * N + dp.ktot / 4 + 8ull * N / 32, k_direct_mark, grid, kDmThreads,
+                   kDmQueueBytes + dp.kmax, st, sc.S, dp.dl, dp.n_items, wc, dp.ghist, kstat, pb, fill,
+                   cand, ctl, bm, totals);
         }
         // segments of a long reference (global path): ~10 reads per bundle, half a warp each
         launch("direct_partial", 16ull * (N / 64),
@@ -812,7 +803,7 @@ void direct_select(gds_ctx* c, SolveCall& sc, bool force_walk, size_t cand_need)
         GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
         launch("direct_walk", 4ull * dp.ktot + 8ull * N / 32, k_direct_select,
                (int)std::min<uint32_t>(sc.ns, (uint32_t)kNumSMs), kDsThreads, dp.kmax * 4, st, sc.S,
-               sc.E, dp.dl, wc, dp.ghist, bm, totals);
+               dp.dl, wc, dp.ghist, bm, totals);
     }
     GDS_CUDA(cudaMemcpyAsync(sc.ds->ctl, ctl, 16, cudaMemcpyDeviceToDevice, st));
 }
@@ -1277,11 +1268,11 @@ void find_bundles(gds_ctx* c, SolveCall& sc) {
     }
     // 0 = choose, 1 = always the radix sort, 2 = the direct histogram whenever eligible
     const int bmode = sc.prm ? (int)sc.prm->bundle_mode : 0;
-    const bool use_direct = N > 0 && !pl.split && bmode != 1 &&
-                            direct_eligible(sc.rd, ns, sc.minlen, sc.maxlen, sc.S, sc.E);
+    const bool use_direct = N > 0 && !pl.split && bmode != 1 && sc.minlen == sc.maxlen &&
+                            direct_eligible(sc.rd, ns, sc.S, sc.E);
     const bool use_gdirect = N > 0 && !use_direct && bmode != 1 &&
                              (uint64_t)n_nodes * ((uint64_t)sc.maxlen - sc.minlen + 1) <= kGDirectMaxKeys;
-    sc.direct_graph = use_direct && sc.minlen == sc.maxlen && !sc.forced_cuts;
+    sc.direct_graph = use_direct && !sc.forced_cuts;
     size_t n_items = N;
     uint32_t* cross_idx = nullptr;
     if (pl.split && N > 0 && !use_gdirect) {  // right parts of the reads that cross a cut

@@ -115,9 +115,9 @@ typedef struct {
     uint32_t seg_len;
     /* how K2 finds the bundles (reads with one (start, length) key): 0 = choose, 1 = always the
      * segmented radix sort, 2 = a sort-free histogram whenever one is eligible: counters in shared
-     * memory (no sample segmented, ref_len x #read-lengths <= 49152 per sample, 16-byte aligned
-     * start/end) or else in global memory (virtual nodes x #read-lengths <= 24 Mi).  All three give
-     * the same graph and the same kept set; gds_result.bundle_path tells which one ran. */
+     * memory (one read length, no sample segmented, ref_len + 1 <= 49152 per sample, 16-byte
+     * aligned start/end) or else in global memory (virtual nodes x #read-lengths <= 24 Mi).  All
+     * three give the same graph and the same kept set; gds_result.bundle_path tells which one ran. */
     uint32_t bundle_mode;
     /* which solve runs on the graph:
      *   0  quasi-MCP — maximum flow by push-relabel (quasi_mcp_cpu_max_flow_solver.cpp:11-100);

@@ -351,7 +351,7 @@ def test_length_hints_fold_validation_into_the_sort(pkg, solver, O):
     assert solver.solve(s, e, [30_000] * 3, 30, read_off=off, params=PRM).n_kept == r0.n_kept
 
 
-def test_direct_histogram_path_equals_sort_path(solver, O):
+def test_histogram_paths_equal_sort_path(solver, O):
     # gds_params.bundle_mode: 30 kb samples with one read length take the sort-free histogram by
     # default (sort_passes == 0); forcing the radix sort must give the same graph and kept set
     parts = [O.gen_reads(4242 + k, 150_000 + 7 * k, 30_000, 150, sh)
@@ -381,7 +381,8 @@ def test_direct_histogram_path_equals_sort_path(solver, O):
         del os.environ["GDS_DIRECT_SELECT"]
     assert rw.sort_passes == 0 and rw.n_kept == res[1].n_kept and rw.verify_violations == 0
     assert np.array_equal(rw.kept_bitmap, res[1].kept_bitmap)
-    # a few read lengths (key = start x #lengths + length) still fit in shared memory
+    # several read lengths take the global histogram, even where (ref_len + 1) x #lengths would
+    # fit in shared memory
     rng = np.random.default_rng(11)
     s2 = rng.integers(0, 9_000, size=400_000).astype(np.uint32)
     e2 = (s2 + rng.integers(148, 152, size=400_000)).astype(np.uint32)
@@ -390,7 +391,20 @@ def test_direct_histogram_path_equals_sort_path(solver, O):
     assert ra.sort_passes == 0 and rb.sort_passes > 0
     assert np.array_equal(ra.kept_bitmap, rb.kept_bitmap) and ra.rounds_total == rb.rounds_total
     assert_parity(O, ra, s2, e2, [9_200], [0, len(s2)], 200)
-    assert ra.bundle_path == 1 and rb.bundle_path == 0
+    assert ra.bundle_path == 2 and rb.bundle_path == 0
+    # ... and so do lengths 150-152 on 15 kb given as hints: same graph and kept set as the sort
+    s6, e6, _, _ = O.gen_reads(640, 40_000, 15_000, 150)
+    e6 = np.where(e6 + 2 < 15_000, e6 + np.arange(len(e6)) % 3, e6).astype(np.uint32)
+    rg = solver.solve(s6, e6, 15_000, 60, params=PRM + (0, 2), verify=True, want_vectors=True,
+                      len_hint=(150, 152))
+    rh = solver.solve(s6, e6, 15_000, 60, params=PRM + (0, 1), verify=True, want_vectors=True,
+                      len_hint=(150, 152))
+    assert rg.bundle_path == 2 and rg.sort_passes == 0 and rh.bundle_path == 0
+    for key in ("fstar", "flow_value", "n_bundles", "n_components", "n_kept", "rounds_total",
+                "pushes", "relabels", "bfs_levels", "verify_violations"):
+        assert rg[key] == rh[key], key
+    assert np.array_equal(rg.kept_bitmap, rh.kept_bitmap)
+    assert np.array_equal(rg.demand, rh.demand) and np.array_equal(rg.cov_capped, rh.cov_capped)
     # a key space beyond shared memory keeps its counters in global memory (L2): same answer again
     e3 = (s2 + rng.integers(100, 300, size=400_000)).astype(np.uint32)
     rc = solver.solve(s2, e3, 9_400, 50, params=PRM + (0, 0), verify=True, want_vectors=True)
@@ -417,17 +431,25 @@ def test_direct_histogram_path_equals_sort_path(solver, O):
 def test_direct_selection_walk_many_tiles_and_duplicates(solver, O):
     # the ordered walk of K5 (direct path): tiny key spaces so that every 4096-read tile holds many
     # reads of one key, quotas that run out in the middle of a tile or span several tiles, ragged
-    # sample offsets (unaligned 16-byte loads at part boundaries)
+    # sample offsets (unaligned 16-byte loads at part boundaries).  Every fourth input has one read
+    # length R, which the shared-memory histogram and its walk need; the others draw lengths per
+    # sample and clip them at the reference's end, so most of them take the global histogram.
     rng = np.random.default_rng(23)
     for it in range(40):
+        walk = it % 4 == 0
         ns = int(rng.integers(1, 4))
         Ls = rng.integers(2, 60, size=ns).astype(np.uint32)
+        R = int(rng.integers(1, int(Ls.min()) + 1))
         ss, ee, off = [], [], [0]
         for L in Ls:
             n = int(rng.integers(0, 30_000))
-            nl = int(rng.integers(1, 4))
-            s = rng.integers(0, L, size=n)
-            e = np.minimum(s + rng.integers(1, 1 + nl, size=n) * int(rng.integers(1, 8)) - 1, L - 1)
+            if walk:
+                s = rng.integers(0, L - R + 1, size=n)
+                e = s + R - 1
+            else:
+                nl = int(rng.integers(1, 4))
+                s = rng.integers(0, L, size=n)
+                e = np.minimum(s + rng.integers(1, 1 + nl, size=n) * int(rng.integers(1, 8)) - 1, L - 1)
             ss.append(s); ee.append(e); off.append(off[-1] + n)
         s = np.concatenate(ss).astype(np.uint32); e = np.concatenate(ee).astype(np.uint32)
         M = int(rng.choice([1, 3, 50, 700, 5000, 20000]))
@@ -436,7 +458,8 @@ def test_direct_selection_walk_many_tiles_and_duplicates(solver, O):
                          want_vectors=True)
         assert r.sort_passes == 0 or len(s) == 0
         assert_parity(O, r, s, e, Ls, off, M)
-        if it % 4 == 0:  # and the ordered walk on the same input
+        if walk:  # and the ordered walk on the same input
+            assert r.bundle_path == 1
             import os
             os.environ["GDS_DIRECT_SELECT"] = "walk"
             try:
@@ -444,6 +467,7 @@ def test_direct_selection_walk_many_tiles_and_duplicates(solver, O):
             finally:
                 del os.environ["GDS_DIRECT_SELECT"]
             assert np.array_equal(rw.kept_bitmap, r.kept_bitmap) and rw.n_kept == r.n_kept
+            assert rw.bundle_path == 1
 
 
 def test_compact_transport_start16_and_implied_end(pkg, solver, O):
@@ -767,9 +791,9 @@ VERDICT_PATHS = {  # bundle path: (reference length, gds_params, length hints)
     "sort_hints": (30_000, PRM + (0, 1), (150, 150)),
     "sort_no_hints": (30_000, PRM + (0, 1), None),
     "segmented": (100_000, (64, 150, 1, 0, 8192, 1), (150, 150)),
-    # several read lengths: the bundle count is read back for the in-CSR sort, and the verdict with
-    # it (15 001 nodes x 3 lengths fit the shared-memory histogram)
-    "direct_several_lengths": (15_000, PRM + (0, 2), (150, 152)),
+    # several read lengths (global histogram): the bundle count is read back for the in-CSR sort,
+    # and the verdict with it
+    "global_several_lengths": (15_000, PRM + (0, 2), (150, 152)),
     "direct_one_length": (30_000, PRM + (0, 2), (150, 150)),
     "global_hist": (100_000, (64, 150, 1, 0, 8192, 0), (150, 150)),
 }
@@ -797,6 +821,6 @@ def test_input_verdicts_on_every_bundle_path(pkg, solver, O, path, kind):
     again = solver.solve(s, e, L, 40, params=prm, len_hint=lh)
     assert ei.value.code == code
     assert str(ei.value).endswith(": %d %s" % (count, what)), str(ei.value)
-    want_path = {"direct_several_lengths": 1, "direct_one_length": 1, "global_hist": 2}.get(path, 0)
+    want_path = {"global_several_lengths": 2, "direct_one_length": 1, "global_hist": 2}.get(path, 0)
     assert good.bundle_path == want_path and good.verify_violations == 0
     assert np.array_equal(again.kept_bitmap, good.kept_bitmap) and again.n_kept == good.n_kept

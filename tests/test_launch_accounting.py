@@ -18,7 +18,8 @@ def _cases(O):
     batch = dict(start=s, end=e, ref_len=[30_000] * 3, read_off=off)
     sl, el, _, _ = O.gen_reads(620, 120_000, 150_000, 150)
     seg = dict(start=sl, end=el, ref_len=150_000)
-    # reads of 150, 151 and 152 positions: 3 x 15 001 keys fit the shared-memory histogram
+    # reads of 150, 151 and 152 positions: several lengths take the global-memory histogram, which
+    # reads the bundle count and the input verdict back in the middle of the call
     sv, ev, _, _ = O.gen_reads(640, 40_000, 15_000, 150)
     ev = np.where(ev + 2 < 15_000, ev + np.arange(len(ev)) % 3, ev).astype(np.uint32)
     several = dict(start=sv, end=ev, ref_len=15_000)
@@ -31,7 +32,7 @@ def _cases(O):
     return {
         "radix_sort": (batch, 60, dict(params=PRM + (0, 1)), {}),
         "direct_one_length": (batch, 60, dict(params=PRM + (0, 2), len_hint=(150, 150)), {}),
-        "direct_several_lengths": (several, 60, dict(params=PRM + (0, 2), len_hint=(150, 152)), {}),
+        "global_several_lengths": (several, 60, dict(params=PRM + (0, 2), len_hint=(150, 152)), {}),
         "global_hist_segmented": (seg, 60, dict(params=(64, 150, 1, 0, 8192, 0)), {}),
         "pair_filter": (filt, 100, dict(params=PRM), {}),
         "direct_walk": (batch, 60, dict(params=PRM + (0, 2)), {"GDS_DIRECT_SELECT": "walk"}),
@@ -41,7 +42,7 @@ def _cases(O):
     }
 
 
-PATHS = ["radix_sort", "direct_one_length", "direct_several_lengths", "global_hist_segmented",
+PATHS = ["radix_sort", "direct_one_length", "global_several_lengths", "global_hist_segmented",
          "pair_filter", "direct_walk", "maxflow_global", "express", "min_cardinality"]
 
 
@@ -71,5 +72,7 @@ def test_profile_accounts_for_every_launch(solver, O, path):
     assert plain.verify_violations == 0
     if path.startswith("direct_"):
         assert plain.bundle_path == 1
+    if path.startswith("global_"):
+        assert plain.bundle_path == 2
     if path == "pair_filter":
         assert np.array_equal(prof.pair_pass, plain.pair_pass)
