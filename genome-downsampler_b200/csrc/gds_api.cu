@@ -118,18 +118,15 @@ void deliver(gds_ctx* c, T* dst, const T* dev_src, size_t n, bool dst_on_device)
 // Diagnostic knobs for tests and measurements.  Read once per call: tests change them between calls.
 struct Knobs {
     bool mf_global;         // GDS_MF=global: the round-1 kernel only
-    bool mf_sm;             // GDS_MF=sm: k_maxflow_sm whenever it fits
     bool mf_optr;           // GDS_MF_OPTR=0: k_maxflow_sm without the out-CSR cache
-    bool mf_warp;           // GDS_MF_WARP=1 (see launch_mf2_shape)
     bool walk;              // GDS_DIRECT_SELECT=walk: K5 of the histogram path takes the ordered walk
     const char* dump_comp;  // GDS_DUMP_COMP=<file>: per-component K3 records
     static Knobs read() {
         const char* mf = getenv("GDS_MF");
         const char* optr = getenv("GDS_MF_OPTR");
-        const char* warp = getenv("GDS_MF_WARP");
         const char* sel = getenv("GDS_DIRECT_SELECT");
-        return Knobs{mf && !strcmp(mf, "global"), mf && !strcmp(mf, "sm"), !optr || optr[0] != '0',
-                     warp && warp[0] == '1', sel && !strcmp(sel, "walk"), getenv("GDS_DUMP_COMP")};
+        return Knobs{mf && !strcmp(mf, "global"), !optr || optr[0] != '0', sel && !strcmp(sel, "walk"),
+                     getenv("GDS_DUMP_COMP")};
     }
 };
 
@@ -321,8 +318,7 @@ Mf2Plan plan_maxflow_sm(uint32_t n_comp, uint32_t max_comp_nodes, bool express_p
     // while (nearly) all components are resident at once.  A batch beyond that (config 5: 512
     // samples of 180 KB each, one per SM, four waves: 3.2 ms) is faster on k_maxflow, whose state
     // lives in L2/HBM but which runs every component concurrently (1.84 ms).
-    pl.classic_ok = !knobs.mf_global &&
-                    (knobs.mf_sm || (unsigned long long)n_comp * 2 <= 3ull * kNumSMs * per_sm);
+    pl.classic_ok = !knobs.mf_global && (unsigned long long)n_comp * 2 <= 3ull * kNumSMs * per_sm;
     if (!pl.classic_ok && !express_possible) return pl;
     pl.on = true;
     pl.smem = (int)((smem_ll + 15) & ~15ll);
@@ -338,11 +334,10 @@ Mf2Plan plan_maxflow_sm(uint32_t n_comp, uint32_t max_comp_nodes, bool express_p
 // k_maxflow: their frontiers hold tens of nodes with ~40 bundles each, the time is the per-bundle
 // global traffic of the warp passes, and 32 warps of 64 registers (k_maxflow) beat 16 warps with the
 // labels in shared memory (config 2 without its filter: 2.6 ms there, 3.0 ms here after batching the
-// loads of eight nodes per warp; 3.4 ms before).  GDS_MF_WARP=1 keeps them here (tests, measurements).
+// loads of eight nodes per warp; 3.4 ms before).
 template <int THREADS, int SLOT>
 void launch_mf2_shape(gds_ctx* c, const Mf2Plan& pl, const Mf2Graph& g, const K3Args& k,
-                      uint32_t* fb_list, uint32_t* fb_count, bool allow_warp,
-                      unsigned long long alg_bytes) {
+                      uint32_t* fb_list, uint32_t* fb_count, unsigned long long alg_bytes) {
     auto kern = k_maxflow_sm<THREADS>;
     raise_smem_limit(reinterpret_cast<const void*>(kern), c->device, pl.smem);
     // one full wave: k.n_comp is an estimate (one component per sample or segment), and the cuts at
@@ -351,7 +346,7 @@ void launch_mf2_shape(gds_ctx* c, const Mf2Plan& pl, const Mf2Graph& g, const K3
     const int grid = kNumSMs * pl.per_sm;
     launch("maxflow", alg_bytes, kern, grid, THREADS, pl.smem, c->stream, g, k.comp_lo, k.comp_hi,
            k.wc, k.qF, k.qT, k.qN, k.qH, k.sp, k.cstats, (uint32_t)pl.smem, pl.qcap, fb_list,
-           fb_count, pl.optr ? 1u : 0u, k.n_comp_dev, k.mft, allow_warp ? 1u : 0u);
+           fb_count, pl.optr ? 1u : 0u, k.n_comp_dev, k.mft);
 }
 
 // K3' (sweep.cuh): the minimum-cardinality solve.  One warp per component.
@@ -1477,7 +1472,7 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
             const Mf2Graph g2{sc.node, bund, sc.in_bid, in_src, d.outdeg, d.indeg, sc.dem_v,
                               sc.vs_d, sc.ns, express_on, mf2.classic_ok ? 1u : 0u, sc.dead};
             (mf2.per_sm >= 2 ? launch_mf2_shape<256, 0> : launch_mf2_shape<512, 1>)(
-                c, mf2, g2, k, fb_list, wc + 2, sc.knobs.mf_warp, mf_bytes);
+                c, mf2, g2, k, fb_list, wc + 2, mf_bytes);
             // whatever the shared-memory kernel could not take
             k.wc = wc + 1;
             launch_maxflow(c, MfArgs{mg, k, max_comp_nodes, fb_list, wc + 2, lab_g}, 0);

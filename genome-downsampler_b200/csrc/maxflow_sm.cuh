@@ -153,7 +153,7 @@ struct Mf2Comp {
     uint32_t lo, n, obase;
     uint32_t word_off, inF_off, bmA_off, bmB_off, optr_off;  // byte offsets (mf2_smem)
     uint32_t W4;
-    uint32_t have_optr, warp_mode, express;
+    uint32_t have_optr, express;
     uint32_t satn_off;  // bmB_off holds the snapshot the walkers read
     Q2 F, T, N, H;
 };
@@ -248,7 +248,7 @@ __device__ __forceinline__ void mf2_mark(const Mf2Comp& C, const Mf2Lvl& L, uint
 __device__ __forceinline__ void mf2_expand_multi(Mf2Shared& sh, const Mf2Lvl& nxt, uint32_t u) {
     const Mf2Comp& C = sh.C;
     const uint32_t in_lo = g_ld(&C.G.in_ptr[C.lo + u]), in_hi = g_ld(&C.G.in_ptr[C.lo + u + 1]);
-    if (C.warp_mode || in_hi - in_lo > kHeavyDeg) {
+    if (in_hi - in_lo > kHeavyDeg) {
         q2_append(C.H, &sh.nH, u);
         return;
     }
@@ -269,7 +269,7 @@ __device__ __forceinline__ void mf2_expand_flow(Mf2Shared& sh, const Mf2Lvl& nxt
     const uint4 hi4 = ld_node_hi(nr);
     const uint4 nx = ld_node_hi(nr + 1);
     if (u > 0 && (int32_t)hi4.y > 0) mf2_mark(C, nxt, u - 1);  // reverse of back arc u -> u-1
-    if (C.warp_mode || (nx.w - hi4.w) + (nx.z - hi4.z) > kHeavyDeg) {
+    if ((nx.w - hi4.w) + (nx.z - hi4.z) > kHeavyDeg) {
         q2_append(C.H, &sh.nH, u);
         return;
     }
@@ -354,20 +354,20 @@ __device__ __forceinline__ void mf2_bfs_heavy(Mf2Shared& sh, const Mf2Lvl& nxt, 
     }
 }
 
-// phase A, nodes with many bundles (warp mode: the whole frontier), one warp each.  The sequential
+// phase A, nodes with many bundles, one warp each.  The sequential
 // "push until the excess is gone" over the bundles in their fixed order is an exclusive prefix sum
 // of the admissible residuals across the lanes (maxflow.cuh).  Memory trips per node: its records;
 // then its last 64 out-bundles and the start nodes of its last 64 in-arcs together (two of each per
 // lane in flight); the flow of an in-bundle only when the labels admit cancelling it.
 template <int THREADS>
-__device__ __forceinline__ void mf2_push_heavy(Mf2Shared& sh, uint32_t nHA, unsigned long long& my_pushes,
+__device__ __forceinline__ void mf2_push_heavy(Mf2Shared& sh, uint32_t nH, unsigned long long& my_pushes,
                                             long long& my_sink) {
     const Mf2Comp& C = sh.C;
     const uint32_t lane = lane_id(), lo = C.lo, n = C.n;
     const uint32_t* word = mf2_smem(C.word_off);
 #pragma unroll 1
-    for (uint32_t h = threadIdx.x >> 5; h < nHA; h += THREADS / 32) {
-        const uint32_t i = C.warp_mode ? h : C.H.get(h);
+    for (uint32_t h = threadIdx.x >> 5; h < nH; h += THREADS / 32) {
+        const uint32_t i = C.H.get(h);
         const uint32_t ent = C.F.get(i);
         const uint32_t v = ent & 0xffffu;
         uint32_t ex = ent >> 16;  // uniform across the warp throughout
@@ -638,7 +638,7 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
              uint32_t* qH_g, SolveParams P, CompStats* __restrict__ stats, uint32_t smem_bytes,
              uint32_t qcap, uint32_t* __restrict__ fb_list, uint32_t* fb_count, uint32_t allow_optr,
              const uint32_t* __restrict__ n_comp_dev,
-             MfTotals* __restrict__ totals, uint32_t allow_warp) {
+             MfTotals* __restrict__ totals) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Mf2Shared& sh = *reinterpret_cast<Mf2Shared*>(smem_raw);
     const uint32_t word_off = kMf2HeaderBytes + 16u * qcap;
@@ -663,7 +663,6 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
         const Mf2Layout lay = mf2_layout(n, have_optr);
         uint32_t* const inF = word + lay.o_inF;
         uint16_t* const optr = reinterpret_cast<uint16_t*>(word + lay.o_optr);
-        const bool warp_mode = 2ull * n_bund > (unsigned long long)kHeavyDeg * n;
         const long long t_begin = clock64();
         if (tid == 0) {
             sh.nF = 0;
@@ -695,13 +694,15 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
             C.optr_off = word_off + 4u * lay.o_optr;
             C.W4 = lay.W4;
             C.have_optr = have_optr;
-            C.warp_mode = warp_mode;
             C.F = Q2{kMf2HeaderBytes, qF_g + lo, qcap};
             C.T = Q2{kMf2HeaderBytes + 4u * qcap, qT_g + lo, qcap};
             C.N = Q2{kMf2HeaderBytes + 8u * qcap, qN_g + lo, qcap};
             C.H = Q2{kMf2HeaderBytes + 12u * qcap, qH_g + lo, qcap};
         }
-        if (!fits || (warp_mode && !allow_warp)) {  // not for this kernel: k_maxflow takes it
+        // k_maxflow takes what does not fit, and the components whose nodes are mostly heavy (variable
+        // read lengths, tens of bundles per node): their time is the per-bundle global traffic of the
+        // warp passes, which shared-memory labels do not shorten (gds_api.cu: launch_mf2_shape)
+        if (!fits || 2ull * n_bund > (unsigned long long)kHeavyDeg * n) {
             if (tid == 0) fb_list[atomicAdd(fb_count, 1u)] = c;
             __syncthreads();
             continue;
@@ -761,12 +762,9 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
             if (lane == 0 && my_supply) atomicAdd(&sh.supply, min(my_supply, 0x10000u));
         }
         __syncthreads();
-        // k_maxflow takes what does not fit, and the components whose nodes are mostly heavy (variable
-        // read lengths, tens of bundles per node): their time is the per-bundle global traffic of the
-        // warp passes, which shared-memory labels do not shorten (config 2: 2.6 ms there, 3.4 ms here)
         // the express schedule: decided from the data alone (oracle: express_component)
         const bool express = G.express_on && (G.express_on == 2 || sh.supply >= kExpressMinSupply) &&
-                             !sh.not_benign && !warp_mode && n <= kExpressMaxNodes && sh.supply <= 0xffffu;
+                             !sh.not_benign && n <= kExpressMaxNodes && sh.supply <= 0xffffu;
         const uint32_t bl = express ? 0u : 1u;  // length of a back arc in the labels
         if (sh.supply > 0xffffu || (!express && !G.classic_ok)) {  // nothing has been written to global memory yet
             __syncthreads();
@@ -846,7 +844,7 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
             // ---------------- phase A: pushes (labels are constant in this phase) ----------------
             const long long t_a = clock64();
 #pragma unroll 1
-            for (uint32_t i = mf2_slot<THREADS>(); i < cntF && !warp_mode; i += THREADS) {
+            for (uint32_t i = mf2_slot<THREADS>(); i < cntF; i += THREADS) {
                 const uint32_t ent = F.get(i);
                 const uint32_t v = ent & 0xffffu;
                 uint32_t ex = ent >> 16;
@@ -955,15 +953,13 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
                 }
                 F.put(i, (ex << 16) | v);
             }
-            if (!warp_mode) __syncthreads();
-            const uint32_t nHA = warp_mode ? cntF : sh.nH;  // uniform
-            if (nHA) {  // ---- heavy nodes (warp mode: the whole frontier), one warp each
-                mf2_push_heavy<THREADS>(sh, nHA, my_pushes, my_sink);
+            __syncthreads();
+            const uint32_t nH = sh.nH;  // uniform
+            if (nH) {  // ---- heavy nodes, one warp each
+                mf2_push_heavy<THREADS>(sh, nH, my_pushes, my_sink);
                 __syncthreads();
-                if (!warp_mode) {
-                    if (tid == 0) sh.nH = 0;
-                    __syncthreads();
-                }
+                if (tid == 0) sh.nH = 0;
+                __syncthreads();
             }
             const uint32_t cntT = sh.nT;
             const long long t_b = clock64();
@@ -998,51 +994,47 @@ k_maxflow_sm(Mf2Graph G, const uint32_t* __restrict__ comp_lo, const uint32_t* _
                 if (left > 0 && dv != kInf16) {
                     ++my_relabels;
                     atomicAdd(&sh.relabels_since, 1u);
-                    if (warp_mode) {
-                        q2_append(H, &sh.nH, i);
+                    const NodeRec* nr = G.node + lo + v;
+                    // residual arcs of v: again loads that do not depend on each other
+                    uint4 bo = make_uint4(0, 0, 0, 0), bi = make_uint4(0, 0, 0, 0);
+                    uint32_t ob = 0, oe = 0;
+                    if (have_optr) {
+                        ob = obase + optr[v];
+                        oe = obase + optr[v + 1];
+                        if (oe > ob) bo = ld_bund(&G.bund[ob]);
+                    }
+                    if (one_each) bi = ld_bund(&G.bund[c_bid]);  // used only if v has in-arcs
+                    const uint4 hi4 = ld_node_hi(nr);
+                    const uint4 r_hi = ld_node_hi(nr + 1);
+                    if (!have_optr) {
+                        ob = hi4.z;
+                        oe = r_hi.z;
+                    }
+                    if ((oe - ob) + (r_hi.w - hi4.w) > kHeavyDeg) {
+                        q2_append(H, &sh.nH, i);  // the min over many bundles: warp pass below
                     } else {
-                        const NodeRec* nr = G.node + lo + v;
-                        // residual arcs of v: again loads that do not depend on each other
-                        uint4 bo = make_uint4(0, 0, 0, 0), bi = make_uint4(0, 0, 0, 0);
-                        uint32_t ob = 0, oe = 0;
-                        if (have_optr) {
-                            ob = obase + optr[v];
-                            oe = obase + optr[v + 1];
-                            if (oe > ob) bo = ld_bund(&G.bund[ob]);
-                        }
-                        if (one_each) bi = ld_bund(&G.bund[c_bid]);  // used only if v has in-arcs
-                        const uint4 hi4 = ld_node_hi(nr);
-                        const uint4 r_hi = ld_node_hi(nr + 1);
-                        if (!have_optr) {
-                            ob = hi4.z;
-                            oe = r_hi.z;
-                        }
-                        if ((oe - ob) + (r_hi.w - hi4.w) > kHeavyDeg) {
-                            q2_append(H, &sh.nH, i);  // the min over many bundles: warp pass below
-                        } else {
-                            uint32_t mn = kInf16;
-                            bool res_any = (int32_t)hi4.x > 0;
-                            if ((int32_t)hi4.x > 0) mn = 0;
+                        uint32_t mn = kInf16;
+                        bool res_any = (int32_t)hi4.x > 0;
+                        if ((int32_t)hi4.x > 0) mn = 0;
 #pragma unroll 1
-                            for (uint32_t b = ob; b < oe; ++b) {
-                                const uint4 br = (have_optr && b == ob) ? bo : ld_bund(&G.bund[b]);
-                                if (br.z < br.y) {
-                                    mn = min(mn, mf2_label(word, br.x - lo));
-                                    res_any = true;
-                                }
+                        for (uint32_t b = ob; b < oe; ++b) {
+                            const uint4 br = (have_optr && b == ob) ? bo : ld_bund(&G.bund[b]);
+                            if (br.z < br.y) {
+                                mn = min(mn, mf2_label(word, br.x - lo));
+                                res_any = true;
                             }
-                            if (express) mf2_sat_set(sh.C, v, !res_any);  // U3: exact, after the barrier
-                            if (v + 1 < n && (int32_t)r_hi.y > 0) mn = min(mn, mf2_label(word, v + 1));
-                            if (v > 0) mn = min(mn, mf2_label(word, v - 1) - (1u - bl));  // labels are >= 1
-#pragma unroll 1
-                            for (uint32_t k = hi4.w; k < r_hi.w; ++k) {
-                                const uint4 br = (one_each && k + 1 == r_hi.w)
-                                                     ? bi
-                                                     : ld_bund(&G.bund[g_ld(&G.in_bid[k])]);
-                                if (br.z > 0) mn = min(mn, mf2_label(word, br.w - lo));
-                            }
-                            nl = mn >= kInf16 - 1 ? kInf16 : mn + 1;
                         }
+                        if (express) mf2_sat_set(sh.C, v, !res_any);  // U3: exact, after the barrier
+                        if (v + 1 < n && (int32_t)r_hi.y > 0) mn = min(mn, mf2_label(word, v + 1));
+                        if (v > 0) mn = min(mn, mf2_label(word, v - 1) - (1u - bl));  // labels are >= 1
+#pragma unroll 1
+                        for (uint32_t k = hi4.w; k < r_hi.w; ++k) {
+                            const uint4 br = (one_each && k + 1 == r_hi.w)
+                                                 ? bi
+                                                 : ld_bund(&G.bund[g_ld(&G.in_bid[k])]);
+                            if (br.z > 0) mn = min(mn, mf2_label(word, br.w - lo));
+                        }
+                        nl = mn >= kInf16 - 1 ? kInf16 : mn + 1;
                     }
                 }
                 word[v] = (nl << 16) | dv;
