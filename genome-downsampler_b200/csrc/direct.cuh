@@ -27,9 +27,6 @@ constexpr int kDhThreads = 1024;
 constexpr int kDirectUnroll = 4;  // 16-byte loads per array in flight per thread
 constexpr int kDkThreads = 256;   // key tiles of the bundle kernels: 4 keys per thread
 constexpr int kDkTile = kDkThreads * 4;
-constexpr int kDsThreads = 1024;
-constexpr int kDsPer = 4;
-constexpr int kDsTile = kDsThreads * kDsPer;
 
 struct DirectLayout {
     const uint64_t* off;       // [ns+1] read offsets
@@ -536,13 +533,11 @@ k_direct_graph(const uint32_t* __restrict__ ghist, DirectLayout dl, uint32_t n_n
 // k_direct_classify writes the 2-bit code of every key (16 per word; a 30 kb sample's table is
 // 7.5 KB) and gives every partial bundle a segment of mult slots in a candidate buffer.
 // k_direct_mark streams the reads' starts once more, in parallel parts like the histogram: code 1
-// sets the kept bit, code 2 appends the read index to the bundle's segment.  k_direct_partial then ranks each partial bundle's candidates (one warp per
-// bundle).  If the candidates do not fit their buffer, ctl[2] is raised and the host repeats the
-// selection with the buffer grown to ctl[1].  If a partial bundle is huge (adversarial input:
-// millions of identical reads), ctl[2] is raised and the host repeats the selection with the
-// ordered walk below instead — same kept set, one CTA per sample.
+// sets the kept bit, code 2 appends the read index to the bundle's segment.  k_direct_partial then
+// ranks each partial bundle's candidates, one warp per bundle whatever its size.  If the candidates
+// do not fit their buffer, ctl[2] is raised and the host repeats the selection with the buffer grown
+// to ctl[1].
 constexpr uint32_t kSatCode = 1, kPartCode = 2;
-constexpr uint32_t kMaxPartialMult = 2048;  // candidates of one bundle ranked by one warp
 // 512 threads x 3 CTAs per SM at 40 registers: the kernel is bound by neither issue slots nor HBM
 // but by its stalls per instruction, so more resident warps pay — 1.27 ms with one CTA of 1024
 // threads (48 registers, half occupancy), 1.14 ms this way (config 5)
@@ -551,14 +546,14 @@ constexpr int kDmCtasPerSm = 3;
 constexpr uint32_t kDmSplit = 3;
 
 // ctl: [0] number of partial bundles, [1] candidate slots handed out, [2] flags: the mark and
-// ranking kernels do nothing when any is set — 1 a partial bundle too large for one warp (ordered
-// walk instead), 2 the candidates do not fit cand_cap (the host grows the buffer and repeats the
-// selection), 4 K2 counted bad reads (the call fails; the mark kernels do not re-validate)
+// ranking kernels do nothing when any is set — 2 the candidates do not fit cand_cap (the host grows
+// the buffer and repeats the selection), 4 K2 counted bad reads (the call fails; the mark kernels
+// do not re-validate)
 __global__ void __launch_bounds__(256)
 k_direct_classify(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ b_slot,
                   uint32_t* __restrict__ ghist, uint32_t* __restrict__ kstat,
                   uint32_t* __restrict__ pb_off, uint32_t* __restrict__ pb_f,
-                  uint32_t* __restrict__ pb_fill, uint32_t* __restrict__ ctl, uint32_t max_mult,
+                  uint32_t* __restrict__ pb_fill, uint32_t* __restrict__ ctl,
                   const uint32_t* __restrict__ B_dev, uint32_t cand_cap,
                   const uint32_t* __restrict__ stats) {
     __shared__ uint32_t tot_n, tot_m, base_n, base_m;
@@ -588,7 +583,6 @@ k_direct_classify(const BundleRec* __restrict__ bund, const uint32_t* __restrict
         code = kPartCode;
         const uint32_t pid = base_n + my_n;
         const uint32_t o = base_m + my_m;
-        if (mult > max_mult) atomicOr(&ctl[2], 1u);  // too many candidates for one warp: ordered walk
         pb_off[pid] = o;
         pb_f[pid] = f;
         pb_fill[pid] = 0;
@@ -847,131 +841,6 @@ k_direct_partial(const uint32_t* __restrict__ pb_off, const uint32_t* __restrict
     kept = __reduce_add_sync(0xffffffffu, kept);
     if (lane == 0 && kept) atomicAdd(&totals[1], (unsigned long long)kept);
 }
-
-// ---- K5 direct, fallback: ordered walk -----------------------------------------------------------
-// One CTA per sample holds the per-key quota (= f) in shared memory and walks the reads in index
-// order, tile by tile; a read whose key still has quota is a candidate.  If a tile holds no more
-// candidates of a key than its quota they are all kept (order irrelevant); otherwise (each key at
-// most once) the candidates of that key are ranked by index.  The walk stops when every quota is
-// used up.
-__global__ void __launch_bounds__(256)
-k_direct_quota(const BundleRec* __restrict__ bund, const uint32_t* __restrict__ b_slot,
-               uint32_t* __restrict__ ghist, const uint32_t* __restrict__ B_dev) {
-    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b < *B_dev) ghist[b_slot[b]] = bund[b].f;
-}
-
-__global__ void __launch_bounds__(kDsThreads, 1)
-k_direct_select(const uint32_t* __restrict__ S, DirectLayout dl, uint32_t* __restrict__ work_counter,
-                const uint32_t* __restrict__ ghist, uint32_t* __restrict__ bitmap,
-                unsigned long long* __restrict__ totals) {
-    extern __shared__ uint32_t quota[];  // per key (start node): flow still to be handed out (as int32)
-    __shared__ uint32_t c_key[kDsTile];
-    __shared__ uint16_t c_pos[kDsTile];
-    __shared__ uint32_t s_k, s_nconf, s_remaining;
-    const uint32_t tid = threadIdx.x;
-    constexpr uint32_t kNone = 0xffffffffu;
-    for (;;) {
-        if (tid == 0) {
-            s_k = atomicAdd(work_counter, 1u);
-            s_remaining = 0;
-        }
-        __syncthreads();
-        const uint32_t k = s_k;
-        if (k >= dl.ns) break;
-        const uint64_t base = dl.off[k];
-        const uint64_t n_k = dl.off[k + 1] - base;
-        const uint32_t kk = dl.kbase[k + 1] - dl.kbase[k];
-        const uint32_t* gq = ghist + dl.kbase[k];
-        uint32_t want = 0;
-        for (uint32_t i = tid; i < kk; i += kDsThreads) {
-            const uint32_t f = gq[i];
-            quota[i] = f;
-            want += f;
-        }
-        want = __reduce_add_sync(0xffffffffu, want);
-        if (lane_id() == 0 && want) atomicAdd(&s_remaining, want);
-        __syncthreads();
-        const uint32_t total = s_remaining;
-        if (total != 0) {
-            const uint32_t n_tiles = (uint32_t)((n_k + kDsTile - 1) / kDsTile);
-            uint32_t ns_[kDsPer];
-            auto fetch = [&](uint32_t t) {
-#pragma unroll
-                for (int q = 0; q < kDsPer; ++q) {
-                    const uint64_t idx = (uint64_t)t * kDsTile + q * kDsThreads + tid;
-                    ns_[q] = idx < n_k ? ld_stream(S + base + idx) : kNone;
-                }
-            };
-            fetch(0);
-            for (uint32_t t = 0; t < n_tiles; ++t) {
-                uint32_t key[kDsPer];
-                bool cand[kDsPer];
-                bool any = false;
-#pragma unroll
-                for (int q = 0; q < kDsPer; ++q) {
-                    key[q] = ns_[q] < kk ? ns_[q] : kNone;
-                    cand[q] = key[q] != kNone && (int32_t)quota[key[q]] > 0;
-                    any |= cand[q];
-                }
-                if (t + 1 < n_tiles) fetch(t + 1);  // in flight while this tile is resolved
-                if (!__syncthreads_or(any)) continue;
-                if (tid == 0) s_nconf = 0;
-#pragma unroll
-                for (int q = 0; q < kDsPer; ++q)
-                    if (cand[q]) atomicSub(&quota[key[q]], 1u);
-                __syncthreads();
-                uint32_t kept = 0;
-                const uint64_t tile0 = base + (uint64_t)t * kDsTile;
-#pragma unroll
-                for (int q = 0; q < kDsPer; ++q) {
-                    if (!cand[q]) continue;
-                    const uint32_t pos = q * kDsThreads + tid;
-                    if ((int32_t)quota[key[q]] >= 0) {  // the tile did not exhaust the key
-                        const uint64_t g = tile0 + pos;
-                        atomicOr(&bitmap[g >> 5], 1u << (g & 31));
-                        ++kept;
-                    } else {
-                        const uint32_t slot = atomicAdd(&s_nconf, 1u);
-                        c_key[slot] = key[q];
-                        c_pos[slot] = (uint16_t)pos;
-                    }
-                }
-                __syncthreads();
-                const uint32_t nconf = s_nconf;
-                if (nconf) {
-                    // more candidates than quota: the lowest-index ones win (each key gets here
-                    // at most once, its quota is zero afterwards)
-                    for (uint32_t e = tid; e < nconf; e += kDsThreads) {
-                        const uint32_t ck = c_key[e];
-                        const uint32_t cp = c_pos[e];
-                        uint32_t rank = 0, cnt = 0;
-                        for (uint32_t j = 0; j < nconf; ++j) {
-                            const bool same = c_key[j] == ck;
-                            cnt += same;
-                            rank += same && c_pos[j] < cp;
-                        }
-                        const int32_t q0 = (int32_t)quota[ck] + (int32_t)cnt;
-                        if ((int32_t)rank < q0) {
-                            const uint64_t g = tile0 + cp;
-                            atomicOr(&bitmap[g >> 5], 1u << (g & 31));
-                            ++kept;
-                        }
-                    }
-                    __syncthreads();
-                    for (uint32_t e = tid; e < nconf; e += kDsThreads) quota[c_key[e]] = 0;
-                }
-                kept = __reduce_add_sync(0xffffffffu, kept);
-                if (lane_id() == 0 && kept) atomicSub(&s_remaining, kept);
-                __syncthreads();
-                if (s_remaining == 0) break;
-            }
-            if (tid == 0) atomicAdd(&totals[1], (unsigned long long)(total - s_remaining));
-        }
-        __syncthreads();
-    }
-}
-
 
 // ---- the same idea with the histogram in global memory ------------------------------------------
 // When the reads have several lengths (config 2), a sample does not fit one SM, or the reference is

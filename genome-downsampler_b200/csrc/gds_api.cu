@@ -57,8 +57,6 @@ struct gds_ctx {
     DevBuf unc, adj, fmult, dead;  // forced reads out, cuts in (graph.cuh)
     DevBuf dhist, dlay, b_slot, ident, dwork;  // direct (sort-free) bundle path
     DevBuf kstat, pbund, cand, dctl, in_src, dem_v, fb_list, in1, lab_g, taken;
-    unsigned sweep_smem_set = 0;  // bit i: the sweep launch shape i has its shared memory set up
-    unsigned direct_attr = 0;                  // bytes of dynamic smem the direct kernels are set up for
     bool atomic_rank = false;  // shared-memory atomics rank in lane order on this device (probed)
     Profiler prof;
 
@@ -119,14 +117,11 @@ void deliver(gds_ctx* c, T* dst, const T* dev_src, size_t n, bool dst_on_device)
 struct Knobs {
     bool mf_global;         // GDS_MF=global: the round-1 kernel only
     bool mf_optr;           // GDS_MF_OPTR=0: k_maxflow_sm without the out-CSR cache
-    bool walk;              // GDS_DIRECT_SELECT=walk: K5 of the histogram path takes the ordered walk
     const char* dump_comp;  // GDS_DUMP_COMP=<file>: per-component K3 records
     static Knobs read() {
         const char* mf = getenv("GDS_MF");
         const char* optr = getenv("GDS_MF_OPTR");
-        const char* sel = getenv("GDS_DIRECT_SELECT");
-        return Knobs{mf && !strcmp(mf, "global"), !optr || optr[0] != '0', sel && !strcmp(sel, "walk"),
-                     getenv("GDS_DUMP_COMP")};
+        return Knobs{mf && !strcmp(mf, "global"), !optr || optr[0] != '0', getenv("GDS_DUMP_COMP")};
     }
 };
 
@@ -360,15 +355,12 @@ struct SweepArgs {
     unsigned long long* fail;
 };
 
-template <int W, int CAP, bool WARP, int SLOT>
+template <int W, int CAP, bool WARP>
 void launch_sweep_shape(gds_ctx* c, const SweepArgs& a, unsigned long long alg_bytes) {
     constexpr int smem = kSweepWarps * (2 * W + 4 * CAP + 2 * 34 + 2 * 32) * 4;
     const int grid = std::max(1, std::min<int>(div_up(a.n_comp, kSweepWarps), kNumSMs * 8));
     auto kern = WARP ? k_sweep_warp<W, CAP> : k_sweep<W, CAP>;
-    if (!(c->sweep_smem_set & (1u << SLOT))) {
-        GDS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        c->sweep_smem_set |= 1u << SLOT;
-    }
+    raise_smem_limit(reinterpret_cast<const void*>(kern), c->device, smem);
     launch("sweep", alg_bytes, kern, grid, kSweepWarps * 32, smem, c->stream, a.g, a.comp_lo,
            a.comp_hi, a.n_comp_dev, a.M, a.wc, a.fail);
 }
@@ -377,9 +369,9 @@ void launch_sweep(gds_ctx* c, const SweepArgs& a, uint32_t maxlen, bool one_len,
                   unsigned long long alg_bytes) {
     using Launch = void (*)(gds_ctx*, const SweepArgs&, unsigned long long);
     static constexpr Launch kShapes[6] = {
-        launch_sweep_shape<256, 64, false, 0>,  launch_sweep_shape<256, 1024, true, 1>,
-        launch_sweep_shape<1024, 64, false, 2>, launch_sweep_shape<1024, 1024, true, 3>,
-        launch_sweep_shape<4096, 64, false, 4>, launch_sweep_shape<4096, 1024, true, 5>};
+        launch_sweep_shape<256, 64, false>,  launch_sweep_shape<256, 1024, true>,
+        launch_sweep_shape<1024, 64, false>, launch_sweep_shape<1024, 1024, true>,
+        launch_sweep_shape<4096, 64, false>, launch_sweep_shape<4096, 1024, true>};
     // one read length: at most a few bundles per position -> one lane walks; several lengths: tens of
     // arrivals per position -> the warp-synchronous walk adds them in parallel
     const int w = maxlen < 256 ? 0 : maxlen < 1024 ? 1 : 2;
@@ -684,15 +676,10 @@ void build_bundles_direct(gds_ctx* c, SolveCall& sc) {
     GDS_CUDA(cudaMemsetAsync(wc, 0, 8, st));
     const DirectLayout dl{sc.foff_dev, sc.reflen_d, sc.base_d, lay_d, lay_d + ns + 1, ns, sc.minlen};
     const unsigned smem = kmax * 4;
-    if (smem > c->direct_attr) {
-        GDS_CUDA(cudaFuncSetAttribute(k_direct_hist, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(kDirectMaxKeys * 4)));
-        GDS_CUDA(cudaFuncSetAttribute(k_direct_select, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(kDirectMaxKeys * 4)));
-        GDS_CUDA(cudaFuncSetAttribute(k_direct_mark, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(kDmQueueBytes + kDirectMaxKeys)));
-        c->direct_attr = kDirectMaxKeys * 4;
-    }
+    raise_smem_limit(reinterpret_cast<const void*>(k_direct_hist), c->device,
+                     (int)(kDirectMaxKeys * 4));
+    raise_smem_limit(reinterpret_cast<const void*>(k_direct_mark), c->device,
+                     (int)(kDmQueueBytes + kDirectMaxKeys));
     launch("direct_hist", 8ull * N + 4ull * ktot, k_direct_hist,
            (int)std::min<uint32_t>(n_items, (uint32_t)kNumSMs), kDhThreads, smem, st, sc.S, sc.E, dl,
            n_items, wc, ghist, kmax, sc.stats());
@@ -740,14 +727,12 @@ void build_bundles_gdirect(gds_ctx* c, SolveCall& sc) {
 }
 
 // K5 on the direct path (direct.cuh): classify the bundles, mark the reads of saturated bundles in
-// one parallel streaming pass, rank the candidates of partial bundles; the ordered walk is the
-// fallback when a partial bundle is too large for one warp (or GDS_DIRECT_SELECT=walk asks for it).
-// Nothing is read back here.  The candidate buffer keeps the size it has (never below N/8 slots or
-// cand_need); k_direct_classify raises ctl flag 2 when the candidates do not fit and flag 1 for a
-// partial bundle too large for one warp, the mark / ranking kernels then do nothing, and
-// select_reads — which sees the flags with the final readback — repeats the selection: with a
-// larger buffer, or with the ordered walk right away (force_walk).
-void direct_select(gds_ctx* c, SolveCall& sc, bool force_walk, size_t cand_need) {
+// one parallel streaming pass, rank the candidates of partial bundles.  Nothing is read back here.
+// The candidate buffer keeps the size it has (never below N/8 slots or cand_need);
+// k_direct_classify raises ctl flag 2 when the candidates do not fit, the mark / ranking kernels
+// then do nothing, and select_reads — which sees the flag with the final readback — repeats the
+// selection with a larger buffer.
+void direct_select(gds_ctx* c, SolveCall& sc, size_t cand_need) {
     cudaStream_t st = sc.st;
     const DirectPlan& dp = sc.direct;
     const uint32_t B = sc.B;
@@ -759,47 +744,34 @@ void direct_select(gds_ctx* c, SolveCall& sc, bool force_walk, size_t cand_need)
     uint32_t* b_slot = c->b_slot.as<uint32_t>();
     uint32_t* ctl = c->dctl.get<uint32_t>(4);
     GDS_CUDA(cudaMemsetAsync(ctl, 0, 16, st));
-    if (dp.global || !(force_walk || sc.knobs.walk)) {
-        uint32_t* kstat = c->kstat.get<uint32_t>(dp.ktot / 16 + 1);
-        uint32_t* pb = c->pbund.get<uint32_t>(3 * ((size_t)B + 1));
-        uint32_t* fill = pb + 2 * ((size_t)B + 1);
-        GDS_CUDA(cudaMemsetAsync(kstat, 0, ((size_t)dp.ktot / 16 + 1) * 4, st));
-        // never below N/8 slots: the share of reads in partial bundles varies from call to call
-        // and regrowing the arena is expensive
-        size_t cand_cap = std::max<size_t>({cand_need, N / 8, c->cand.cap / 4, (size_t)1});
-        cand_cap = std::min<size_t>(cand_cap, 0xffffffffu);
-        uint32_t* cand = c->cand.get<uint32_t>(cand_cap);
-        // a partial bundle beyond kMaxPartialMult reads sends the shared-memory path to the
-        // ordered walk; the global path has no walk and lets one warp grind through it
-        launch("direct_classify", 20ull * B, k_direct_classify, div_up(B, 256), 256, 0, st, bund,
-               b_slot, dp.ghist, kstat, pb, pb + B + 1, fill, ctl,
-               dp.global ? 0xffffffffu : kMaxPartialMult, B_dev, (uint32_t)cand_cap, sc.stats());
-        if (dp.global) {
-            launch("gdirect_mark", 8ull * N + dp.ktot / 4 + 8ull * N / 32, k_gdirect_mark,
-                   div_up((long long)N, kGdTile), kGdThreads, 0, st, sc.S, sc.E, N, dp.gl, dp.ghist,
-                   kstat, pb, fill, cand, bm, totals, ctl);
-        } else {
-            uint32_t* wc = c->dwork.as<uint32_t>() + 1;
-            GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
-            const int grid = (int)std::min<uint32_t>(dp.n_items * kDmSplit, (uint32_t)kNumSMs * kDmCtasPerSm);
-            launch("direct_mark", 4ull * N + dp.ktot / 4 + 8ull * N / 32, k_direct_mark, grid, kDmThreads,
-                   kDmQueueBytes + dp.kmax, st, sc.S, dp.dl, dp.n_items, wc, dp.ghist, kstat, pb, fill,
-                   cand, ctl, bm, totals);
-        }
-        // segments of a long reference (global path): ~10 reads per bundle, half a warp each
-        launch("direct_partial", 16ull * (N / 64),
-               dp.global ? k_direct_partial<true> : k_direct_partial<false>, kNumSMs * 32, 256, 0, st,
-               pb, pb + B + 1, fill, cand, ctl, bm, totals);
+    uint32_t* kstat = c->kstat.get<uint32_t>(dp.ktot / 16 + 1);
+    uint32_t* pb = c->pbund.get<uint32_t>(3 * ((size_t)B + 1));
+    uint32_t* fill = pb + 2 * ((size_t)B + 1);
+    GDS_CUDA(cudaMemsetAsync(kstat, 0, ((size_t)dp.ktot / 16 + 1) * 4, st));
+    // never below N/8 slots: the share of reads in partial bundles varies from call to call
+    // and regrowing the arena is expensive
+    size_t cand_cap = std::max<size_t>({cand_need, N / 8, c->cand.cap / 4, (size_t)1});
+    cand_cap = std::min<size_t>(cand_cap, 0xffffffffu);
+    uint32_t* cand = c->cand.get<uint32_t>(cand_cap);
+    launch("direct_classify", 20ull * B, k_direct_classify, div_up(B, 256), 256, 0, st, bund,
+           b_slot, dp.ghist, kstat, pb, pb + B + 1, fill, ctl, B_dev, (uint32_t)cand_cap,
+           sc.stats());
+    if (dp.global) {
+        launch("gdirect_mark", 8ull * N + dp.ktot / 4 + 8ull * N / 32, k_gdirect_mark,
+               div_up((long long)N, kGdTile), kGdThreads, 0, st, sc.S, sc.E, N, dp.gl, dp.ghist,
+               kstat, pb, fill, cand, bm, totals, ctl);
     } else {
-        // ordered walk: one CTA per sample, quota per key in shared memory
-        launch("direct_quota", 24ull * B, k_direct_quota, div_up(B, 256), 256, 0, st, bund, b_slot,
-               dp.ghist, B_dev);
         uint32_t* wc = c->dwork.as<uint32_t>() + 1;
         GDS_CUDA(cudaMemsetAsync(wc, 0, 4, st));
-        launch("direct_walk", 4ull * dp.ktot + 8ull * N / 32, k_direct_select,
-               (int)std::min<uint32_t>(sc.ns, (uint32_t)kNumSMs), kDsThreads, dp.kmax * 4, st, sc.S,
-               dp.dl, wc, dp.ghist, bm, totals);
+        const int grid = (int)std::min<uint32_t>(dp.n_items * kDmSplit, (uint32_t)kNumSMs * kDmCtasPerSm);
+        launch("direct_mark", 4ull * N + dp.ktot / 4 + 8ull * N / 32, k_direct_mark, grid, kDmThreads,
+               kDmQueueBytes + dp.kmax, st, sc.S, dp.dl, dp.n_items, wc, dp.ghist, kstat, pb, fill,
+               cand, ctl, bm, totals);
     }
+    // segments of a long reference (global path): ~10 reads per bundle, half a warp each
+    launch("direct_partial", 16ull * (N / 64),
+           dp.global ? k_direct_partial<true> : k_direct_partial<false>, kNumSMs * 32, 256, 0, st,
+           pb, pb + B + 1, fill, cand, ctl, bm, totals);
     GDS_CUDA(cudaMemcpyAsync(sc.ds->ctl, ctl, 16, cudaMemcpyDeviceToDevice, st));
 }
 
@@ -1488,8 +1460,7 @@ void solve_flow(gds_ctx* c, SolveCall& sc) {
 
 // K5 (selection), K6 (verification) and the final readback.  One pass in the normal case.  On a
 // histogram path the selection may have to be repeated once: the final readback is the first time
-// the host sees that the candidates of the partial bundles did not fit their buffer (it grows) or
-// that a partial bundle needs the ordered walk.
+// the host sees that the candidates of the partial bundles did not fit their buffer (it grows).
 void select_reads(gds_ctx* c, SolveCall& sc) {
     const uint32_t B = sc.B, n_onodes = sc.n_onodes;
     const uint64_t N = sc.N;
@@ -1501,14 +1472,13 @@ void select_reads(gds_ctx* c, SolveCall& sc) {
     uint32_t* bm = sc.bm = (sc.out_dev && out->kept_bitmap) ? out->kept_bitmap
                                                             : c->bitmap.get<uint32_t>(n_words + 1);
     StatsBlock& h = sc.hstat;
-    bool force_walk = false;
     size_t cand_need = 0;
     for (int attempt = 0;; ++attempt) {
         if (sc.do_solve) {
             GDS_CUDA(cudaMemsetAsync(bm, 0, n_words * 4, st));
             if (attempt) GDS_CUDA(cudaMemsetAsync(&sc.ds->n_kept, 0, 16, st));  // n_kept, violations
             if (B && sc.direct.on)
-                direct_select(c, sc, force_walk, cand_need);
+                direct_select(c, sc, cand_need);
             else if (B)
                 launch("select", 8ull * B + 8ull * N / 32, k_select, div_up(B, 256), 256, 0, st,
                        c->b_first.as<uint32_t>(), c->bund.as<BundleRec>(), sc.sorted_idx, B, bm, totals);
@@ -1538,9 +1508,8 @@ void select_reads(gds_ctx* c, SolveCall& sc) {
         d2h_sync(c, &h, sc.ds, 1);
         input_verdict(h);
         const uint32_t cflags = sc.do_solve && B && sc.direct.on ? h.ctl[2] : 0;
-        if (attempt || !(cflags & 3u)) break;
-        force_walk = (cflags & 1u) != 0;  // ordered walk (shared-memory path)
-        cand_need = (size_t)h.ctl[1] + 1;  // or the buffer the candidates need
+        if (attempt || !(cflags & 2u)) break;
+        cand_need = (size_t)h.ctl[1] + 1;  // the buffer the candidates need
     }
     out->n_bundles = h.n_bundles;
     out->n_components = h.n_comp;

@@ -371,16 +371,6 @@ def test_histogram_paths_equal_sort_path(solver, O):
         assert np.array_equal(res[bmode].demand, res[1].demand)
         assert np.array_equal(res[bmode].cov_capped, res[1].cov_capped)
     assert_parity(O, res[0], s, e, [30_000] * 3, off, 300)
-    # K5 of the histogram path has two implementations (parallel mark + partial-bundle ranking,
-    # and the ordered walk it falls back to): same kept set
-    import os
-    os.environ["GDS_DIRECT_SELECT"] = "walk"
-    try:
-        rw = solver.solve(s, e, [30_000] * 3, 300, read_off=off, params=PRM + (0, 2), verify=True)
-    finally:
-        del os.environ["GDS_DIRECT_SELECT"]
-    assert rw.sort_passes == 0 and rw.n_kept == res[1].n_kept and rw.verify_violations == 0
-    assert np.array_equal(rw.kept_bitmap, res[1].kept_bitmap)
     # several read lengths take the global histogram, even where (ref_len + 1) x #lengths would
     # fit in shared memory
     rng = np.random.default_rng(11)
@@ -428,22 +418,23 @@ def test_histogram_paths_equal_sort_path(solver, O):
     assert_parity(O, re, sb, eb, [150_000, 20_000], offb, 60, prm_seg)
 
 
-def test_direct_selection_walk_many_tiles_and_duplicates(solver, O):
-    # the ordered walk of K5 (direct path): tiny key spaces so that every 4096-read tile holds many
-    # reads of one key, quotas that run out in the middle of a tile or span several tiles, ragged
-    # sample offsets (unaligned 16-byte loads at part boundaries).  Every fourth input has one read
-    # length R, which the shared-memory histogram and its walk need; the others draw lengths per
-    # sample and clip them at the reference's end, so most of them take the global histogram.
+def test_direct_selection_tiny_key_spaces_and_duplicates(solver, O):
+    # K5 of the histogram paths on tiny key spaces: thousands of reads per key, so partial bundles of
+    # far more than 128 candidates (k_direct_partial's bisection over candidates beyond its
+    # registers), and ragged sample offsets (unaligned 16-byte loads at part boundaries).  Every
+    # fourth input has one read length R, which the shared-memory histogram needs; the others draw
+    # lengths per sample and clip them at the reference's end, so most of them take the global
+    # histogram.
     rng = np.random.default_rng(23)
     for it in range(40):
-        walk = it % 4 == 0
+        one_len = it % 4 == 0
         ns = int(rng.integers(1, 4))
         Ls = rng.integers(2, 60, size=ns).astype(np.uint32)
         R = int(rng.integers(1, int(Ls.min()) + 1))
         ss, ee, off = [], [], [0]
         for L in Ls:
             n = int(rng.integers(0, 30_000))
-            if walk:
+            if one_len:
                 s = rng.integers(0, L - R + 1, size=n)
                 e = s + R - 1
             else:
@@ -458,16 +449,8 @@ def test_direct_selection_walk_many_tiles_and_duplicates(solver, O):
                          want_vectors=True)
         assert r.sort_passes == 0 or len(s) == 0
         assert_parity(O, r, s, e, Ls, off, M)
-        if walk:  # and the ordered walk on the same input
+        if one_len:
             assert r.bundle_path == 1
-            import os
-            os.environ["GDS_DIRECT_SELECT"] = "walk"
-            try:
-                rw = solver.solve(s, e, Ls, M, read_off=off, params=PRM + (0, 2), verify=True)
-            finally:
-                del os.environ["GDS_DIRECT_SELECT"]
-            assert np.array_equal(rw.kept_bitmap, r.kept_bitmap) and rw.n_kept == r.n_kept
-            assert rw.bundle_path == 1
 
 
 def test_compact_transport_start16_and_implied_end(pkg, solver, O):

@@ -629,12 +629,15 @@ def test_selection_retry_grows_the_candidate_buffer(pkg, O):
 
 
 @gpu
-def test_selection_retry_forces_the_ordered_walk(pkg, O):
-    # 5000 identical reads, M = 17: one partial bundle of more than 2048 reads is too large for one
-    # warp's ranking, so the call repeats the selection with the ordered walk
+def test_selection_ranks_a_partial_bundle_beyond_2048_reads(pkg, O):
+    # 5000 identical reads, M = 17: one partial bundle of 5000 candidates on the shared-memory
+    # histogram path, ranked by one warp's bisection.  Its candidates overflow the N/8 slots of a
+    # fresh context, so the selection runs twice.
     s = np.full(5000, 10, np.uint32)
     e = np.full(5000, 60, np.uint32)
     r, again, unhinted, prof = _retry_then_unhinted(pkg, O, s, e, 100, 17, PRM + (0, 0), (51, 51))
     assert r.bundle_path == 1 and r.n_bundles == 1
-    assert prof.get("direct_mark") == 1 and prof.get("direct_walk") == 1, prof
+    assert r.partial_bundles == 1 and r.partial_candidates == 5000
+    assert prof.get("direct_classify") == 2 and prof.get("direct_partial") == 2, prof
+    assert "direct_walk" not in prof and "direct_quota" not in prof, prof
     assert pkg.Solver.bitmap_to_indices(r.kept_bitmap, 5000).tolist() == list(range(17))

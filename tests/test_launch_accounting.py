@@ -35,7 +35,6 @@ def _cases(O):
         "global_several_lengths": (several, 60, dict(params=PRM + (0, 2), len_hint=(150, 152)), {}),
         "global_hist_segmented": (seg, 60, dict(params=(64, 150, 1, 0, 8192, 0)), {}),
         "pair_filter": (filt, 100, dict(params=PRM), {}),
-        "direct_walk": (batch, 60, dict(params=PRM + (0, 2)), {"GDS_DIRECT_SELECT": "walk"}),
         "maxflow_global": (batch, 60, dict(params=PRM), {"GDS_MF": "global"}),
         "express": (batch, 400, dict(params=PRM), {}),
         "min_cardinality": (batch, 60, dict(params=PRM + (0, 0, 1)), {}),
@@ -43,7 +42,7 @@ def _cases(O):
 
 
 PATHS = ["radix_sort", "direct_one_length", "global_several_lengths", "global_hist_segmented",
-         "pair_filter", "direct_walk", "maxflow_global", "express", "min_cardinality"]
+         "pair_filter", "maxflow_global", "express", "min_cardinality"]
 
 
 @pytest.mark.parametrize("path", PATHS)

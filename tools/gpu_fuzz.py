@@ -1,7 +1,7 @@
 """Randomised parity campaign (GPU vs oracle replay), wider than the pytest fuzz: batches, ragged and
-empty samples, variable lengths (heavy nodes), short segments, read-length hints, both bundle paths
-(radix sort / shared-memory histogram), both K5 variants of the histogram path (mark + partial
-ranking / ordered walk) and the compact transport (16-bit starts, implied ends).
+empty samples, variable lengths (heavy nodes), short segments, read-length hints, the bundle paths
+(radix sort / shared-memory or global-memory histogram) and the compact transport (16-bit starts,
+implied ends).
 Run from the repo root on a GPU box:  python tools/gpu_fuzz.py [N_CASES] [SEED]"""
 import os
 import sys
@@ -51,9 +51,6 @@ def main():
         if len(s) and rng.integers(0, 2):
             hint = (int(lens.min()), int(lens.max()))
         bmode = int(rng.integers(0, 3))  # gds_params.bundle_mode: choose / sort / histogram
-        walk = bool(rng.integers(0, 4) == 0)
-        if walk:
-            os.environ["GDS_DIRECT_SELECT"] = "walk"
         s_in, e_in = s, e
         if len(s) and lens.min() == lens.max() and rng.integers(0, 2):  # compact transport
             hint = (int(lens.min()), int(lens.max()))
@@ -75,13 +72,11 @@ def main():
         except Exception as ex:  # noqa: BLE001
             ok = False
             print("case %d raised %r" % (it, ex))
-        finally:
-            os.environ.pop("GDS_DIRECT_SELECT", None)
         if not ok:
             bad += 1
-            print("MISMATCH case %d: ns=%d n=%d Ls=%s M=%d prm=%s hint=%s bundle_mode=%d walk=%s "
-                  "compact=%s schedule=%d" % (it, ns, len(s), Ls.tolist(), M, prm, hint, bmode, walk,
-                                  (e_in is None, s_in.dtype.name), sched), flush=True)
+            print("MISMATCH case %d: ns=%d n=%d Ls=%s M=%d prm=%s hint=%s bundle_mode=%d "
+                  "compact=%s schedule=%d" % (it, ns, len(s), Ls.tolist(), M, prm, hint, bmode,
+                                              (e_in is None, s_in.dtype.name), sched), flush=True)
             if bad > 5:
                 break
     print("fuzz: %d cases, %d mismatches, %d components on the express schedule" % (it + 1, bad, n_express))
