@@ -240,6 +240,13 @@ void launch_maxflow(gds_ctx* c, const MfArgs& a, unsigned long long alg_bytes) {
 }
 
 constexpr int kMf2MaxSmem = 227 * 1024;
+constexpr uint32_t kMf2MinQcap = 256;  // staged entries per frontier queue, at the least
+// The express schedule runs only in k_maxflow_sm, and a component the launch cannot hold goes to
+// k_maxflow: every launch, even one clamped to kMf2MaxSmem with the smallest queues, must hold the
+// largest express component, or its schedule would depend on the other components of the call.
+static_assert(kMf2HeaderBytes + 16u * kMf2MinQcap + mf2_node_bytes(kExpressMaxNodes, false) <=
+                  (uint32_t)kMf2MaxSmem,
+              "an express component must fit every k_maxflow_sm launch");
 
 // Whether this call's components go to k_maxflow_sm, and with which launch shape.
 // gds_params.seg_len == 0 (include/gds.h): 16 384 positions, stretched by up to a quarter when that
@@ -288,11 +295,12 @@ Mf2Plan plan_maxflow_sm(uint32_t n_comp, uint32_t max_comp_nodes, bool express_p
     uint32_t qcap = 2048;
     bool optr = knobs.mf_optr;
     // the queues shrink before the node arrays do
-    while (qcap > 256 && need(nmax, optr, qcap) > kMf2MaxSmem) qcap >>= 1;
+    while (qcap > kMf2MinQcap && need(nmax, optr, qcap) > kMf2MaxSmem) qcap >>= 1;
     if (need(nmax, optr, qcap) > kMf2MaxSmem) optr = false;
-    if (need(nmax, optr, qcap) > kMf2MaxSmem && max_comp_nodes > nmax) return pl;
     long long smem_ll = need(nmax, optr, qcap);
-    if (smem_ll > kMf2MaxSmem) smem_ll = kMf2MaxSmem;  // the largest does not fit; smaller ones may
+    // the largest does not fit (beyond 50 672 nodes): the launch takes all an SM has, which holds
+    // every express component (static_assert above); the kernel puts the longer ones on fb_list
+    if (smem_ll > kMf2MaxSmem) smem_ll = kMf2MaxSmem;
     // CTAs per SM: by shared memory, and never more than two (128 registers x 256 threads each)
     auto resident = [&](long long bytes) {
         return std::min(2, std::max(1, (int)((228 * 1024) / (bytes + 1024))));

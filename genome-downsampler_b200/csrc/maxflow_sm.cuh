@@ -69,8 +69,8 @@ constexpr uint32_t kExpressMaxNodes = 40961, kExpressEdge = 512, kExpressMinSupp
 struct Mf2Layout {
     uint32_t W, W4, o_inF, o_A, o_B, o_Sn, o_optr, words;
 };
-__host__ __device__ inline Mf2Layout mf2_layout(uint32_t n, bool optr) {
-    Mf2Layout L;
+__host__ __device__ constexpr Mf2Layout mf2_layout(uint32_t n, bool optr) {
+    Mf2Layout L{};
     L.W = (n + 31u) / 32u;
     L.W4 = (L.W + 3u) & ~3u;
     L.o_inF = n;
@@ -81,7 +81,7 @@ __host__ __device__ inline Mf2Layout mf2_layout(uint32_t n, bool optr) {
     L.words = L.o_optr + (optr ? (n + 2u) / 2u : 0u);
     return L;
 }
-__host__ __device__ inline uint32_t mf2_node_bytes(uint32_t n, bool optr) {
+__host__ __device__ constexpr uint32_t mf2_node_bytes(uint32_t n, bool optr) {
     return 4u * mf2_layout(n, optr).words;
 }
 

@@ -681,10 +681,14 @@ def test_maxflow_fallback_list(solver, O):
     sc = np.concatenate([s2, s3]); ec = np.concatenate([e2, e3])
     offc = np.array([0, len(s2), len(sc)], np.uint64)
     prm = (64, 150, 1, 0, 0xffffffff)  # no segmentation: a 90 001-node component
+    solver.kernel_profile_reset()
     r2 = solver.solve(sc, ec, [90_000, 20_000], 30, read_off=offc, params=prm, verify=True,
-                      want_vectors=True)
+                      want_vectors=True, profile=True)
+    launches = {k["name"]: k["launches"] for k in solver.kernel_profile()}
     assert r2.n_components == 2
     assert_parity(O, r2, sc, ec, [90_000, 20_000], offc, 30, prm)
+    # the 20 001-node component in k_maxflow_sm, the 90 001-node one on the list for k_maxflow
+    assert launches["maxflow"] == 2, launches
 
 
 def test_zero_length_reads_are_accepted_and_never_kept(solver, O, pkg):
